@@ -2,6 +2,7 @@
 """bench.py — the driver's benchmark contract for the TUNA SCF two-electron hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload direct:et400|stored:n2_ccpvtz|...]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[4], the one the metric's "1/2/4/8 B200 ... % FP64 peak" is quoted on, at its largest
 point): the synthetic even-tempered N2 diatomic at nbf=800 (ncart 1102), direct ERI + J/K, one density.  The other sweep
@@ -169,6 +170,24 @@ def host_threads():
     return len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as <out_dir>/<name>.npy in float64, so that two builds can be compared output for output.  Above
+    DUMP_LIMIT_BYTES in all, every array is cut to a fixed, seeded sample of its flattened elements (the same elements on every
+    run of the same workload), sized so that the files stay under the limit."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_LIMIT_BYTES - 4096 * len(arrays)          # room for the .npy headers
+    for name, a in arrays.items():
+        if total > budget:
+            keep = budget * a.size // total
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, size=keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # CPU reference arm (oracle/_ref = the unmodified reference engine; numpy einsum = the reference's J/K, tuna_scf.py:42,70)
 # ----------------------------------------------------------------------------------------------------------------
@@ -309,8 +328,9 @@ def time_steps(torch, stream, fn, steps, warmup, flush, dist=None):
     return total_ms
 
 
-def bench_stored(torch, wl, steps, warmup, device):
-    """configs[1]-style: dense tensor resident, fused J+K per step."""
+def bench_stored(torch, wl, steps, warmup, device, outputs=None):
+    """configs[1]-style: dense tensor resident, fused J+K per step.  With a dict `outputs`, J and K of the last timed step are
+    stored in it as host arrays shaped like the return of coulomb_and_exchange."""
     import tuna_b200
     from tuna_b200.basis import flatten
     ctx = tuna_b200.Context(device)
@@ -330,6 +350,9 @@ def bench_stored(torch, wl, steps, warmup, device):
     flush = L2Flush(torch)
     l0 = ctx.counts()["launches"]
     ms = time_steps(torch, stream, lambda: ctx.jk_stored_dev(nD, dP.data_ptr(), dJK[0].data_ptr(), dJK[1].data_ptr()), steps, warmup, flush)
+    if outputs is not None:
+        jk = dJK.cpu().numpy()
+        outputs["J"], outputs["K"] = (jk[0], jk[1]) if nD > 1 else (jk[0, 0], jk[1, 0])
     launches = ctx.counts()["launches"] - l0 - 2 * warmup * ((nD + 3) // 4)
     # per-launch kernel time from the context's own events on the same stream
     kms = []
@@ -548,8 +571,11 @@ def run_ours(args, wl):
         if world > 1:
             raise SystemExit("stored mode is a single-GPU workload (SURVEY.md 8e); use a direct: workload for --gpus > 1")
         sampler.start()
-        res, ctx = bench_stored(torch, wl, args.steps, args.warmup, local)
+        outputs = {} if args.dump_outputs else None
+        res, ctx = bench_stored(torch, wl, args.steps, args.warmup, local, outputs)
         clocks = sampler.stop()
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         line = {"metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"],
                 "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                 "config": {"workload": res["workload"], "nbf": res["nbf"], "ncart": res["ncart"], "mode": "stored", "l2": res["l2"]},
@@ -578,6 +604,9 @@ def run_ours(args, wl):
     fb.stream.synchronize()
     l0 = ctx.counts()["launches"]
     ms = time_steps(torch, fb.stream, fb.build_device, args.steps, 0, flush, ddist)
+    if args.dump_outputs and rank == 0:       # after the all-reduce every rank holds the full J and K
+        jk = fb.dJK.cpu().numpy()
+        dump_outputs(args.dump_outputs, {"J": jk[0], "K": jk[1]} if nD > 1 else {"J": jk[0, 0], "K": jk[1, 0]})
     launches = ctx.counts()["launches"] - l0
     k_ms = ctx.last_kernel_ms(3)
     evaluated = ctx.counts()["evaluated_last_direct"]
@@ -683,7 +712,13 @@ def main():
     ap.add_argument("--tau", type=float, default=1e-16)
     ap.add_argument("--no-stored", action="store_true", help="skip the extra stored-mode (configs[1]) and sweep measurements at N=1")
     ap.add_argument("--extra-one-electron", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write J and K of the last timed step as DIR/J.npy and "
+                                                          "DIR/K.npy (float64; a fixed, seeded sample above 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.extra_one_electron:       # child of the N=1 run: one-electron integrals of configs[1] and of the headline basis
         print(json.dumps([bench_one_electron(load_workload("stored:n2_ccpvtz")), bench_one_electron(load_workload(args.workload))]), flush=True)
         return

@@ -63,6 +63,17 @@ def test_oracle_vs_compiled_reference(oracle, name):
     close(oracle.cross_overlap(fb, sub), refc, f"{name} S_cross")
 
 
+@pytest.mark.parametrize("name", list(CHARGES))
+def test_oracle_vs_reference_scf_matrices(oracle, name):
+    """The spherical images of S, T and V_NE against the matrices the reference's own SCF used (fixtures), without the reference tree."""
+    g = load_golden(name)
+    fb = oracle_basis(oracle, g)
+    S, T, V = oracle.one_electron(fb, *molecule_inputs(fb, name))[:3]
+    U = np.array(g["U"])
+    assert np.abs(U @ S @ U.T - np.array(g["S"])).max() < 1e-12
+    assert np.abs(U @ T @ U.T - np.array(g["T"])).max() < 1e-11 and np.abs(U @ V @ U.T - np.array(g["V_NE"])).max() < 1e-11
+
+
 @pytest.fixture(scope="module")
 def emul():
     so = os.path.join(HERE, "host_emul", "libemul_oneel.so")
