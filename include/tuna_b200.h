@@ -76,7 +76,9 @@ int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, doub
 /* Direct (integral-driven) Fock contraction: same J and K, in the basis of U (nbf x nbf matrices), never
  * materialising the tensor: 8-fold symmetry, Schwarz screening |Q_ij Q_kl| max|P| < tau skipped.
  * tau <= 0 disables screening.  tuna_jk_direct accepts any real P (a non-symmetric density is split into its symmetric and
- * antisymmetric parts: J[P] = J[S], K[P] = K[S] + K[A]); tuna_jk_direct_dev expects symmetric densities (SCF densities are).
+ * antisymmetric parts: J[P] = J[S], K[P] = K[S] + K[A]).  tuna_jk_direct_dev REQUIRES symmetric densities and does not check:
+ * it builds K = U (Kacc + Kacc^T) U^T, symmetric by construction, so for a non-symmetric P it silently drops K[A].  Callers with
+ * possibly asymmetric densities (e.g. guess densities, asymmetric at ~1e-8) use tuna_jk_direct.
  * The cached quartet lists are pre-screened with tau / (1e3 max(1, max|P|)) for host densities; tuna_jk_direct_dev assumes max|P| <= ~10
  * (scale larger device densities down - J and K are linear in P).  J and K are accumulated as 64-bit integers (order independent):
  * repeated builds are bitwise identical; |J|, |K| < 2^42 in the unnormalised Cartesian working basis is required. */

@@ -1621,14 +1621,18 @@ extern "C" int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, doubl
         const char* env_tile = getenv("TUNA_B200_JK_TILE_KB");
         const char* env_st = getenv("TUNA_B200_JK_STAGES");
         const char* env_cps = getenv("TUNA_B200_JK_CTAS_PER_SM");
-        const size_t tile_budget = (env_tile ? atoi(env_tile) : 24) * 1024;
+        // knobs are clamped to what the kernel can run: a zero tile would divide by zero, zero stages would leave the consumers waiting
+        // on an mbarrier no copy ever completes, zero CTAs per SM an empty grid, and a ring larger than 227 KB would not launch
+        const size_t tile_budget = (size_t)(env_tile ? std::min(64, std::max(1, atoi(env_tile))) : 24) * 1024;
         int q = (int)((nn * sizeof(double) + tile_budget - 1) / tile_budget);
         int R = (n + q - 1) / q;
         R = (R + r - 1) / r * r;                       // whole row groups per tile
         q = (n + R - 1) / R;
-        const int nstage = env_st ? std::min(atoi(env_st), JK_MAX_STAGES) : 3;
+        int nstage = env_st ? std::max(1, std::min(atoi(env_st), JK_MAX_STAGES)) : 3;
+        const size_t smem_fixed = (2 * (size_t)nwarp * 4 + (size_t)4 * r * n) * sizeof(double) + JK_MAX_STAGES * sizeof(uint64_t) + 16;
+        while (nstage > 1 && (size_t)nstage * R * n * sizeof(double) + smem_fixed > 227 * 1024) --nstage;
         const long long total = (long long)n * n;
-        const int grid = (int)std::min<long long>((long long)ctx->sm_count * (env_cps ? atoi(env_cps) : 2), total);
+        const int grid = (int)std::min<long long>((long long)ctx->sm_count * (env_cps ? std::max(1, atoi(env_cps)) : 2), total);
         const int kslots = (int)((total / grid + 1 + n - 1) / n) + 2;
         const int nslots = grid * kslots;
         const size_t need_kpart = (size_t)nslots * 4 * n + (size_t)(nslots + 1) / 2 + 8;       // doubles: partial rows + row tags
@@ -2133,6 +2137,15 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     return TUNA_OK;
 }
 
+// Register budget of a job's own k_shell4_one launch.  A G = 256, NB <= 2 class whose shared-memory footprint already limits the SM to
+// two 256-thread CTAs gets the 128-register build (no spills, more loads in flight in the unrolled digestion); TUNA_B200_REG_TIER=0
+// forces the default build.  Grouped jobs (k_shell4_multi) always use the default build.
+static int shell4_one_regs(const tuna_ctx::Job4Host& jh) {
+    static const bool tiers = !(getenv("TUNA_B200_REG_TIER") && atoi(getenv("TUNA_B200_REG_TIER")) == 0);
+    const size_t by_smem = std::max<size_t>(1, (size_t)(228 * 1024) / (jh.smem + 1024));
+    return tiers && jh.G == 256 && jh.nb <= 2 && by_smem * jh.threads * 128 <= 65536 ? 128 : TUNA_SHELL4_REGS;
+}
+
 // Job list of the shell-quartet engine for threshold tau and nD densities.
 static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
     int rc;
@@ -2300,12 +2313,15 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
     }
     if (const char* dump = getenv("TUNA_B200_DUMP_JOBS")) {       // development aid: the job table in launch order
         if (FILE* f = fopen(dump, "w")) {
-            fprintf(f, "idx,La,Lb,Lc,Ld,nppAB,nppCD,G,nb,threads,smem,total,nout,nint,itmax,nchunk,nitems,allowed,own\n");
+            // regs: register budget of the kernel build that runs the job; terms: 1 = term-list digestion, 0 = separable;
+            // psplit / ksplit: work items per shell quartet and ket chunks among them
+            fprintf(f, "idx,La,Lb,Lc,Ld,nppAB,nppCD,G,nb,threads,smem,total,nout,nint,itmax,nchunk,nitems,allowed,own,regs,terms,psplit,ksplit,nD\n");
             int idx = 0;
             for (const auto& jh : jobs4)
-                fprintf(f, "%d,%d,%d,%d,%d,%d,%d,%d,%d,%d,%zu,%d,%d,%d,%d,%d,%lld,%.0f,%d\n", idx++, jh.job.La, jh.job.Lb, jh.job.Lc, jh.job.Ld, jh.job.nppAB,
-                        jh.job.nppCD, jh.G, jh.nb, jh.threads, jh.smem, jh.job.total, jh.job.ct.nwork, jh.job.ct.itmax, jh.job.ct.itmax, jh.job.ct.nchunk,
-                        jh.job.nitems, jh.allowed, (int)jh.own_launch);
+                fprintf(f, "%d,%d,%d,%d,%d,%d,%d,%d,%d,%d,%zu,%d,%d,%d,%d,%d,%lld,%.0f,%d,%d,%d,%d,%d,%d\n", idx++, jh.job.La, jh.job.Lb, jh.job.Lc, jh.job.Ld,
+                        jh.job.nppAB, jh.job.nppCD, jh.G, jh.nb, jh.threads, jh.smem, jh.job.total, jh.job.ct.nwork, jh.job.ct.itmax, jh.job.ct.itmax,
+                        jh.job.ct.nchunk, jh.job.nitems, jh.allowed, (int)jh.own_launch, jh.own_launch ? shell4_one_regs(jh) : TUNA_SHELL4_REGS,
+                        (int)(jh.job.ct.nterm2 > 0), jh.job.psplit, jh.job.ksplit, nD);
             fclose(f);
         }
     }
@@ -2331,11 +2347,8 @@ static cudaError_t launch_shell4_one(tuna_ctx* ctx, const tuna_ctx::Job4Host& jh
     const size_t by_smem = std::max<size_t>(1, (size_t)(228 * 1024) / (jh.smem + 1024));
     const size_t by_thr = std::max<size_t>(1, 2048 / jh.threads);
     blocks = std::min<long long>(blocks, (long long)ctx->sm_count * (long long)std::min(by_smem, by_thr) * 2);
-    // a class whose shared-memory footprint already limits the SM to two 256-thread CTAs gets the 128-register build (no spills,
-    // more loads in flight in the unrolled digestion); TUNA_B200_REG_TIER=0 forces the 64-register build
     if constexpr (GG == 256 && NB <= 2) {
-        static const bool tiers = !(getenv("TUNA_B200_REG_TIER") && atoi(getenv("TUNA_B200_REG_TIER")) == 0);
-        if (tiers && by_smem * jh.threads * 128 <= 65536) return launch_shell4_one_r<GG, NB, 128>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
+        if (shell4_one_regs(jh) == 128) return launch_shell4_one_r<GG, NB, 128>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
     }
     return launch_shell4_one_r<GG, NB, TUNA_SHELL4_REGS>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
 }
