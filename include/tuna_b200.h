@@ -87,6 +87,17 @@ int tuna_jk_direct_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, doub
 /* Multi-GPU sharding of the quartet list for tuna_jk_direct*: this context evaluates only its share and
  * returns PARTIAL J/K, to be summed over ranks by the caller (one all-reduce per build, SURVEY.md 8e). */
 int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks);
+/* Direct J/K of ONE Fock build spread over nctx contexts on pairwise distinct devices of this process: same basis and transform in
+ * every context, ctxs[r] sharded as (r, nctx) with tuna_set_shard.  Each rank accumulates its share of the quartets on its own device
+ * (enqueued from one host thread per device, all joined before the call returns); the 64-bit integer accumulators of all ranks are
+ * pulled to ctxs[0]'s device and summed there before the conversion to FP64, so J and K are bitwise identical to tuna_jk_direct /
+ * tuna_jk_direct_dev on one context (within FP64 round-off for bases that run the per-component kernel).  nctx == 1 is tuna_jk_direct.
+ * TUNA_ERR_ARG: nctx < 1, a null or repeated context, two contexts on one device.  TUNA_ERR_STATE: a context with a different basis or
+ * transform (ncart, nbf, checksums of the arrays given to tuna_set_basis / tuna_set_transform) or a shard other than (r, nctx).
+ * Errors are reported through tuna_last_error(ctxs[0]), the failing rank named. */
+int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* P, double* J, double* K, double tau);
+/* dP, dJ, dK on ctxs[0]'s device, enqueued on ctxs[0]'s stream; symmetric densities only, as tuna_jk_direct_dev. */
+int tuna_jk_direct_group_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau);
 
 /* AO -> MO / spin-orbital four-index transformation of a dense ERI tensor (SURVEY.md 8f-2):
  *   tuna_ci.transform_ERI_AO_to_MO(ERI_AO, C, ...)        tuna_ci.py:204-255   so_layout = 0, C1 = C2 = C
@@ -125,7 +136,9 @@ int tuna_cross_overlap(tuna_ctx* ctx, int n1, const double* origins_z1, const in
  * [5] kernels launched by this context so far, [6] ncart, [7] nbf. */
 int tuna_get_counts(const tuna_ctx* ctx, int64_t counts[8]);
 /* Device time (ms, CUDA events on the launching stream) of the dominant kernel of the last call:
- * which = 0 ERI fill, 1 cart->sph, 2 stored J/K, 3 direct J/K, 4 AO->MO transformation, 5 one-electron integrals.  Synchronises the stream. */
+ * which = 0 ERI fill, 1 cart->sph, 2 stored J/K, 3 direct J/K (the accumulation of the last density pass), 4 AO->MO transformation,
+ * 5 one-electron integrals, 6 on ctxs[0] of a tuna_jk_direct_group call with nctx > 1: from the end of the last rank's accumulation to
+ * J/K ready (pull, sum, finish) of the last density pass.  Synchronises the stream. */
 int tuna_last_kernel_ms(tuna_ctx* ctx, int which, float* ms);
 /* Algorithmic FP64 flop count of the reference algorithm for the parity-surviving unique quartets of the
  * current basis (formula F(a,b) of SURVEY.md section 8d), and the J/K digestion flops per density. */

@@ -2,7 +2,7 @@
 ERI evaluation (tuna_integrals) + Coulomb/exchange contraction (tuna_scf), behind the reference's own
 Python call signatures.  See DESIGN.md and INTEGRATION.md."""
 from . import workloads  # noqa: F401
-from ._lib import Context, TunaError  # noqa: F401
+from ._lib import Context, DeviceGroup, TunaError  # noqa: F401
 from .basis import Basis  # noqa: F401
 from .provider import (  # noqa: F401
     ERIHandle, calculate_coulomb_matrix, calculate_cross_basis_overlap_matrix, calculate_one_electron_integrals, calculate_electron_repulsion_integral, calculate_electron_repulsion_integrals,

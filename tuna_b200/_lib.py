@@ -18,7 +18,7 @@ EXPORTS = [
     "tuna_eri_fill_cart", "tuna_eri_cart_to_sph", "tuna_eri_download", "tuna_eri_upload", "tuna_eri_single", "tuna_schwarz",
     "tuna_jk_stored", "tuna_jk_stored_dev", "tuna_jk_direct", "tuna_jk_direct_dev", "tuna_set_shard", "tuna_get_counts",
     "tuna_last_kernel_ms", "tuna_algorithmic_flops", "tuna_fp64_peak_probe", "tuna_eri_transform", "tuna_eri_transform_dev",
-    "tuna_eri_transform_spin_blocked", "tuna_one_electron", "tuna_cross_overlap",
+    "tuna_eri_transform_spin_blocked", "tuna_one_electron", "tuna_cross_overlap", "tuna_jk_direct_group", "tuna_jk_direct_group_dev",
 ]
 
 _lib = None
@@ -70,6 +70,8 @@ def load() -> ctypes.CDLL:
         "tuna_eri_transform_spin_blocked": (ci, [vp, ci, c_dp, ci, c_dp, ci, c_dp]),
         "tuna_one_electron": (ci, [vp, ci, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp]),
         "tuna_cross_overlap": (ci, [vp] + [ci, c_dp, c_ip, c_ip, c_lp, c_dp, c_dp] * 2 + [c_dp]),
+        "tuna_jk_direct_group": (ci, [ctypes.POINTER(vp), ci, ci, c_dp, c_dp, c_dp, cd]),
+        "tuna_jk_direct_group_dev": (ci, [ctypes.POINTER(vp), ci, ci, vp, vp, vp, cd]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -115,6 +117,8 @@ class Context:
         self.ncart = 0
         self.nbf = 0
         self.n_stored = 0
+        self.basis_flat = None      # the arrays of set_basis and the U of set_transform, for a DeviceGroup over the same basis
+        self.U = None
 
     # -- error mapping: MemoryError like pyx:1120/1290, everything else the reference's TunaError ------------
     def _raise(self, rc, msg=None):
@@ -155,6 +159,7 @@ class Context:
                                           off.ctypes.data_as(i64p), _dp(exps), _dp(ce)))
         self.ncart, self.nbf, self.n_stored = len(oz), 0, 0
         self.lmn = lmn
+        self.basis_flat, self.U = (oz, lmn, nprim, exps, ce), None
 
     def set_transform(self, U):
         U = np.ascontiguousarray(U, dtype=np.float64)
@@ -162,6 +167,7 @@ class Context:
             raise error_class(f"tuna_b200: transformation matrix has shape {U.shape}, expected (nbf, {self.ncart})")
         self._ck(self._lib.tuna_set_transform(self._h, U.shape[0], _dp(U)))
         self.nbf = U.shape[0]
+        self.U = U
 
     def eri_fill_cart(self):
         self._ck(self._lib.tuna_eri_fill_cart(self._h))
@@ -317,3 +323,83 @@ class Context:
         t = ctypes.c_double()
         self._ck(self._lib.tuna_fp64_peak_probe(self._h, ctypes.byref(t)))
         return t.value
+
+
+class DeviceGroup:
+    """One direct Fock build spread over several GPUs of this process (tuna_jk_direct_group): one Context per device, rank r sharded as
+    (r, len(devices)); the integer accumulators of all ranks are summed on devices[0] before the conversion to FP64, so J and K are bitwise
+    equal to a single Context's.  devices[0] receives the densities and returns J and K."""
+
+    def __init__(self, devices):
+        devices = [int(d) for d in devices]
+        if not devices or len(set(devices)) != len(devices) or min(devices) < 0:
+            raise error_class(f"tuna_b200: a device group needs distinct non-negative device ordinals, got {devices}")
+        self.devices = devices
+        self.contexts = []
+        try:
+            for r, d in enumerate(devices):
+                self.contexts.append(Context(d))
+                self.contexts[-1].set_shard(r, len(devices))
+        except BaseException:
+            self.close()
+            raise
+        self._ptrs = (ctypes.c_void_p * len(devices))(*[c._h.value for c in self.contexts])
+        self._lib = self.contexts[0]._lib
+
+    @property
+    def ncart(self):
+        return self.contexts[0].ncart
+
+    @property
+    def nbf(self):
+        return self.contexts[0].nbf
+
+    def set_basis(self, origins_z, lmn, nprim, exps, coef_eff):
+        for c in self.contexts:
+            c.set_basis(origins_z, lmn, nprim, exps, coef_eff)
+
+    def set_transform(self, U):
+        for c in self.contexts:
+            c.set_transform(U)
+
+    def _ck(self, rc):
+        if rc:
+            self.contexts[0]._raise(rc)
+
+    def jk_direct(self, P, tau=1e-16, want_j=True, want_k=True):
+        """Same contract as Context.jk_direct: (n, n) or (nD, n, n), any real P, host arrays in and out."""
+        P = np.ascontiguousarray(P, dtype=np.float64)
+        n = self.nbf
+        single = P.ndim == 2
+        Ps = P[None] if single else P
+        if Ps.ndim != 3 or Ps.shape[1:] != (n, n):
+            raise error_class(f"tuna_b200: density matrix has shape {P.shape}, expected ({n}, {n})")
+        J = np.empty_like(Ps) if want_j else None
+        K = np.empty_like(Ps) if want_k else None
+        self._ck(self._lib.tuna_jk_direct_group(self._ptrs, len(self.contexts), Ps.shape[0], _dp(Ps), _dp(J), _dp(K), ctypes.c_double(tau)))
+        if single:
+            return (J[0] if want_j else None), (K[0] if want_k else None)
+        return J, K
+
+    def jk_direct_dev(self, nD, dP, dJ, dK, tau=1e-16):
+        """Device pointers on devices[0], enqueued on the stream of contexts[0]; symmetric densities only (tuna_jk_direct_dev)."""
+        self._ck(self._lib.tuna_jk_direct_group_dev(self._ptrs, len(self.contexts), nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ), ctypes.c_void_p(dK),
+                                                    ctypes.c_double(tau)))
+
+    def counts(self) -> dict:
+        """Counters of contexts[0], with evaluated_last_direct summed over all ranks."""
+        per_rank = [c.counts() for c in self.contexts]
+        out = dict(per_rank[0])
+        out["evaluated_last_direct"] = sum(c["evaluated_last_direct"] for c in per_rank)
+        return out
+
+    def close(self):
+        for c in self.contexts:
+            c.close()
+        self.contexts = []
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

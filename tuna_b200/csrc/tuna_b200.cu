@@ -17,11 +17,13 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cstdio>
 #include <cstring>
 #include <map>
 #include <new>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/tuna_b200.h"
@@ -89,7 +91,8 @@ struct tuna_ctx {
     unsigned long long* d_scalars = nullptr;   // [0] max|P| bits, [1] evaluated-quartet counter
 
     int shard_rank = 0, shard_n = 1;
-    cudaEvent_t ev[6][2] = {};
+    cudaEvent_t ev[7][2] = {};
+    uint64_t basis_sum = 0, U_sum = 0;     // checksums of the arrays given to tuna_set_basis / tuna_set_transform (tuna_jk_direct_group)
 
     // AO -> MO four-index transformation (mo_transform.cuh): two ping-pong work buffers, grown on demand
     double* d_mo_ws[2] = {nullptr, nullptr};
@@ -127,6 +130,9 @@ struct tuna_ctx {
     // point with larger densities scale them down (J and K are linear in P).
     double dens_bound = 1e3;
     long long* d_fix = nullptr; size_t cap_fix = 0;      // reproducible accumulation: [J hi | J lo | K hi | K lo], nD * ncart^2 words each
+    long long* d_peer = nullptr; size_t cap_peer = 0;    // tuna_jk_direct_group on ctxs[0]: the other ranks' accumulators, pulled for k_fix_reduce
+    cudaEvent_t ev_group = nullptr;                      // tuna_jk_direct_group: cross-device ordering (density ready / accumulate done / pulled)
+    unsigned long long peers_tried = 0;                  // tuna_jk_direct_group on ctxs[0]: devices whose peer access with this one was requested
     CsrDev Uf, Uft;                 // U * diag(f) and its transpose: per-component norms folded into the rotation
     int direct_engine = 1;          // 1 = shell engine when the basis groups into shells, 0 = per-component kernel
 
@@ -149,6 +155,13 @@ struct tuna_ctx {
     catch (const std::exception& e_) { if (ctx) ctx->err = std::string("internal error: ") + e_.what(); return TUNA_ERR_STATE; } \
     catch (...) { if (ctx) ctx->err = "internal error"; return TUNA_ERR_STATE; }
 
+// FNV-1a over raw bytes: tuna_jk_direct_group compares the basis and transform of its contexts with it
+static uint64_t checksum(const void* p, size_t bytes, uint64_t h = 1469598103934665603ull) {
+    const unsigned char* c = static_cast<const unsigned char*>(p);
+    for (size_t i = 0; i < bytes; ++i) h = (h ^ c[i]) * 1099511628211ull;
+    return h;
+}
+
 static int check_pair_symmetry(tuna_ctx* ctx);
 static int ensure_shell4(tuna_ctx* ctx, double tau, int nD);
 static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const double* Psym, double* Jc, double* Kc, double tau, long long fix_lo);
@@ -156,13 +169,14 @@ static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const dou
 
 // Opt-in to more than 48 KB of dynamic shared memory.  The attribute is PER DEVICE (a process may hold contexts on several GPUs), so the
 // "already done" flag is a bit per device ordinal, one flag word per kernel instantiation.
+// tuna_jk_direct_group enqueues from one host thread per device, hence the atomic.
 template <auto Kernel>
 static cudaError_t opt_in_smem(const tuna_ctx* ctx) {
-    static unsigned long long done = 0;
+    static std::atomic<unsigned long long> done{0};
     const unsigned long long bit = 1ull << (ctx->device & 63);
-    if (done & bit) return cudaSuccess;
+    if (done.load() & bit) return cudaSuccess;
     const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) done |= bit;
+    if (e == cudaSuccess) done.fetch_or(bit);
     return e;
 }
 
@@ -1180,8 +1194,9 @@ int tuna_ctx_create(int device, tuna_ctx** out) {
     ctx->sm_count = prop.multiProcessorCount;
     CK(cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking));
     ctx->stream = ctx->own_stream;
-    for (int w = 0; w < 6; ++w)
+    for (int w = 0; w < 7; ++w)
         for (int s = 0; s < 2; ++s) CK(cudaEventCreate(&ctx->ev[w][s]));
+    CK(cudaEventCreateWithFlags(&ctx->ev_group, cudaEventDisableTiming));
     for (int a = 0; a < tuna_ctx::NAUX; ++a) {
         CK(cudaStreamCreateWithFlags(&ctx->aux[a], cudaStreamNonBlocking));
         CK(cudaEventCreateWithFlags(&ctx->ev_join[a], cudaEventDisableTiming));
@@ -1214,7 +1229,7 @@ int tuna_ctx_destroy(tuna_ctx* ctx) {
     dev_free(&ctx->d_P); dev_free(&ctx->d_J); dev_free(&ctx->d_K);
     dev_free(&ctx->d_Pc); dev_free(&ctx->d_Jc); dev_free(&ctx->d_Kc); dev_free(&ctx->d_tmp); dev_free(&ctx->d_Kpart);
     for (auto& kv : ctx->class_tabs4) dev_free(&kv.second.blob);
-    dev_free(&ctx->d_fix);
+    dev_free(&ctx->d_fix); dev_free(&ctx->d_peer);
     dev_free(&ctx->d_pairA); dev_free(&ctx->d_pairB); dev_free(&ctx->d_pair_rec); dev_free(&ctx->d_rec);
     dev_free(&ctx->d_pairQ); dev_free(&ctx->d_sh_ao); dev_free(&ctx->d_class_lists); dev_free(&ctx->d_finv);
     for (auto& js : ctx->jobsets4) free_jobset4(js);
@@ -1224,8 +1239,9 @@ int tuna_ctx_destroy(tuna_ctx* ctx) {
     dev_free(&ctx->Uft.rowptr); dev_free(&ctx->Uft.col); dev_free(&ctx->Uft.val);
     if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
     dev_free(&ctx->d_mo_ws[0]); dev_free(&ctx->d_mo_ws[1]);
-    for (int w = 0; w < 6; ++w)
+    for (int w = 0; w < 7; ++w)
         for (int s = 0; s < 2; ++s) if (ctx->ev[w][s]) cudaEventDestroy(ctx->ev[w][s]);
+    if (ctx->ev_group) cudaEventDestroy(ctx->ev_group);
     for (int a = 0; a < tuna_ctx::NAUX; ++a) {
         if (ctx->aux[a]) { cudaStreamSynchronize(ctx->aux[a]); cudaStreamDestroy(ctx->aux[a]); }
         if (ctx->ev_join[a]) cudaEventDestroy(ctx->ev_join[a]);
@@ -1273,6 +1289,10 @@ int tuna_set_basis(tuna_ctx* ctx, int ncart, const double* origins_z, const int3
         FAIL(TUNA_ERR_NOMEM, "host allocation failed while copying the basis");
     }
     ctx->ncart = ncart;
+    ctx->basis_sum = checksum(B.oz.data(), B.oz.size() * sizeof(B.oz[0]), checksum(B.lmn.data(), B.lmn.size() * sizeof(B.lmn[0]),
+                     checksum(B.nprim.data(), B.nprim.size() * sizeof(B.nprim[0]), checksum(B.off.data(), B.off.size() * sizeof(B.off[0]),
+                     checksum(B.exps.data(), B.exps.size() * sizeof(B.exps[0]), checksum(B.ceff.data(), B.ceff.size() * sizeof(B.ceff[0])))))));
+    ctx->U_sum = 0;
     ctx->pairs_ready = false;
     ctx->pt = PairTable();
     ctx->n_unique = ctx->n_surviving = ctx->n_primq = 0;
@@ -1315,6 +1335,7 @@ int tuna_set_transform(tuna_ctx* ctx, int nbf, const double* U) try {
         if ((rc = build_csr(ctx, ctx->Uft, nc, nbf, uft))) return rc;
     }
     ctx->nbf = nbf;
+    ctx->U_sum = checksum(u.data(), u.size() * sizeof(double), (uint64_t)nbf);
     ctx->U_identity = (nbf == nc);
     for (int p = 0; p < nbf && ctx->U_identity; ++p)
         for (int a = 0; a < nc; ++a)
@@ -2416,37 +2437,11 @@ static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const dou
     return TUNA_OK;
 }
 
-// Core of direct mode on DEVICE buffers: nD densities, bit d of anti_mask marks density d as antisymmetric
-// (its K is Kacc - Kacc^T and its J vanishes); all others must be symmetric.
-static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti_mask, double* dJ, double* dK, double tau);
-
-// Densities are processed in passes small enough for the largest class of the basis to fit its J/K blocks in shared memory.
-static int jk_direct_core(tuna_ctx* ctx, int nD, const double* dP, unsigned anti_mask, double* dJ, double* dK, double tau) {
-    if (ctx->ncart == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_basis first");
-    if (ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_transform first");
-    if (nD <= 0 || nD > 16 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct: bad arguments (1 <= nD <= 16)");
-    int nd_max = 4;
-    if (ctx->direct_engine == 1 && ctx->ss.ok) {
-        int Lmax = 0;
-        for (const auto& sh : ctx->ss.shells) Lmax = std::max(Lmax, sh.L);
-        // staged densities + accumulators of the largest class: about 4 (nc + 4)^2 + 8 nc^2 doubles per density next to ~9000 doubles of tables
-        const int nc = ctx->stab.nc[Lmax], per_density = 4 * (nc + 4) * (nc + 4) + 8 * nc * nc;
-        while (nd_max > 1 && nd_max * per_density + 9000 > SHELL4_SMEM_DOUBLES) --nd_max;
-    }
-    const int npass = (nD + nd_max - 1) / nd_max, per = (nD + npass - 1) / npass;
-    const size_t nn = (size_t)ctx->nbf * ctx->nbf;
-    for (int d0 = 0; d0 < nD; d0 += per) {
-        const int nd = std::min(per, nD - d0);
-        int rc = jk_direct_pass(ctx, nd, dP + d0 * nn, (anti_mask >> d0) & ((1u << nd) - 1u), dJ ? dJ + d0 * nn : nullptr, dK ? dK + d0 * nn : nullptr, tau);
-        if (rc) return rc;
-    }
-    return TUNA_OK;
-}
-
-static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti_mask, double* dJ, double* dK, double tau) {
-    if (ctx->ncart == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_basis first");
-    if (ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_transform first");
-    if (nD <= 0 || nD > 16 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct: bad arguments (1 <= nD <= 16)");
+// Direct mode on DEVICE buffers, in two halves that tuna_jk_direct_group runs on different devices.
+// jk_direct_accumulate: P_cart = U^T P U, then the shell engine's integer accumulators d_fix (the per-component kernel: d_Jc / d_Kc).
+// jk_direct_finish: J = U (Jacc + Jacc^T) U^T, K = U (Kacc +- Kacc^T) U^T from those accumulators; bit d of anti_mask marks density d as
+// antisymmetric (its K is Kacc - Kacc^T and its J vanishes); all others must be symmetric.
+static int jk_direct_accumulate(tuna_ctx* ctx, int nD, const double* dP, double tau) {
     const int nc = ctx->ncart, nb = ctx->nbf;
     const bool shell = ctx->direct_engine == 1 && ctx->ss.ok;
     int rc;
@@ -2455,7 +2450,6 @@ static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
     if (shell && (rc = ensure_shell4(ctx, tau, nD))) return rc;
     const size_t ncc = (size_t)nc * nc;
     const CsrDev& Uin = shell ? ctx->Uft : ctx->Ut;      // the shell engine works with unnormalised components: U' = U diag(f)
-    const CsrDev& Uout = shell ? ctx->Uf : ctx->U;
     // P_cart = U^T P U
     if ((rc = rotate(ctx, Uin, dP, ctx->d_tmp, nD, nb))) return rc;                          // [d][a][q] = sum_p U[p,a] P[d][p][q]
     if ((rc = rotate(ctx, Uin, ctx->d_tmp, ctx->d_Pc, (int64_t)nD * nc, 1))) return rc;      // [d][a][b] = sum_q U[q,b] tmp[d][a][q]
@@ -2487,8 +2481,6 @@ static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
         double* Jw = reinterpret_cast<double*>(ctx->d_fix);
         double* Kw = reinterpret_cast<double*>(ctx->d_fix + 2 * nacc);
         if ((rc = launch_shell4_jobs(ctx, nD, ctx->d_Pc, ctx->d_tmp, Jw, Kw, tau, (long long)nacc))) return rc;
-        k_fixed_to_double<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_fix, ctx->d_Jc, ctx->d_Kc, nacc);
-        ctx->launches++;
     } else {
         k_jk_direct<<<grid_for(ctx, ctx->task_begin[4] / ctx->shard_n + 1, 128, 16), 128, 0, ctx->stream>>>(
             table_dev(ctx), ctx->d_boys, ctx->d_herm, ctx->d_Q, ctx->d_Pc, ctx->d_Jc, ctx->d_Kc, nc, nD, tau, ctx->d_scalars, ctx->d_scalars + 1,
@@ -2497,7 +2489,19 @@ static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
         CK(cudaGetLastError());
     }
     CK(cudaEventRecord(ctx->ev[3][1], ctx->stream));
-    // J = U (Jacc + Jacc^T) U^T,  K = U (Kacc +- Kacc^T) U^T
+    return TUNA_OK;
+}
+
+static int jk_direct_finish(tuna_ctx* ctx, int nD, unsigned anti_mask, double* dJ, double* dK) {
+    const int nc = ctx->ncart, nb = ctx->nbf;
+    const bool shell = ctx->direct_engine == 1 && ctx->ss.ok;
+    const size_t ncc = (size_t)nc * nc, nacc = (size_t)nD * ncc;
+    const CsrDev& Uout = shell ? ctx->Uf : ctx->U;
+    int rc;
+    if (shell) {
+        k_fixed_to_double<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_fix, ctx->d_Jc, ctx->d_Kc, nacc);
+        ctx->launches++;
+    }
     for (int which = 0; which < 2; ++which) {
         double* acc = which == 0 ? ctx->d_Jc : ctx->d_Kc;
         double* out = which == 0 ? dJ : dK;
@@ -2508,6 +2512,243 @@ static int jk_direct_pass(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
         if ((rc = rotate(ctx, Uout, ctx->d_tmp, out, (int64_t)nD * nb, 1))) return rc;    // [d][p][q]
     }
     CK(cudaGetLastError());
+    return TUNA_OK;
+}
+
+// Densities are processed in passes small enough for the largest class of the basis to fit its J/K blocks in shared memory.
+static int direct_pass_densities(const tuna_ctx* ctx, int nD) {
+    int nd_max = 4;
+    if (ctx->direct_engine == 1 && ctx->ss.ok) {
+        int Lmax = 0;
+        for (const auto& sh : ctx->ss.shells) Lmax = std::max(Lmax, sh.L);
+        // staged densities + accumulators of the largest class: about 4 (nc + 4)^2 + 8 nc^2 doubles per density next to ~9000 doubles of tables
+        const int nc = ctx->stab.nc[Lmax], per_density = 4 * (nc + 4) * (nc + 4) + 8 * nc * nc;
+        while (nd_max > 1 && nd_max * per_density + 9000 > SHELL4_SMEM_DOUBLES) --nd_max;
+    }
+    const int npass = (nD + nd_max - 1) / nd_max;
+    return (nD + npass - 1) / npass;
+}
+
+static int jk_direct_core(tuna_ctx* ctx, int nD, const double* dP, unsigned anti_mask, double* dJ, double* dK, double tau) {
+    if (ctx->ncart == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_basis first");
+    if (ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: call tuna_set_transform first");
+    if (nD <= 0 || nD > 16 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct: bad arguments (1 <= nD <= 16)");
+    const int per = direct_pass_densities(ctx, nD);
+    const size_t nn = (size_t)ctx->nbf * ctx->nbf;
+    for (int d0 = 0; d0 < nD; d0 += per) {
+        const int nd = std::min(per, nD - d0);
+        int rc = jk_direct_accumulate(ctx, nd, dP + d0 * nn, tau);
+        if (!rc) rc = jk_direct_finish(ctx, nd, (anti_mask >> d0) & ((1u << nd) - 1u), dJ ? dJ + d0 * nn : nullptr, dK ? dK + d0 * nn : nullptr);
+        if (rc) return rc;
+    }
+    return TUNA_OK;
+}
+
+// Host densities -> ctx's pinned staging buffer h_pin.  A general P splits into symmetric S and antisymmetric A parts: J[P] = J[S],
+// K[P] = K[S] + K[A] with K[A] antisymmetric.  SCF densities are symmetric to round-off (reference guess densities are not always:
+// asymmetry ~1e-8 was observed); a density stack with max|P - P^T| > 1e-15 max|P| runs as 2 nD densities, S first, the A parts marked in
+// anti_mask.  Sets ctx->dens_bound from max|P|.
+static int stage_host_density(tuna_ctx* ctx, int nD, const double* P, int* nDrun, unsigned* anti_mask) {
+    const int nb = ctx->nbf;
+    const size_t nn = (size_t)nb * nb;
+    double pmax = 0.0, amax = 0.0;
+    for (int d = 0; d < nD; ++d)
+        for (int i = 0; i < nb; ++i)
+            for (int j = 0; j <= i; ++j) {
+                const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
+                pmax = std::max(pmax, std::max(std::fabs(x), std::fabs(y)));
+                amax = std::max(amax, std::fabs(x - y));
+            }
+    const bool general = amax > 1e-15 * pmax;
+    ctx->dens_bound = std::max(1e3, 1e3 * pmax);          // static pre-screening stays below the device's exact density-weighted test
+    *nDrun = general ? 2 * nD : nD;
+    *anti_mask = 0;
+    int rc;
+    if ((rc = ensure_mats(ctx, *nDrun, nb, ctx->ncart))) return rc;
+    double* hP = ctx->h_pin;
+    if (!general) {
+        std::memcpy(hP, P, (size_t)nD * nn * sizeof(double));
+    } else {
+        for (int d = 0; d < nD; ++d) {
+            *anti_mask |= 1u << (nD + d);
+            for (int i = 0; i < nb; ++i)
+                for (int j = 0; j < nb; ++j) {
+                    const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
+                    hP[d * nn + (size_t)i * nb + j] = 0.5 * (x + y);
+                    hP[(nD + d) * nn + (size_t)i * nb + j] = 0.5 * (x - y);
+                }
+        }
+    }
+    return TUNA_OK;
+}
+
+// ctx->d_J / d_K (nDrun densities, as staged by stage_host_density) -> the caller's J and K; adds K[A] to K[S] for a general P.
+static int unstage_host_results(tuna_ctx* ctx, int nD, int nDrun, double* J, double* K) {
+    const size_t nn = (size_t)ctx->nbf * ctx->nbf, bytes = (size_t)nDrun * nn * sizeof(double);
+    double* hJ = ctx->h_pin + (size_t)nDrun * nn;
+    double* hK = hJ + (size_t)nDrun * nn;
+    if (J) CK(cudaMemcpyAsync(hJ, ctx->d_J, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (K) CK(cudaMemcpyAsync(hK, ctx->d_K, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (J) std::memcpy(J, hJ, (size_t)nD * nn * sizeof(double));
+    if (K) {
+        std::memcpy(K, hK, (size_t)nD * nn * sizeof(double));
+        if (nDrun > nD)
+            for (size_t x = 0; x < (size_t)nD * nn; ++x) K[x] += hK[(size_t)nD * nn + x];
+    }
+    return TUNA_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// one direct build over several devices (tuna_jk_direct_group)
+// ------------------------------------------------------------------------------------------------
+// acc[i] += stage[i] + stage[stride + i] + ... (npeer terms, in rank order).  For the shell engine's integer words T is unsigned: the sum
+// wraps exactly like the atomicAdd on unsigned long long of DevPolicy::accumulate, so N partial accumulators add up to the 1-device words.
+template <typename T>
+__global__ void k_fix_reduce(T* __restrict__ acc, const T* __restrict__ stage, size_t count, size_t stride, int npeer) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x) {
+        T s = acc[i];
+        for (int p = 0; p < npeer; ++p) s += stage[(size_t)p * stride + i];
+        acc[i] = s;
+    }
+}
+
+static int group_check(tuna_ctx* const* ctxs, int nctx) {
+    if (!ctxs || nctx < 1 || !ctxs[0]) return TUNA_ERR_ARG;
+    tuna_ctx* ctx = ctxs[0];
+    if (nctx > 64) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: at most 64 contexts");
+    for (int r = 1; r < nctx; ++r) {
+        if (!ctxs[r]) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: context of rank " + std::to_string(r) + " is null");
+        for (int q = 0; q < r; ++q) {
+            if (ctxs[q] == ctxs[r]) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: ranks " + std::to_string(q) + " and " + std::to_string(r) + " are the same context");
+            if (ctxs[q]->device == ctxs[r]->device)
+                FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: ranks " + std::to_string(q) + " and " + std::to_string(r) + " are both on device " + std::to_string(ctxs[r]->device));
+        }
+    }
+    if (ctx->ncart == 0 || ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct_group: basis and transform must be set first");
+    for (int r = 0; r < nctx; ++r) {
+        const tuna_ctx* c = ctxs[r];
+        if (c->ncart != ctx->ncart || c->nbf != ctx->nbf || c->basis_sum != ctx->basis_sum || c->U_sum != ctx->U_sum || c->direct_engine != ctx->direct_engine)
+            FAIL(TUNA_ERR_STATE, "tuna_jk_direct_group: rank " + std::to_string(r) + " holds a different basis or transform than rank 0");
+        if (c->shard_rank != r || c->shard_n != nctx)
+            FAIL(TUNA_ERR_STATE, "tuna_jk_direct_group: rank " + std::to_string(r) + " is sharded as (" + std::to_string(c->shard_rank) + ", " +
+                                 std::to_string(c->shard_n) + "), expected (" + std::to_string(r) + ", " + std::to_string(nctx) + ")");
+    }
+    return TUNA_OK;
+}
+
+// One rank's accumulate half, enqueued from its own host thread; a peer then records ev_group for ctxs[0] to wait on.
+static int group_accumulate(tuna_ctx* ctx, int nD, const double* dP, double tau, bool peer) try {
+    CK(cudaSetDevice(ctx->device));
+    if (int rc = jk_direct_accumulate(ctx, nD, dP, tau)) return rc;
+    if (peer) CK(cudaEventRecord(ctx->ev_group, ctx->stream));
+    return TUNA_OK;
+} TUNA_CATCH
+
+// dP, dJ, dK on ctxs[0]'s device; group_check has passed and every rank's dens_bound is set.
+static int jk_direct_group_core(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, unsigned anti_mask, double* dJ, double* dK, double tau) {
+    tuna_ctx* ctx = ctxs[0];
+    if (nctx == 1) return jk_direct_core(ctx, nD, dP, anti_mask, dJ, dK, tau);
+    if (nD <= 0 || nD > 16 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: bad arguments (1 <= nD <= 16)");
+    const int nc = ctx->ncart, nb = ctx->nbf, npeer = nctx - 1;
+    const bool fixed = ctx->direct_engine == 1 && ctx->ss.ok;
+    const int per = direct_pass_densities(ctx, nD);
+    const size_t nn = (size_t)nb * nb;
+    int rc;
+    for (int d0 = 0; d0 < nD; d0 += per) {
+        const int nd = std::min(per, nD - d0);
+        const size_t nacc = (size_t)nd * nc * nc, words = fixed ? 4 * nacc : 2 * nacc;     // one rank's accumulators
+        const double* P0 = dP + d0 * nn;
+        // 1. the pass's densities to every peer, after whatever produced them on ctxs[0]'s stream
+        CK(cudaEventRecord(ctx->ev_group, ctx->stream));
+        for (int r = 1; r < nctx; ++r) {
+            tuna_ctx* c = ctxs[r];
+            const unsigned long long bit = 1ull << (c->device & 63);
+            if (!(ctx->peers_tried & bit)) {      // direct peer copies where the link allows them; without, the copies go through the host
+                int ab = 0, ba = 0;
+                CK(cudaDeviceCanAccessPeer(&ab, ctx->device, c->device));
+                CK(cudaDeviceCanAccessPeer(&ba, c->device, ctx->device));
+                if (ab && ba) {
+                    CK(cudaSetDevice(ctx->device));
+                    cudaDeviceEnablePeerAccess(c->device, 0);      // "already enabled" (e.g. by torch) or a refusal only costs speed
+                    cudaGetLastError();
+                    CK(cudaSetDevice(c->device));
+                    cudaDeviceEnablePeerAccess(ctx->device, 0);
+                    cudaGetLastError();
+                }
+                ctx->peers_tried |= bit;
+            }
+            CK(cudaSetDevice(c->device));
+            if ((rc = ensure_mats(c, nd, nb, nc))) { ctx->err = "rank " + std::to_string(r) + ": " + c->err; return rc; }
+            CK(cudaStreamWaitEvent(c->stream, ctx->ev_group, 0));
+            CK(cudaMemcpyPeerAsync(c->d_P, c->device, P0, ctx->device, (size_t)nd * nn * sizeof(double), c->stream));
+        }
+        // 2. accumulate on every rank, enqueued from one host thread per device (all joined here)
+        std::vector<int> rcs(nctx, TUNA_OK);
+        {
+            std::vector<std::thread> threads;
+            try {
+                for (int r = 1; r < nctx; ++r)
+                    threads.emplace_back([&rcs, ctxs, r, nd, tau] { rcs[r] = group_accumulate(ctxs[r], nd, ctxs[r]->d_P, tau, true); });
+            } catch (const std::exception& e) {
+                for (auto& t : threads) t.join();
+                FAIL(TUNA_ERR_STATE, std::string("tuna_jk_direct_group: cannot start a host thread: ") + e.what());
+            }
+            rcs[0] = group_accumulate(ctx, nd, P0, tau, false);
+            for (auto& t : threads) t.join();
+        }
+        for (int r = 0; r < nctx; ++r)
+            if (rcs[r]) {
+                if (r > 0) ctx->err = "rank " + std::to_string(r) + ": " + ctxs[r]->err;
+                return rcs[r];
+            }
+        CK(cudaSetDevice(ctx->device));
+        // 3. pull every peer's accumulators into the staging buffer once its accumulate is done (one auxiliary stream per peer)
+        if (ctx->cap_peer < npeer * words) {
+            CK(cudaStreamSynchronize(ctx->stream));
+            ctx->cap_peer = 0;
+            if ((rc = dev_alloc(ctx, &ctx->d_peer, npeer * words))) return rc;
+            ctx->cap_peer = npeer * words;
+        }
+        for (int r = 1; r < nctx; ++r) CK(cudaStreamWaitEvent(ctx->stream, ctxs[r]->ev_group, 0));
+        CK(cudaEventRecord(ctx->ev[6][0], ctx->stream));
+        for (int r = 1; r < nctx; ++r) {
+            const tuna_ctx* c = ctxs[r];
+            cudaStream_t st = ctx->aux[(r - 1) % tuna_ctx::NAUX];
+            cudaEvent_t done = ctx->ev_join[(r - 1) % tuna_ctx::NAUX];
+            long long* dst = ctx->d_peer + (size_t)(r - 1) * words;
+            CK(cudaStreamWaitEvent(st, ctx->ev[6][0], 0));
+            if (fixed) {
+                CK(cudaMemcpyPeerAsync(dst, ctx->device, c->d_fix, c->device, words * sizeof(long long), st));
+            } else {
+                CK(cudaMemcpyPeerAsync(dst, ctx->device, c->d_Jc, c->device, nacc * sizeof(double), st));
+                CK(cudaMemcpyPeerAsync(dst + nacc, ctx->device, c->d_Kc, c->device, nacc * sizeof(double), st));
+            }
+            CK(cudaEventRecord(done, st));
+            CK(cudaStreamWaitEvent(ctx->stream, done, 0));
+        }
+        // 6. (enqueued now) no peer overwrites its accumulators in a later pass or call before they are pulled
+        CK(cudaEventRecord(ctx->ev_group, ctx->stream));
+        for (int r = 1; r < nctx; ++r) {
+            CK(cudaSetDevice(ctxs[r]->device));
+            CK(cudaStreamWaitEvent(ctxs[r]->stream, ctx->ev_group, 0));
+        }
+        CK(cudaSetDevice(ctx->device));
+        // 4. sum into ctxs[0]'s accumulators, 5. finish there
+        if (fixed) {
+            k_fix_reduce<<<grid_for(ctx, (int64_t)words, 256, 8), 256, 0, ctx->stream>>>(reinterpret_cast<unsigned long long*>(ctx->d_fix),
+                reinterpret_cast<const unsigned long long*>(ctx->d_peer), words, words, npeer);
+        } else {
+            const double* stage = reinterpret_cast<const double*>(ctx->d_peer);
+            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Jc, stage, nacc, words, npeer);
+            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Kc, stage + nacc, nacc, words, npeer);
+            ctx->launches++;
+        }
+        ctx->launches++;
+        CK(cudaGetLastError());
+        if ((rc = jk_direct_finish(ctx, nd, (anti_mask >> d0) & ((1u << nd) - 1u), dJ ? dJ + d0 * nn : nullptr, dK ? dK + d0 * nn : nullptr))) return rc;
+        CK(cudaEventRecord(ctx->ev[6][1], ctx->stream));
+    }
     return TUNA_OK;
 }
 
@@ -2524,54 +2765,39 @@ int tuna_jk_direct(tuna_ctx* ctx, int nD, const double* P, double* J, double* K,
     if (ctx->ncart == 0 || ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct: basis and transform must be set first");
     if (nD <= 0 || nD > 8 || !P) FAIL(TUNA_ERR_ARG, "tuna_jk_direct: bad arguments (1 <= nD <= 8)");
     CK(cudaSetDevice(ctx->device));
-    const int nb = ctx->nbf;
-    const size_t nn = (size_t)nb * nb;
-    // A general P splits into symmetric S and antisymmetric A parts: J[P] = J[S], K[P] = K[S] + K[A] with K[A] antisymmetric.
-    // SCF densities are symmetric to round-off (reference guess densities are not always: asymmetry ~1e-8 was observed).
-    double pmax = 0.0, amax = 0.0;
-    for (int d = 0; d < nD; ++d)
-        for (int i = 0; i < nb; ++i)
-            for (int j = 0; j <= i; ++j) {
-                const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
-                pmax = std::max(pmax, std::max(std::fabs(x), std::fabs(y)));
-                amax = std::max(amax, std::fabs(x - y));
-            }
-    const bool general = amax > 1e-15 * pmax;
-    ctx->dens_bound = std::max(1e3, 1e3 * pmax);          // static pre-screening stays below the device's exact density-weighted test
-    const int nDrun = general ? 2 * nD : nD;
-    int rc;
-    if ((rc = ensure_mats(ctx, nDrun, nb, ctx->ncart))) return rc;
-    const size_t bytes = (size_t)nDrun * nn * sizeof(double);
-    double* hP = ctx->h_pin;
-    double* hJ = hP + (size_t)nDrun * nn;
-    double* hK = hJ + (size_t)nDrun * nn;
-    unsigned anti_mask = 0;
-    if (!general) {
-        std::memcpy(hP, P, bytes);
-    } else {
-        for (int d = 0; d < nD; ++d) {
-            anti_mask |= 1u << (nD + d);
-            for (int i = 0; i < nb; ++i)
-                for (int j = 0; j < nb; ++j) {
-                    const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
-                    hP[d * nn + (size_t)i * nb + j] = 0.5 * (x + y);
-                    hP[(nD + d) * nn + (size_t)i * nb + j] = 0.5 * (x - y);
-                }
-        }
-    }
-    CK(cudaMemcpyAsync(ctx->d_P, hP, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    int rc, nDrun;
+    unsigned anti_mask;
+    if ((rc = stage_host_density(ctx, nD, P, &nDrun, &anti_mask))) return rc;
+    CK(cudaMemcpyAsync(ctx->d_P, ctx->h_pin, (size_t)nDrun * ctx->nbf * ctx->nbf * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     if ((rc = jk_direct_core(ctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J : nullptr, K ? ctx->d_K : nullptr, tau))) return rc;
-    if (J) CK(cudaMemcpyAsync(hJ, ctx->d_J, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    if (K) CK(cudaMemcpyAsync(hK, ctx->d_K, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (J) std::memcpy(J, hJ, (size_t)nD * nn * sizeof(double));
-    if (K) {
-        std::memcpy(K, hK, (size_t)nD * nn * sizeof(double));
-        if (general)
-            for (size_t x = 0; x < (size_t)nD * nn; ++x) K[x] += hK[(size_t)nD * nn + x];
-    }
-    return TUNA_OK;
+    return unstage_host_results(ctx, nD, nDrun, J, K);
 } TUNA_CATCH
+
+int tuna_jk_direct_group_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau) {
+    tuna_ctx* ctx = (ctxs && nctx >= 1) ? ctxs[0] : nullptr;
+    try {
+        if (int rc = group_check(ctxs, nctx)) return rc;
+        CK(cudaSetDevice(ctx->device));
+        for (int r = 1; r < nctx; ++r) ctxs[r]->dens_bound = ctx->dens_bound;
+        return jk_direct_group_core(ctxs, nctx, nD, dP, 0u, dJ, dK, tau);
+    } TUNA_CATCH
+}
+
+int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* P, double* J, double* K, double tau) {
+    tuna_ctx* ctx = (ctxs && nctx >= 1) ? ctxs[0] : nullptr;
+    try {
+        int rc, nDrun;
+        if ((rc = group_check(ctxs, nctx))) return rc;
+        if (nD <= 0 || nD > 8 || !P) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group: bad arguments (1 <= nD <= 8)");
+        CK(cudaSetDevice(ctx->device));
+        unsigned anti_mask;
+        if ((rc = stage_host_density(ctx, nD, P, &nDrun, &anti_mask))) return rc;
+        for (int r = 1; r < nctx; ++r) ctxs[r]->dens_bound = ctx->dens_bound;
+        CK(cudaMemcpyAsync(ctx->d_P, ctx->h_pin, (size_t)nDrun * ctx->nbf * ctx->nbf * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        if ((rc = jk_direct_group_core(ctxs, nctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J : nullptr, K ? ctx->d_K : nullptr, tau))) return rc;
+        return unstage_host_results(ctx, nD, nDrun, J, K);
+    } TUNA_CATCH
+}
 
 int tuna_get_counts(const tuna_ctx* c, int64_t counts[8]) {
     if (!c || !counts) return TUNA_ERR_ARG;
@@ -2592,7 +2818,7 @@ int tuna_get_counts(const tuna_ctx* c, int64_t counts[8]) {
 }
 
 int tuna_last_kernel_ms(tuna_ctx* ctx, int which, float* ms) {
-    if (!ctx || !ms || which < 0 || which > 5) return TUNA_ERR_ARG;
+    if (!ctx || !ms || which < 0 || which > 6) return TUNA_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaEventElapsedTime(ms, ctx->ev[which][0], ctx->ev[which][1]));

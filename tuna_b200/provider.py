@@ -28,17 +28,61 @@ from .basis import flatten
 DEFAULT_TAU = float(os.environ.get("TUNA_B200_TAU", "1e-16"))      # Schwarz threshold of direct mode (SURVEY.md 8d)
 _settings = {"mode": os.environ.get("TUNA_B200_MODE", "auto"), "device": int(os.environ.get("TUNA_B200_DEVICE", "0")),
              "stored_fraction": 0.40, "tau": DEFAULT_TAU}
+_devices = None      # devices of direct J/K (None: _settings["device"] alone); "all" = every visible device, resolved on first use
 
 
-def configure(mode=None, device=None, tau=None, stored_fraction=None):
+def _parse_devices(spec):
+    """'all', a comma list '0,1,3' or a sequence of ordinals -> 'all' or a list of distinct non-negative ints."""
+    if isinstance(spec, str):
+        if spec.strip().lower() == "all":
+            return "all"
+        try:
+            spec = [int(x) for x in spec.split(",") if x.strip()]
+        except ValueError:
+            raise _lib.error_class(f"tuna_b200: devices must be 'all' or a comma list of ordinals, got {spec!r}") from None
+    devices = [int(d) for d in spec]
+    if not devices or len(set(devices)) != len(devices) or min(devices) < 0:
+        raise _lib.error_class(f"tuna_b200: devices must be distinct non-negative ordinals, got {devices}")
+    return devices
+
+
+def _set_devices(spec):
+    global _devices
+    _devices = _parse_devices(spec)
+    _settings["device"] = 0 if _devices == "all" else _devices[0]
+
+
+def configured_devices():
+    """The devices direct J/K runs on; the first is the primary device (one-electron integrals, stored mode, the dense fill)."""
+    global _devices
+    if _devices == "all":
+        import torch  # plumbing only: the number of visible devices
+        n = torch.cuda.device_count()
+        if n < 1:
+            raise _lib.error_class("tuna_b200: devices='all' but no CUDA device is visible")
+        _devices = list(range(n))
+    return list(_devices) if _devices is not None else [_settings["device"]]
+
+
+if os.environ.get("TUNA_B200_DEVICES", "").strip():
+    _set_devices(os.environ["TUNA_B200_DEVICES"])
+
+
+def configure(mode=None, device=None, tau=None, stored_fraction=None, devices=None):
     """mode: 'stored' (dense tensor on the device), 'direct' (integral-driven J/K) or 'auto' (stored when
-    8*ncart^4 bytes fit in `stored_fraction` of free device memory or a post-HF consumer needs the tensor)."""
+    8*ncart^4 bytes fit in `stored_fraction` of free device memory or a post-HF consumer needs the tensor).
+    devices: 'all' or a list of ordinals (or a comma list); direct-mode J/K of one Fock build is spread over all of them
+    (DeviceGroup), everything else runs on devices[0].  device=d is devices=[d]."""
     if mode is not None:
         if mode not in ("stored", "direct", "auto"):
             raise _lib.error_class(f"tuna_b200: unknown mode {mode!r}")
         _settings["mode"] = mode
+    if device is not None and devices is not None:
+        raise _lib.error_class("tuna_b200: give either device or devices")
     if device is not None:
-        _settings["device"] = int(device)
+        _set_devices([device])
+    if devices is not None:
+        _set_devices(devices)
     if tau is not None:
         _settings["tau"] = float(tau)
     if stored_fraction is not None:
@@ -47,7 +91,7 @@ def configure(mode=None, device=None, tau=None, stored_fraction=None):
 
 def _free_device_bytes():
     import torch  # plumbing only: device memory query
-    free, _ = torch.cuda.mem_get_info(_settings["device"])
+    free, _ = torch.cuda.mem_get_info(configured_devices()[0])
     return free
 
 
@@ -65,6 +109,7 @@ class ERIHandle:
         self.ctx, self.n, self.basis_kind, self.mode = ctx, int(n), basis_kind, mode
         self._host = None
         self._jk_cache = []     # [(P, J, K)] most recent first
+        self._group = None      # direct mode over several devices: DeviceGroup built on the first J/K call
 
     shape = property(lambda self: (self.n,) * 4)
     ndim = 4
@@ -348,6 +393,15 @@ def coulomb_and_exchange(P, ERI_AO, want_j=True, want_k=True):
         return h.ctx.jk_stored(P, want_j, want_k)
     # any real P: the library splits a non-symmetric density into its symmetric and antisymmetric parts (K[P] = K[S] + K[A] with
     # K[A] antisymmetric, J[P] = J[S]); the reference's guess densities are asymmetric at the 1e-8 level
+    devices = configured_devices()
+    if len(devices) > 1:
+        if h._group is None or h._group.devices != devices:
+            # the handle's own context stays unsharded (dense fill on demand, single integrals, Schwarz factors)
+            group = _lib.DeviceGroup(devices)
+            group.set_basis(*h.ctx.basis_flat)
+            group.set_transform(h.ctx.U)
+            h._group = group
+        return h._group.jk_direct(P, _settings["tau"], want_j, want_k)
     return h.ctx.jk_direct(P, _settings["tau"], want_j, want_k)
 
 
