@@ -5,7 +5,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "tuna_b200.cu")
-DEPS = [SRC, os.path.join(HERE, "csrc", "eri_core.cuh"), os.path.join(HERE, "csrc", "pairtable.hpp"),
+DEPS = [SRC, os.path.join(HERE, "csrc", "devbuf.hpp"), os.path.join(HERE, "csrc", "eri_core.cuh"), os.path.join(HERE, "csrc", "pairtable.hpp"),
         os.path.join(HERE, "csrc", "shell_jk.cuh"), os.path.join(HERE, "csrc", "shell_host.hpp"), os.path.join(HERE, "csrc", "shell4.cuh"), os.path.join(HERE, "csrc", "shell4_host.hpp"), os.path.join(HERE, "csrc", "mo_transform.cuh"), os.path.join(HERE, "csrc", "oneel_core.cuh"), os.path.join(os.path.dirname(HERE), "include", "tuna_b200.h")]
 OUT = os.environ.get("TUNA_B200_LIB") or os.path.join(HERE, "libtuna_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "../../include/tuna_b200.h"
+#include "devbuf.hpp"
 #include "eri_core.cuh"
 #include "pairtable.hpp"
 #include "shell_host.hpp"
@@ -42,9 +43,8 @@ using namespace tuna;
 // ------------------------------------------------------------------------------------------------
 struct CsrDev {
     int rows = 0, cols = 0;
-    int* rowptr = nullptr;
-    int* col = nullptr;
-    double* val = nullptr;
+    DevBuf<int> rowptr, col;
+    DevBuf<double> val;
 };
 
 struct tuna_ctx {
@@ -54,18 +54,17 @@ struct tuna_ctx {
     int64_t launches = 0;
     int sm_count = 148;
 
-    double* d_boys = nullptr;
-    double* d_herm = nullptr;
+    DevBuf<double> d_boys, d_herm;
 
     // basis + pair table
     HostBasis hb;
     PairTable pt;
     bool pairs_ready = false;         // the AO-pair table is built on first use by an ERI / J/K call (one-electron integrals do not need it)
     int ncart = 0;
-    int* d_pi = nullptr; int* d_pj = nullptr; int* d_cls = nullptr; int* d_npp = nullptr;
-    int64_t* d_ppoff = nullptr;
-    double* d_pp = nullptr;
-    double* d_Q = nullptr;            // Schwarz factor per sorted pair (lazy)
+    DevBuf<int> d_pi, d_pj, d_cls, d_npp;
+    DevBuf<int64_t> d_ppoff;
+    DevBuf<double> d_pp;
+    DevBuf<double> d_Q;               // Schwarz factor per sorted pair (lazy)
     int64_t task_begin[5] = {0, 0, 0, 0, 0};
     int64_t n_unique = 0, n_surviving = 0, n_primq = 0, n_eval_last = 0;
     double alg_eri_flops = 0, alg_digest_flops = 0;
@@ -76,52 +75,50 @@ struct tuna_ctx {
     CsrDev U, Ut;
 
     // dense tensors
-    double* d_eri_cart = nullptr;
-    double* d_eri_sph = nullptr;      // "stored" tensor of dimension n_stored
+    DevBuf<double> d_eri_cart;
+    DevBuf<double> d_eri_sph;         // "stored" tensor of dimension n_stored
     int n_stored = 0;
     bool eri_pair_sym = false;        // (il|kj) == (kj|il) holds for the stored tensor: the symmetric streaming J/K kernel may be used
 
     // J/K workspaces
-    double* d_P = nullptr; double* d_J = nullptr; double* d_K = nullptr;   // nD * n^2 staging (spherical)
-    double* d_Pc = nullptr; double* d_Jc = nullptr; double* d_Kc = nullptr; double* d_tmp = nullptr;  // Cartesian
-    double* d_Kpart = nullptr;
-    double* d_fnorm = nullptr;        // per-component norms (shell engine fill mode)
-    size_t cap_mat = 0, cap_cart = 0, cap_kpart = 0;
-    double* h_pin = nullptr; size_t cap_pin = 0;
-    unsigned long long* d_scalars = nullptr;   // [0] max|P| bits, [1] evaluated-quartet counter
+    DevBuf<double> d_P, d_J, d_K;                  // nD * n^2 staging (spherical)
+    DevBuf<double> d_Pc, d_Jc, d_Kc, d_tmp;        // Cartesian
+    DevBuf<double> d_Kpart;
+    DevBuf<double> d_fnorm;           // per-component norms (shell engine fill mode)
+    PinnedBuf<double> h_pin;
+    DevBuf<unsigned long long> d_scalars;      // [0] max|P| bits, [1] evaluated-quartet counter
 
     int shard_rank = 0, shard_n = 1;
     cudaEvent_t ev[7][2] = {};
     uint64_t basis_sum = 0, U_sum = 0;     // checksums of the arrays given to tuna_set_basis / tuna_set_transform (tuna_jk_direct_group)
 
     // AO -> MO four-index transformation (mo_transform.cuh): two ping-pong work buffers, grown on demand
-    double* d_mo_ws[2] = {nullptr, nullptr};
-    size_t cap_mo[2] = {0, 0};
+    DevBuf<double> d_mo_ws[2];
 
     // shell-quartet engine (shell_jk.cuh)
     ShellTab stab;
     ShellSystem ss;
     bool shell_ready = false;
-    int* d_pairA = nullptr; int* d_pairB = nullptr; long long* d_pair_rec = nullptr; double* d_rec = nullptr; double* d_pairQ = nullptr;
-    int* d_sh_ao = nullptr; int* d_class_lists = nullptr; double* d_finv = nullptr;
-    double* d_eval = nullptr;
+    DevBuf<int> d_pairA, d_pairB; DevBuf<long long> d_pair_rec; DevBuf<double> d_rec, d_pairQ;
+    DevBuf<int> d_sh_ao, d_class_lists; DevBuf<double> d_finv;
+    DevBuf<double> d_eval;
     std::vector<size_t> class_list_off;
     static constexpr int NAUX = 16;
     int naux = 16;                   // streams in use (TUNA_B200_STREAMS, 1..16; measured: 16 helps the launch-bound small systems, neutral at nbf 800)
     cudaStream_t aux[NAUX] = {};     // class jobs of one build are independent (integer-atomic accumulation): launches are dealt round-robin to these streams
     cudaEvent_t ev_fork = nullptr, ev_join[NAUX] = {};
     // generation-4 shell engine (shell4.cuh): per-class tables and the job list; the pair data above is shared
-    struct ClassTab4Dev { Class4Host host; Class4Dev view; unsigned char* blob = nullptr; };
+    struct ClassTab4Dev { Class4Host host; Class4Dev view; DevBuf<unsigned char> blob; };
     struct Job4Host { Shell4Job job; int G = 1, threads = 128, gpc = 1, nb = 1; size_t smem = 0; double allowed = 0; bool own_launch = true; };
     std::map<int, ClassTab4Dev> class_tabs4;     // key La | Lb<<4 | Lc<<8 | Ld<<12 | nD<<16
     // job lists are cached per (threshold, densities per pass, rank count): a build with nD = 5 runs passes of 2, 2 and 1 densities, and
     // direct SCF alternates between thresholds rarely - none of that may rebuild lists or reallocate inside a Fock build
     struct Group4 { int G = 1, threads = 128, njobs = 0, job_off = 0, ctas_per_sm = 1; long long nunits = 0; size_t smem = 0;
-                    Shell4Job* d_jobs = nullptr; long long* d_unit_prefix = nullptr; };      // light jobs of one group size in one persistent launch
-    struct JobSet4 { double tau = -1.0, dens_bound = 0.0; int nD = 0, shard_n = 0; std::vector<Job4Host> jobs; std::vector<Group4> groups; long long* d_prefix = nullptr;
+                    DevBuf<Shell4Job> d_jobs; DevBuf<long long> d_unit_prefix; };      // light jobs of one group size in one persistent launch
+    struct JobSet4 { double tau = -1.0, dens_bound = 0.0; int nD = 0, shard_n = 0; std::vector<Job4Host> jobs; std::vector<Group4> groups; DevBuf<long long> d_prefix;
                      // fill job set (nD == 0): scratch rows of all work items, every job's descriptor and the prefix of (shell quartet, fill entry) counts for the scatter pass
-                     double* d_scratch = nullptr; Shell4Job* d_all_jobs = nullptr; long long* d_scatter_pre = nullptr; long long scatter_total = 0;
-                     int* d_fill_pairs = nullptr; };
+                     DevBuf<double> d_scratch; DevBuf<Shell4Job> d_all_jobs; DevBuf<long long> d_scatter_pre; long long scatter_total = 0;
+                     DevBuf<int> d_fill_pairs; };
     std::vector<JobSet4> jobsets4;
     int cur_jobset4 = -1;
     // The job lists are pre-screened on the host with tau / dens_bound, dens_bound = an upper bound of max |P| in the engine's working
@@ -129,8 +126,8 @@ struct tuna_ctx {
     // back-rotation of an h shell can amplify by ~1e2).  tuna_jk_direct raises it for larger host densities; callers of the _dev entry
     // point with larger densities scale them down (J and K are linear in P).
     double dens_bound = 1e3;
-    long long* d_fix = nullptr; size_t cap_fix = 0;      // reproducible accumulation: [J hi | J lo | K hi | K lo], nD * ncart^2 words each
-    long long* d_peer = nullptr; size_t cap_peer = 0;    // tuna_jk_direct_group on ctxs[0]: the other ranks' accumulators, pulled for k_fix_reduce
+    DevBuf<long long> d_fix;          // reproducible accumulation: [J hi | J lo | K hi | K lo], nD * ncart^2 words each
+    DevBuf<long long> d_peer;         // tuna_jk_direct_group on ctxs[0]: the other ranks' accumulators, pulled for k_fix_reduce
     cudaEvent_t ev_group = nullptr;                      // tuna_jk_direct_group: cross-device ordering (density ready / accumulate done / pulled)
     unsigned long long peers_tried = 0;                  // tuna_jk_direct_group on ctxs[0]: devices whose peer access with this one was requested
     CsrDev Uf, Uft;                 // U * diag(f) and its transpose: per-component norms folded into the rotation
@@ -148,6 +145,9 @@ struct tuna_ctx {
     } while (0)
 
 #define FAIL(code, msg) do { ctx->err = (msg); return (code); } while (0)
+
+// At least n elements in buf (DevBuf::grow); on failure ctx->err says why and the caller returns TUNA_ERR_NOMEM.
+#define GROW(buf, n) do { if (const int rc_ = (buf).grow((n), ctx->err)) return rc_; } while (0)
 
 // No exception may cross the C ABI (include/tuna_b200.h): every entry point that touches std containers is a function-try-block.
 #define TUNA_CATCH                                                                                                     \
@@ -180,27 +180,6 @@ static cudaError_t opt_in_smem(const tuna_ctx* ctx) {
     return e;
 }
 
-
-template <typename T>
-static int dev_alloc(tuna_ctx* ctx, T** p, size_t count) {
-    if (*p) { cudaFree(*p); *p = nullptr; }
-    if (count == 0) return TUNA_OK;
-    cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-    if (e != cudaSuccess) {
-        *p = nullptr;
-        cudaGetLastError();
-        ctx->err = "cudaMalloc of " + std::to_string(count * sizeof(T)) + " bytes failed: " + cudaGetErrorString(e);
-        return TUNA_ERR_NOMEM;
-    }
-    return TUNA_OK;
-}
-template <typename T>
-static void dev_free(T** p) { if (*p) { cudaFree(*p); *p = nullptr; } }
-static void free_jobset4(tuna_ctx::JobSet4& js) {
-    dev_free(&js.d_prefix); dev_free(&js.d_scratch); dev_free(&js.d_all_jobs); dev_free(&js.d_scatter_pre); dev_free(&js.d_fill_pairs);
-    for (auto& g : js.groups) { dev_free(&g.d_jobs); dev_free(&g.d_unit_prefix); }
-    js.groups.clear();
-}
 
 // ------------------------------------------------------------------------------------------------
 // device helpers
@@ -1077,10 +1056,9 @@ static int build_csr(tuna_ctx* ctx, CsrDev& M, int rows, int cols, const std::ve
         rowptr[r + 1] = (int)col.size();
     }
     M.rows = rows; M.cols = cols;
-    int rc;
-    if ((rc = dev_alloc(ctx, &M.rowptr, rowptr.size()))) return rc;
-    if ((rc = dev_alloc(ctx, &M.col, std::max<size_t>(col.size(), 1)))) return rc;
-    if ((rc = dev_alloc(ctx, &M.val, std::max<size_t>(val.size(), 1)))) return rc;
+    GROW(M.rowptr, rowptr.size());
+    GROW(M.col, std::max<size_t>(col.size(), 1));
+    GROW(M.val, std::max<size_t>(val.size(), 1));
     CK(cudaMemcpyAsync(M.rowptr, rowptr.data(), rowptr.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     if (!col.empty()) {
         CK(cudaMemcpyAsync(M.col, col.data(), col.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
@@ -1109,30 +1087,16 @@ static int rotate(tuna_ctx* ctx, const CsrDev& M, const double* in, double* out,
 }
 
 static int ensure_mats(tuna_ctx* ctx, int nD, int n, int ncart) {
-    int rc;
     const size_t need = (size_t)nD * n * n;
-    if (need > ctx->cap_mat) {
-        if ((rc = dev_alloc(ctx, &ctx->d_P, need))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_J, need))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_K, need))) return rc;
-        ctx->cap_mat = need;
-    }
+    GROW(ctx->d_P, need);
+    GROW(ctx->d_J, need);
+    GROW(ctx->d_K, need);
     const size_t needc = (size_t)nD * ncart * ncart;
-    if (ncart > 0 && needc > ctx->cap_cart) {
-        if ((rc = dev_alloc(ctx, &ctx->d_Pc, needc))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_Jc, needc))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_Kc, needc))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_tmp, needc))) return rc;
-        ctx->cap_cart = needc;
-    }
-    const size_t needp = 3 * need * sizeof(double);
-    if (needp > ctx->cap_pin) {
-        if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
-        ctx->h_pin = nullptr;
-        cudaError_t e = cudaMallocHost((void**)&ctx->h_pin, needp);
-        if (e != cudaSuccess) { cudaGetLastError(); ctx->cap_pin = 0; FAIL(TUNA_ERR_NOMEM, "pinned host allocation failed"); }
-        ctx->cap_pin = needp;
-    }
+    GROW(ctx->d_Pc, needc);
+    GROW(ctx->d_Jc, needc);
+    GROW(ctx->d_Kc, needc);
+    GROW(ctx->d_tmp, needc);
+    GROW(ctx->h_pin, 3 * need);
     return TUNA_OK;
 }
 
@@ -1146,13 +1110,12 @@ static int ensure_pairs(tuna_ctx* ctx) {
         FAIL(TUNA_ERR_NOMEM, "host allocation failed while building the pair table");
     }
     const PairTable& T = ctx->pt;
-    int rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_pi, (size_t)T.npair))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_pj, (size_t)T.npair))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_cls, (size_t)T.npair))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_npp, (size_t)T.npair))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_ppoff, (size_t)T.npair))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_pp, T.pp.size()))) return rc;
+    GROW(ctx->d_pi, (size_t)T.npair);
+    GROW(ctx->d_pj, (size_t)T.npair);
+    GROW(ctx->d_cls, (size_t)T.npair);
+    GROW(ctx->d_npp, (size_t)T.npair);
+    GROW(ctx->d_ppoff, (size_t)T.npair);
+    GROW(ctx->d_pp, T.pp.size());
     CK(cudaMemcpyAsync(ctx->d_pi, T.pi.data(), T.npair * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(ctx->d_pj, T.pj.data(), T.npair * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(ctx->d_cls, T.cls.data(), T.npair * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
@@ -1169,10 +1132,12 @@ static int ensure_schwarz(tuna_ctx* ctx) {
     int rc;
     if ((rc = ensure_pairs(ctx))) return rc;
     if (ctx->d_Q) return TUNA_OK;
-    if ((rc = dev_alloc(ctx, &ctx->d_Q, (size_t)ctx->pt.npair))) return rc;
-    k_schwarz<<<grid_for(ctx, ctx->pt.npair, 128, 16), 128, 0, ctx->stream>>>(table_dev(ctx), ctx->d_boys, ctx->d_herm, ctx->d_Q, ctx->pt.npair);
+    DevBuf<double> Q;         // published only once its kernel is launched: d_Q != nullptr means "filled"
+    GROW(Q, (size_t)ctx->pt.npair);
+    k_schwarz<<<grid_for(ctx, ctx->pt.npair, 128, 16), 128, 0, ctx->stream>>>(table_dev(ctx), ctx->d_boys, ctx->d_herm, Q, ctx->pt.npair);
     ctx->launches++;
     CK(cudaGetLastError());
+    ctx->d_Q = std::move(Q);
     return TUNA_OK;
 }
 
@@ -1206,10 +1171,9 @@ int tuna_ctx_create(int device, tuna_ctx** out) {
     std::vector<double> boys, herm;
     build_boys_table(boys);
     build_hermite_poly_table(herm);
-    int rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_boys, boys.size()))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_herm, herm.size()))) return rc;
-    if ((rc = dev_alloc(ctx, &ctx->d_scalars, (size_t)4))) return rc;
+    GROW(ctx->d_boys, boys.size());
+    GROW(ctx->d_herm, herm.size());
+    GROW(ctx->d_scalars, (size_t)4);
     CK(cudaMemcpy(ctx->d_boys, boys.data(), boys.size() * sizeof(double), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(ctx->d_herm, herm.data(), herm.size() * sizeof(double), cudaMemcpyHostToDevice));
     CK(cudaMemset(ctx->d_scalars, 0, 4 * sizeof(unsigned long long)));
@@ -1220,25 +1184,6 @@ int tuna_ctx_destroy(tuna_ctx* ctx) {
     if (!ctx) return TUNA_OK;
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    dev_free(&ctx->d_boys); dev_free(&ctx->d_herm); dev_free(&ctx->d_scalars);
-    dev_free(&ctx->d_pi); dev_free(&ctx->d_pj); dev_free(&ctx->d_cls); dev_free(&ctx->d_npp); dev_free(&ctx->d_ppoff); dev_free(&ctx->d_pp);
-    dev_free(&ctx->d_Q);
-    dev_free(&ctx->U.rowptr); dev_free(&ctx->U.col); dev_free(&ctx->U.val);
-    dev_free(&ctx->Ut.rowptr); dev_free(&ctx->Ut.col); dev_free(&ctx->Ut.val);
-    dev_free(&ctx->d_eri_cart); dev_free(&ctx->d_eri_sph);
-    dev_free(&ctx->d_P); dev_free(&ctx->d_J); dev_free(&ctx->d_K);
-    dev_free(&ctx->d_Pc); dev_free(&ctx->d_Jc); dev_free(&ctx->d_Kc); dev_free(&ctx->d_tmp); dev_free(&ctx->d_Kpart);
-    for (auto& kv : ctx->class_tabs4) dev_free(&kv.second.blob);
-    dev_free(&ctx->d_fix); dev_free(&ctx->d_peer);
-    dev_free(&ctx->d_pairA); dev_free(&ctx->d_pairB); dev_free(&ctx->d_pair_rec); dev_free(&ctx->d_rec);
-    dev_free(&ctx->d_pairQ); dev_free(&ctx->d_sh_ao); dev_free(&ctx->d_class_lists); dev_free(&ctx->d_finv);
-    for (auto& js : ctx->jobsets4) free_jobset4(js);
-    dev_free(&ctx->d_fnorm);
-    dev_free(&ctx->d_eval);
-    dev_free(&ctx->Uf.rowptr); dev_free(&ctx->Uf.col); dev_free(&ctx->Uf.val);
-    dev_free(&ctx->Uft.rowptr); dev_free(&ctx->Uft.col); dev_free(&ctx->Uft.val);
-    if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
-    dev_free(&ctx->d_mo_ws[0]); dev_free(&ctx->d_mo_ws[1]);
     for (int w = 0; w < 7; ++w)
         for (int s = 0; s < 2; ++s) if (ctx->ev[w][s]) cudaEventDestroy(ctx->ev[w][s]);
     if (ctx->ev_group) cudaEventDestroy(ctx->ev_group);
@@ -1296,14 +1241,13 @@ int tuna_set_basis(tuna_ctx* ctx, int ncart, const double* origins_z, const int3
     ctx->pairs_ready = false;
     ctx->pt = PairTable();
     ctx->n_unique = ctx->n_surviving = ctx->n_primq = 0;
-    dev_free(&ctx->d_Q);
-    dev_free(&ctx->d_eri_cart);
-    dev_free(&ctx->d_eri_sph);
+    ctx->d_Q.reset();
+    ctx->d_eri_cart.reset();
+    ctx->d_eri_sph.reset();
     ctx->n_stored = 0;
     ctx->nbf = 0;
     build_shell_tab(ctx->stab);
     ctx->shell_ready = false;
-    for (auto& js : ctx->jobsets4) free_jobset4(js);
     ctx->jobsets4.clear();
     ctx->cur_jobset4 = -1;
     detect_shells(ctx->hb, ctx->stab, ctx->ss);     // ss.ok == false -> direct mode uses the per-component kernel
@@ -1361,13 +1305,11 @@ int tuna_eri_fill_cart(tuna_ctx* ctx) try {
     bool engine = ctx->direct_engine == 1 && ctx->ss.ok && (ef ? atoi(ef) != 0 : contracted);
     // the dense tensor is never sharded (every rank holds all of it): the fill runs as rank 0 of 1, whatever tuna_set_shard said
     struct ShardGuard { tuna_ctx* c; int r, n; ~ShardGuard() { c->shard_rank = r; c->shard_n = n; } } guard{ctx, ctx->shard_rank, ctx->shard_n};
-    if ((rc = dev_alloc(ctx, &ctx->d_eri_cart, count))) return rc;
+    GROW(ctx->d_eri_cart, count);
     if (engine) {
         ctx->shard_rank = 0; ctx->shard_n = 1;
         rc = ensure_shell4(ctx, 0.0, 0);
-        if (rc) {       // drop the half-built fill job set; when only the scratch rows did not fit, the per-AO-quartet kernel (no scratch) takes over
-            if (!ctx->jobsets4.empty() && ctx->jobsets4.back().nD == 0) { free_jobset4(ctx->jobsets4.back()); ctx->jobsets4.pop_back(); }
-            ctx->cur_jobset4 = -1;
+        if (rc) {       // when only the scratch rows did not fit, the per-AO-quartet kernel (no scratch) takes over
             if (rc != TUNA_ERR_NOMEM) return rc;
             engine = false;
         }
@@ -1393,7 +1335,6 @@ int tuna_eri_fill_cart(tuna_ctx* ctx) try {
     CK(cudaEventRecord(ctx->ev[0][1], ctx->stream));
     if (engine) {       // the scratch rows (the unique integrals once per primitive chunk) are only needed until the scatter pass has run
         CK(cudaStreamSynchronize(ctx->stream));
-        free_jobset4(ctx->jobsets4[ctx->cur_jobset4]);
         ctx->jobsets4.erase(ctx->jobsets4.begin() + ctx->cur_jobset4);
         ctx->cur_jobset4 = -1;
     }
@@ -1406,18 +1347,16 @@ int tuna_eri_cart_to_sph(tuna_ctx* ctx, int keep_cart) try {
     if (ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_eri_cart_to_sph: call tuna_set_transform first");
     CK(cudaSetDevice(ctx->device));
     const int64_t nc = ctx->ncart, nb = ctx->nbf;
-    double* t1 = nullptr; double* t2 = nullptr;
     int rc;
-    dev_free(&ctx->d_eri_sph);
+    ctx->d_eri_sph.reset();
     ctx->n_stored = 0;
     CK(cudaEventRecord(ctx->ev[1][0], ctx->stream));
     if (ctx->U_identity) {   // CARTHARM: no rotation (tuna_kernel.py:481-483)
         if (keep_cart) {
-            if ((rc = dev_alloc(ctx, &ctx->d_eri_sph, (size_t)(nc * nc * nc * nc)))) return rc;
+            GROW(ctx->d_eri_sph, (size_t)(nc * nc * nc * nc));
             CK(cudaMemcpyAsync(ctx->d_eri_sph, ctx->d_eri_cart, (size_t)(nc * nc * nc * nc) * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
         } else {
-            ctx->d_eri_sph = ctx->d_eri_cart;
-            ctx->d_eri_cart = nullptr;
+            ctx->d_eri_sph = std::move(ctx->d_eri_cart);
         }
         CK(cudaEventRecord(ctx->ev[1][1], ctx->stream));
         ctx->n_stored = (int)nc;
@@ -1426,10 +1365,11 @@ int tuna_eri_cart_to_sph(tuna_ctx* ctx, int keep_cart) try {
     }
     // Four single-index passes ping-ponging between two work buffers; every allocation happens before the timed region and nothing
     // synchronises inside it (stream order is enough).  Without keep_cart the Cartesian tensor's own storage is the second buffer.
-    if ((rc = dev_alloc(ctx, &t1, (size_t)(nb * nc * nc * nc)))) return rc;
-    if (keep_cart && (rc = dev_alloc(ctx, &t2, (size_t)(nb * nb * nc * nc)))) { dev_free(&t1); return rc; }
-    if ((rc = dev_alloc(ctx, &ctx->d_eri_sph, (size_t)(nb * nb * nb * nb)))) { dev_free(&t1); dev_free(&t2); return rc; }
-    double* w2 = keep_cart ? t2 : ctx->d_eri_cart;
+    DevBuf<double> t1, t2;
+    GROW(t1, (size_t)(nb * nc * nc * nc));
+    if (keep_cart) GROW(t2, (size_t)(nb * nb * nc * nc));
+    GROW(ctx->d_eri_sph, (size_t)(nb * nb * nb * nb));
+    double* w2 = keep_cart ? t2.get() : ctx->d_eri_cart.get();
     CK(cudaEventRecord(ctx->ev[1][0], ctx->stream));
     rc = rotate(ctx, ctx->U, ctx->d_eri_cart, t1, 1, nc * nc * nc);
     if (!rc) rc = rotate(ctx, ctx->U, t1, w2, nb, nc * nc);
@@ -1437,9 +1377,8 @@ int tuna_eri_cart_to_sph(tuna_ctx* ctx, int keep_cart) try {
     if (!rc) rc = rotate(ctx, ctx->U, t1, ctx->d_eri_sph, nb * nb * nb, 1);
     if (!rc) { CK(cudaEventRecord(ctx->ev[1][1], ctx->stream)); }
     cudaStreamSynchronize(ctx->stream);
-    dev_free(&t1); dev_free(&t2);
-    if (!keep_cart) dev_free(&ctx->d_eri_cart);
-    if (rc) { dev_free(&ctx->d_eri_sph); return rc; }
+    if (!keep_cart) ctx->d_eri_cart.reset();
+    if (rc) { ctx->d_eri_sph.reset(); return rc; }
     ctx->n_stored = (int)nb;
     return check_pair_symmetry(ctx);
 } TUNA_CATCH
@@ -1459,9 +1398,9 @@ int tuna_eri_upload(tuna_ctx* ctx, int n, const double* host_in) try {
     if (!ctx || !host_in || n <= 0) return TUNA_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     const size_t count = (size_t)n * n * n * n;
-    int rc;
     ctx->n_stored = 0;
-    if ((rc = dev_alloc(ctx, &ctx->d_eri_sph, count))) return rc;
+    ctx->d_eri_sph.reset();
+    GROW(ctx->d_eri_sph, count);
     CK(cudaMemcpyAsync(ctx->d_eri_sph, host_in, count * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->n_stored = n;
@@ -1487,16 +1426,14 @@ int tuna_eri_single(tuna_ctx* ctx, int i, int j, int k, int l, double* out) try 
         for (int b = 0; b < B.nprim[j]; ++b, r += PP_DOUBLES) fill_prim_record(r, B, i, j, B.off[i] + a, B.off[j] + b, scratch);
     for (int a = 0; a < B.nprim[k]; ++a)
         for (int b = 0; b < B.nprim[l]; ++b, r += PP_DOUBLES) fill_prim_record(r, B, k, l, B.off[k] + a, B.off[l] + b, scratch);
-    double* d = nullptr;
-    int rc;
-    if ((rc = dev_alloc(ctx, &d, rec.size() + 1))) return rc;
+    DevBuf<double> d;
+    GROW(d, rec.size() + 1);
     CK(cudaMemcpyAsync(d + 1, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     k_eri_single<<<1, 32, 0, ctx->stream>>>(d + 1, nA, cA, d + 1 + (size_t)nA * PP_DOUBLES, nB, cB, ctx->d_boys, ctx->d_herm, d);
     ctx->launches++;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, d, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    dev_free(&d);
     return TUNA_OK;
 } TUNA_CATCH
 
@@ -1560,7 +1497,6 @@ static int jk_stored_sym(tuna_ctx* ctx, int nD, const double* dP, double* dJ, do
     const int grid = (int)std::min<long long>((long long)ctx->sm_count, (long long)nn);
     const int kslots = (int)((nn / grid + 1 + n - 1) / n) + 2;
     const int nslots = grid * kslots;
-    int rc;
     for (int d0 = 0; d0 < nD; d0 += nd_max) {
         const int nd = std::min(nd_max, nD - d0);
         const size_t fixed = ((size_t)nd * nn + (size_t)2 * nd * r * n) * sizeof(double) + 2 * 16 * sizeof(uint64_t) + 128;
@@ -1570,11 +1506,7 @@ static int jk_stored_sym(tuna_ctx* ctx, int nD, const double* dP, double* dJ, do
         const size_t smem = (size_t)nstage * tile_bytes + fixed;
         // workspace: Kslot rows | Krow tags | Jpart
         const size_t o_krow = (size_t)nslots * nd_max * n, o_jpart = o_krow + (size_t)(nslots + 1) / 2 + 2;
-        const size_t need = o_jpart + (size_t)grid * nd_max * nn;
-        if (need > ctx->cap_kpart) {
-            if ((rc = dev_alloc(ctx, &ctx->d_Kpart, need))) return rc;
-            ctx->cap_kpart = need;
-        }
+        GROW(ctx->d_Kpart, o_jpart + (size_t)grid * nd_max * nn);
         double* Kslot = ctx->d_Kpart;
         int* Krow = reinterpret_cast<int*>(ctx->d_Kpart + o_krow);
         double* Jpart = ctx->d_Kpart + o_jpart;
@@ -1657,17 +1589,11 @@ extern "C" int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, doubl
         const int kslots = (int)((total / grid + 1 + n - 1) / n) + 2;
         const int nslots = grid * kslots;
         const size_t need_kpart = (size_t)nslots * 4 * n + (size_t)(nslots + 1) / 2 + 8;       // doubles: partial rows + row tags
-        if (dK && need_kpart > ctx->cap_kpart) {
-            if ((rc = dev_alloc(ctx, &ctx->d_Kpart, need_kpart))) return rc;
-            ctx->cap_kpart = need_kpart;
-        }
+        if (dK) GROW(ctx->d_Kpart, need_kpart);
         CK(cudaEventRecord(ctx->ev[2][0], ctx->stream));
         for (int d0 = 0; d0 < nD; d0 += 4) {
             const int nd = std::min(4, nD - d0);
-            if (!dK && need_kpart > ctx->cap_kpart) {      // K not requested: the kernel still needs scratch rows
-                if ((rc = dev_alloc(ctx, &ctx->d_Kpart, need_kpart))) return rc;
-                ctx->cap_kpart = need_kpart;
-            }
+            if (!dK) GROW(ctx->d_Kpart, need_kpart);      // K not requested: the kernel still needs scratch rows
             double* Kslot = ctx->d_Kpart;
             int* Krow = reinterpret_cast<int*>(ctx->d_Kpart + (size_t)nslots * 4 * n);
             CK(cudaMemsetAsync(Krow, 0xFF, (size_t)nslots * sizeof(int), ctx->stream));
@@ -1699,10 +1625,7 @@ extern "C" int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, doubl
     const int nchunk = (n + lch - 1) / lch;
     const int nwarp = (threads + 31) / 32;
     const size_t need_kpart = (size_t)std::min(nD, 4) * n * nchunk * n;
-    if (dK && need_kpart > ctx->cap_kpart) {
-        if ((rc = dev_alloc(ctx, &ctx->d_Kpart, need_kpart))) return rc;
-        ctx->cap_kpart = need_kpart;
-    }
+    if (dK) GROW(ctx->d_Kpart, need_kpart);
     CK(cudaEventRecord(ctx->ev[2][0], ctx->stream));
     for (int d0 = 0; d0 < nD; d0 += 4) {
         const int nd = std::min(4, nD - d0);
@@ -1710,7 +1633,7 @@ extern "C" int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, doubl
         dim3 grid(nchunk, n);
         const double* P = dP + d0 * nn;
         double* J = dJ ? dJ + d0 * nn : nullptr;
-        double* Kp = dK ? ctx->d_Kpart : nullptr;
+        double* Kp = dK ? ctx->d_Kpart.get() : nullptr;
         switch (nd) {
             case 1: k_jk_stored<1><<<grid, threads, smem, ctx->stream>>>(ctx->d_eri_sph, P, J, Kp, n, r, lch, nchunk); break;
             case 2: k_jk_stored<2><<<grid, threads, smem, ctx->stream>>>(ctx->d_eri_sph, P, J, Kp, n, r, lch, nchunk); break;
@@ -1745,7 +1668,7 @@ int tuna_jk_stored(tuna_ctx* ctx, int nD, const double* P, double* J, double* K)
     double* hK = hJ + (size_t)nD * n * n;
     std::memcpy(hP, P, bytes);
     CK(cudaMemcpyAsync(ctx->d_P, hP, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    if ((rc = tuna_jk_stored_dev(ctx, nD, ctx->d_P, J ? ctx->d_J : nullptr, K ? ctx->d_K : nullptr))) return rc;
+    if ((rc = tuna_jk_stored_dev(ctx, nD, ctx->d_P, J ? ctx->d_J.get() : nullptr, K ? ctx->d_K.get() : nullptr))) return rc;
     if (J) CK(cudaMemcpyAsync(hJ, ctx->d_J, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     if (K) CK(cudaMemcpyAsync(hK, ctx->d_K, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -1789,13 +1712,10 @@ static int mo_transform_core(tuna_ctx* ctx, int n, const double* dT, int n1, con
     const size_t N = (size_t)n, N1 = (size_t)n1, N2 = (size_t)n2;
     const size_t s1 = N1 * N * N * N, s2 = N1 * N1 * N * N, s3 = N2 * N1 * N1 * N;
     const size_t need[2] = {std::max(s1, s3), s2};
-    int rc;
     for (int b = 0; b < 2; ++b)
-        if (ctx->cap_mo[b] < need[b]) {
-            ctx->cap_mo[b] = 0;
+        if (ctx->d_mo_ws[b].capacity() < need[b]) {
             CK(cudaStreamSynchronize(ctx->stream));
-            if ((rc = dev_alloc(ctx, &ctx->d_mo_ws[b], need[b]))) return rc;
-            ctx->cap_mo[b] = need[b];
+            GROW(ctx->d_mo_ws[b], need[b]);
         }
     double* A = ctx->d_mo_ws[0];
     double* B = ctx->d_mo_ws[1];
@@ -1831,28 +1751,17 @@ int tuna_eri_transform(tuna_ctx* ctx, int n, const double* eri_host, int n1, con
     const size_t n4 = (size_t)n * n * n * n, nout = (size_t)n1 * n1 * n2 * n2;
     if (!eri_host && (!ctx->d_eri_sph || ctx->n_stored != n))
         FAIL(TUNA_ERR_STATE, "tuna_eri_transform: no stored tensor of that dimension is resident and no host tensor was given");
-    double* dT = nullptr; double* dC = nullptr; double* dOut = nullptr;
-    int rc = TUNA_OK;
-    if (eri_host && (rc = dev_alloc(ctx, &dT, n4))) return rc;
-    if (!rc) rc = dev_alloc(ctx, &dC, (size_t)n * (n1 + n2));
-    if (!rc) rc = dev_alloc(ctx, &dOut, nout);
-    auto cleanup = [&]() { dev_free(&dT); dev_free(&dC); dev_free(&dOut); };
-    if (rc) { cleanup(); return rc; }
-    cudaError_t e = cudaSuccess;
-    if (eri_host) e = cudaMemcpyAsync(dT, eri_host, n4 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dC, C1, (size_t)n * n1 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dC + (size_t)n * n1, C2, (size_t)n * n2 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { cleanup(); ctx->err = std::string("tuna_eri_transform upload: ") + cudaGetErrorString(e); return TUNA_ERR_CUDA; }
-    rc = mo_transform_core(ctx, n, eri_host ? dT : ctx->d_eri_sph, n1, dC, n2, dC + (size_t)n * n1, so_layout, dOut);
-    if (!rc) {
-        e = cudaMemcpyAsync(out_host, dOut, nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) { ctx->err = std::string("tuna_eri_transform: ") + cudaGetErrorString(e); rc = TUNA_ERR_CUDA; }
-    } else {
-        cudaStreamSynchronize(ctx->stream);
-    }
-    cleanup();
-    return rc;
+    DevBuf<double> dT, dC, dOut;
+    if (eri_host) GROW(dT, n4);
+    GROW(dC, (size_t)n * (n1 + n2));
+    GROW(dOut, nout);
+    if (eri_host) CK(cudaMemcpyAsync(dT, eri_host, n4 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(dC, C1, (size_t)n * n1 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(dC + (size_t)n * n1, C2, (size_t)n * n2 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    if (int rc = mo_transform_core(ctx, n, eri_host ? dT : ctx->d_eri_sph, n1, dC, n2, dC + (size_t)n * n1, so_layout, dOut)) return rc;
+    CK(cudaMemcpyAsync(out_host, dOut, nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return TUNA_OK;
 } TUNA_CATCH
 
 int tuna_eri_transform_spin_blocked(tuna_ctx* ctx, int n1, const double* C1, int n2, const double* C2, int so_layout, double* out_host) try {
@@ -1862,27 +1771,18 @@ int tuna_eri_transform_spin_blocked(tuna_ctx* ctx, int n1, const double* C1, int
     CK(cudaSetDevice(ctx->device));
     const int n = ctx->n_stored, N = 2 * n;
     const size_t N4 = (size_t)N * N * N * N, nout = (size_t)n1 * n1 * n2 * n2;
-    double* dG = nullptr; double* dC = nullptr; double* dOut = nullptr;
-    int rc = dev_alloc(ctx, &dG, N4);
-    if (!rc) rc = dev_alloc(ctx, &dC, (size_t)N * (n1 + n2));
-    if (!rc) rc = dev_alloc(ctx, &dOut, nout);
-    auto cleanup = [&]() { dev_free(&dG); dev_free(&dC); dev_free(&dOut); };
-    if (rc) { cleanup(); return rc; }
-    cudaError_t e = cudaMemcpyAsync(dC, C1, (size_t)N * n1 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dC + (size_t)N * n1, C2, (size_t)N * n2 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { cleanup(); ctx->err = std::string("tuna_eri_transform_spin_blocked upload: ") + cudaGetErrorString(e); return TUNA_ERR_CUDA; }
+    DevBuf<double> dG, dC, dOut;
+    GROW(dG, N4);
+    GROW(dC, (size_t)N * (n1 + n2));
+    GROW(dOut, nout);
+    CK(cudaMemcpyAsync(dC, C1, (size_t)N * n1 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(dC + (size_t)N * n1, C2, (size_t)N * n2 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     k_spin_block<<<(unsigned)((size_t)N * N), 256, 0, ctx->stream>>>(ctx->d_eri_sph, dG, n);
     ctx->launches++;
-    rc = mo_transform_core(ctx, N, dG, n1, dC, n2, dC + (size_t)N * n1, so_layout, dOut);
-    if (!rc) {
-        e = cudaMemcpyAsync(out_host, dOut, nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) { ctx->err = std::string("tuna_eri_transform_spin_blocked: ") + cudaGetErrorString(e); rc = TUNA_ERR_CUDA; }
-    } else {
-        cudaStreamSynchronize(ctx->stream);
-    }
-    cleanup();
-    return rc;
+    if (int rc = mo_transform_core(ctx, N, dG, n1, dC, n2, dC + (size_t)N * n1, so_layout, dOut)) return rc;
+    CK(cudaMemcpyAsync(out_host, dOut, nout * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return TUNA_OK;
 } TUNA_CATCH
 
 }  // extern "C"
@@ -1891,16 +1791,18 @@ int tuna_eri_transform_spin_blocked(tuna_ctx* ctx, int n1, const double* C1, int
 // One-electron integrals (SURVEY.md 8f-3): overlap, kinetic, nuclear attraction, dipole, diagonal quadrupole
 // (tuna_integral.pyx:282-445) and the cross-basis overlap (:626-778); math in oneel_core.cuh
 // ------------------------------------------------------------------------------------------------
-struct BasisDev {
+struct BasisDev {       // kernel argument: a view of a BasisBuf
     int n = 0;
     double* oz = nullptr; int* lmn = nullptr; int* nprim = nullptr; int64_t* off = nullptr; double* exps = nullptr; double* ceff = nullptr;
 };
 
-static void basis_dev_free(BasisDev& B) {
-    dev_free(&B.oz); dev_free(&B.lmn); dev_free(&B.nprim); dev_free(&B.off); dev_free(&B.exps); dev_free(&B.ceff);
-}
+struct BasisBuf {
+    int n = 0;
+    DevBuf<double> oz; DevBuf<int> lmn, nprim; DevBuf<int64_t> off; DevBuf<double> exps, ceff;
+    BasisDev view() const { return BasisDev{n, oz, lmn, nprim, off, exps, ceff}; }
+};
 
-static int basis_dev_upload(tuna_ctx* ctx, BasisDev& B, int n, const double* oz, const int32_t* lmn, const int32_t* nprim, const int64_t* off,
+static int basis_dev_upload(tuna_ctx* ctx, BasisBuf& B, int n, const double* oz, const int32_t* lmn, const int32_t* nprim, const int64_t* off,
                             const double* exps, const double* ceff) {
     int64_t tot = 0;
     for (int i = 0; i < n; ++i) {
@@ -1910,10 +1812,12 @@ static int basis_dev_upload(tuna_ctx* ctx, BasisDev& B, int n, const double* oz,
         tot = std::max<int64_t>(tot, off[i] + nprim[i]);
     }
     B.n = n;
-    int rc;
-    if ((rc = dev_alloc(ctx, &B.oz, (size_t)n)) || (rc = dev_alloc(ctx, &B.lmn, (size_t)3 * n)) || (rc = dev_alloc(ctx, &B.nprim, (size_t)n)) ||
-        (rc = dev_alloc(ctx, &B.off, (size_t)n)) || (rc = dev_alloc(ctx, &B.exps, (size_t)tot)) || (rc = dev_alloc(ctx, &B.ceff, (size_t)tot)))
-        return rc;
+    GROW(B.oz, (size_t)n);
+    GROW(B.lmn, (size_t)3 * n);
+    GROW(B.nprim, (size_t)n);
+    GROW(B.off, (size_t)n);
+    GROW(B.exps, (size_t)tot);
+    GROW(B.ceff, (size_t)tot);
     CK(cudaMemcpyAsync(B.oz, oz, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(B.lmn, lmn, (size_t)3 * n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(B.nprim, nprim, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
@@ -1966,36 +1870,26 @@ int tuna_one_electron(tuna_ctx* ctx, int n_atoms, const double* atom_z, const do
     std::vector<double> at((size_t)2 * n_atoms + 3);
     for (int a = 0; a < n_atoms; ++a) { at[a] = atom_z[a]; at[n_atoms + a] = atom_charge[a]; }
     for (int c = 0; c < 3; ++c) at[2 * n_atoms + c] = dipole_origin[c];
-    BasisDev B;
-    double* d_at = nullptr; double* d_out = nullptr;
-    int rc = basis_dev_upload(ctx, B, n, H.oz.data(), lmn32.data(), np32.data(), H.off.data(), H.exps.data(), H.ceff.data());
-    if (!rc) rc = dev_alloc(ctx, &d_at, at.size());
-    if (!rc) rc = dev_alloc(ctx, &d_out, 9 * nn);
-    cudaError_t e = cudaSuccess;
-    if (!rc) {
-        e = cudaMemcpyAsync(d_at, at.data(), at.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaEventRecord(ctx->ev[5][0], ctx->stream);
-        if (e == cudaSuccess) {
-            k_one_electron<<<(unsigned)((nn + 127) / 128), 128, 0, ctx->stream>>>(B, n_atoms, d_at, ctx->d_boys, d_out);
-            ctx->launches++;
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(ctx->ev[5][1], ctx->stream);
-        // straight into the caller's buffers (page-locked when they come from the Python layer): no staging vector, no second copy
-        double* dst[5] = {S, T, V, D, Q};
-        const size_t cnt[5] = {nn, nn, nn, 3 * nn, 3 * nn};
-        size_t off = 0;
-        for (int k = 0; k < 5; ++k) {
-            if (e == cudaSuccess) e = cudaMemcpyAsync(dst[k], d_out + off, cnt[k] * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-            off += cnt[k];
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    } else {
-        cudaStreamSynchronize(ctx->stream);
+    BasisBuf B;
+    DevBuf<double> d_at, d_out;
+    if (int rc = basis_dev_upload(ctx, B, n, H.oz.data(), lmn32.data(), np32.data(), H.off.data(), H.exps.data(), H.ceff.data())) return rc;
+    GROW(d_at, at.size());
+    GROW(d_out, 9 * nn);
+    CK(cudaMemcpyAsync(d_at, at.data(), at.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaEventRecord(ctx->ev[5][0], ctx->stream));
+    k_one_electron<<<(unsigned)((nn + 127) / 128), 128, 0, ctx->stream>>>(B.view(), n_atoms, d_at, ctx->d_boys, d_out);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->ev[5][1], ctx->stream));
+    // straight into the caller's buffers (page-locked when they come from the Python layer): no staging vector, no second copy
+    double* dst[5] = {S, T, V, D, Q};
+    const size_t cnt[5] = {nn, nn, nn, 3 * nn, 3 * nn};
+    size_t off = 0;
+    for (int k = 0; k < 5; ++k) {
+        CK(cudaMemcpyAsync(dst[k], d_out + off, cnt[k] * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        off += cnt[k];
     }
-    basis_dev_free(B); dev_free(&d_at); dev_free(&d_out);
-    if (rc) return rc;
-    if (e != cudaSuccess) FAIL(TUNA_ERR_CUDA, std::string("tuna_one_electron: ") + cudaGetErrorString(e));
+    CK(cudaStreamSynchronize(ctx->stream));
     return TUNA_OK;
 } TUNA_CATCH
 
@@ -2006,25 +1900,18 @@ int tuna_cross_overlap(tuna_ctx* ctx, int n1, const double* oz1, const int32_t* 
     if (n1 <= 0 || n2 <= 0 || !oz1 || !lmn1 || !nprim1 || !off1 || !exps1 || !ceff1 || !oz2 || !lmn2 || !nprim2 || !off2 || !exps2 || !ceff2 || !S12)
         FAIL(TUNA_ERR_ARG, "tuna_cross_overlap: bad arguments");
     CK(cudaSetDevice(ctx->device));
-    BasisDev A, B;
-    double* d_out = nullptr;
+    BasisBuf A, B;
+    DevBuf<double> d_out;
     const size_t count = (size_t)n1 * n2;
-    int rc = basis_dev_upload(ctx, A, n1, oz1, lmn1, nprim1, off1, exps1, ceff1);
-    if (!rc) rc = basis_dev_upload(ctx, B, n2, oz2, lmn2, nprim2, off2, exps2, ceff2);
-    if (!rc) rc = dev_alloc(ctx, &d_out, count);
-    cudaError_t e = cudaSuccess;
-    if (!rc) {
-        k_cross_overlap<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(A, B, d_out);
-        ctx->launches++;
-        e = cudaGetLastError();
-        if (e == cudaSuccess) e = cudaMemcpyAsync(S12, d_out, count * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    } else {
-        cudaStreamSynchronize(ctx->stream);
-    }
-    basis_dev_free(A); basis_dev_free(B); dev_free(&d_out);
-    if (rc) return rc;
-    if (e != cudaSuccess) FAIL(TUNA_ERR_CUDA, std::string("tuna_cross_overlap: ") + cudaGetErrorString(e));
+    int rc;
+    if ((rc = basis_dev_upload(ctx, A, n1, oz1, lmn1, nprim1, off1, exps1, ceff1))) return rc;
+    if ((rc = basis_dev_upload(ctx, B, n2, oz2, lmn2, nprim2, off2, exps2, ceff2))) return rc;
+    GROW(d_out, count);
+    k_cross_overlap<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(A.view(), B.view(), d_out);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(S12, d_out, count * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return TUNA_OK;
 } TUNA_CATCH
 
@@ -2043,19 +1930,19 @@ static int ensure_shell_pairs(tuna_ctx* ctx) {
             build_shell_pairs(S, ctx->stab, ctx->pt, q, ctx->ncart);
         } catch (const std::bad_alloc&) { FAIL(TUNA_ERR_NOMEM, "host allocation failed while building shell pairs"); }
         const size_t np = S.pairA.size();
-        if ((rc = dev_alloc(ctx, &ctx->d_pairA, np))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_pairB, np))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_pair_rec, np))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_pairQ, np))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_rec, S.rec.size()))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_sh_ao, S.sh_ao.size()))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_finv, (size_t)ctx->ncart))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_fnorm, (size_t)ctx->ncart))) return rc;
-        if ((rc = dev_alloc(ctx, &ctx->d_eval, (size_t)1))) return rc;
+        GROW(ctx->d_pairA, np);
+        GROW(ctx->d_pairB, np);
+        GROW(ctx->d_pair_rec, np);
+        GROW(ctx->d_pairQ, np);
+        GROW(ctx->d_rec, S.rec.size());
+        GROW(ctx->d_sh_ao, S.sh_ao.size());
+        GROW(ctx->d_finv, (size_t)ctx->ncart);
+        GROW(ctx->d_fnorm, (size_t)ctx->ncart);
+        GROW(ctx->d_eval, (size_t)1);
         std::vector<int> lists;
         ctx->class_list_off.clear();
         for (auto& c : S.classes) { ctx->class_list_off.push_back(lists.size()); lists.insert(lists.end(), c.pairs.begin(), c.pairs.end()); }
-        if ((rc = dev_alloc(ctx, &ctx->d_class_lists, lists.size()))) return rc;
+        GROW(ctx->d_class_lists, lists.size());
         std::vector<double> finv(ctx->ncart);
         for (int i = 0; i < ctx->ncart; ++i) finv[i] = 1.0 / S.fnorm[i];
         CK(cudaMemcpyAsync(ctx->d_pairA, S.pairA.data(), np * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
@@ -2091,7 +1978,7 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     const int key = La | Lb << 4 | Lc << 8 | Ld << 12 | nD << 16;
     auto it = ctx->class_tabs4.find(key);
     if (it != ctx->class_tabs4.end()) { *out = &it->second; return TUNA_OK; }
-    tuna_ctx::ClassTab4Dev& E = ctx->class_tabs4[key];
+    tuna_ctx::ClassTab4Dev E;         // cached only once its blob is uploaded and its view set
     {
         const char* eb = getenv("TUNA_B200_IT_BUDGET");
         const char* es = getenv("TUNA_B200_S_BUDGET");
@@ -2140,8 +2027,7 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     const size_t o_fl = add(C.fill.data(), C.fill.size() * 4), o_f0 = add(C.chunk_f0.data(), C.chunk_f0.size() * 4), o_fp = add(C.fperm.data(), C.fperm.size() * 4);
     std::vector<unsigned char> host(total, 0);
     for (const Piece& p : pieces) if (p.bytes) std::memcpy(host.data() + p.off, p.src, p.bytes);
-    int rc;
-    if ((rc = dev_alloc(ctx, &E.blob, total))) return rc;
+    GROW(E.blob, total);
     CK(cudaMemcpyAsync(E.blob, host.data(), total, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     Class4Dev& V = E.view;
@@ -2154,7 +2040,7 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     V.terms = (const unsigned*)(E.blob + o_tm); V.tptr = (const unsigned*)(E.blob + o_tp);
     V.wfl = (const unsigned*)(E.blob + o_wf); V.wlist = (const unsigned short*)(E.blob + o_wl);
     V.fill = (const unsigned*)(E.blob + o_fl); V.chunk_f0 = (const int*)(E.blob + o_f0); V.fperm = (const unsigned*)(E.blob + o_fp);
-    *out = &E;
+    *out = &ctx->class_tabs4.emplace(key, std::move(E)).first->second;
     return TUNA_OK;
 }
 
@@ -2176,14 +2062,12 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             ctx->cur_jobset4 = (int)i;
             return TUNA_OK;
         }
+    ctx->cur_jobset4 = -1;
     if (ctx->jobsets4.size() >= 6) {
         CK(cudaStreamSynchronize(ctx->stream));
-        free_jobset4(ctx->jobsets4.front());
         ctx->jobsets4.erase(ctx->jobsets4.begin());
     }
-    ctx->jobsets4.emplace_back();
-    ctx->cur_jobset4 = (int)ctx->jobsets4.size() - 1;
-    tuna_ctx::JobSet4& JS = ctx->jobsets4.back();
+    tuna_ctx::JobSet4 JS;         // cached only once complete: a failed build frees whatever it allocated
     JS.tau = tau; JS.nD = nD; JS.shard_n = ctx->shard_n; JS.dens_bound = ctx->dens_bound;
     std::vector<tuna_ctx::Job4Host>& jobs4 = JS.jobs;
     const ShellSystem& S = ctx->ss;
@@ -2256,12 +2140,12 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             jobs4.push_back(jh);
             job_cls.push_back({cb, ck});
         }
-    if ((rc = dev_alloc(ctx, &JS.d_prefix, std::max<size_t>(all_prefix.size(), 1)))) return rc;
+    GROW(JS.d_prefix, std::max<size_t>(all_prefix.size(), 1));
     CK(cudaMemcpyAsync(JS.d_prefix, all_prefix.data(), all_prefix.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     for (size_t j = 0; j < jobs4.size(); ++j) jobs4[j].job.item_prefix = JS.d_prefix + prefix_off[j];
     if (fill) {
-        if ((rc = dev_alloc(ctx, &JS.d_scratch, (size_t)std::max<long long>(fill_run, 1)))) return rc;
+        GROW(JS.d_scratch, (size_t)std::max<long long>(fill_run, 1));
         // (bra pair, ket pair) of every item, job after job in the order of all_prefix
         std::vector<int> fpairs;
         std::vector<size_t> fp_off;
@@ -2272,7 +2156,7 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             for (size_t ib = 0; ib < S.classes[cb].pairs.size(); ++ib)
                 for (long long k = 0; k < pf[ib + 1] - pf[ib]; ++k) { fpairs.push_back(S.classes[cb].pairs[ib]); fpairs.push_back(S.classes[ck].pairs[(size_t)k]); }
         }
-        if ((rc = dev_alloc(ctx, &JS.d_fill_pairs, std::max<size_t>(fpairs.size(), 1)))) return rc;
+        GROW(JS.d_fill_pairs, std::max<size_t>(fpairs.size(), 1));
         CK(cudaMemcpyAsync(JS.d_fill_pairs, fpairs.data(), fpairs.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         for (size_t j = 0; j < jobs4.size(); ++j) { jobs4[j].job.fill_scratch = JS.d_scratch; jobs4[j].job.fill_pairs = JS.d_fill_pairs + fp_off[j]; }
@@ -2310,12 +2194,12 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             g.job_off = (int)(((max_smem + 7) / 8 + 1) & ~(size_t)1);
             g.smem = (size_t)g.job_off * 8 + sizeof(Shell4Job) + 16;
             g.ctas_per_sm = (int)std::max<size_t>(1, std::min<size_t>(2048 / threads, (228 * 1024) / (g.smem + 1024)));
-            if ((rc = dev_alloc(ctx, &g.d_jobs, js.size()))) return rc;
-            if ((rc = dev_alloc(ctx, &g.d_unit_prefix, up.size()))) return rc;
+            GROW(g.d_jobs, js.size());
+            GROW(g.d_unit_prefix, up.size());
             CK(cudaMemcpyAsync(g.d_jobs, js.data(), js.size() * sizeof(Shell4Job), cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaMemcpyAsync(g.d_unit_prefix, up.data(), up.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaStreamSynchronize(ctx->stream));
-            JS.groups.push_back(g);
+            JS.groups.push_back(std::move(g));
         }
     }
     if (fill) {       // descriptors of ALL jobs and the prefix of their (shell quartet, fill entry) counts for the scatter pass
@@ -2326,8 +2210,8 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             js.push_back(jh.job); pre.push_back(pre.back() + (jh.job.nitems + ipg - 1) / ipg);
         }
         JS.scatter_total = pre.back();
-        if ((rc = dev_alloc(ctx, &JS.d_all_jobs, std::max<size_t>(js.size(), 1)))) return rc;
-        if ((rc = dev_alloc(ctx, &JS.d_scatter_pre, pre.size()))) return rc;
+        GROW(JS.d_all_jobs, std::max<size_t>(js.size(), 1));
+        GROW(JS.d_scatter_pre, pre.size());
         CK(cudaMemcpyAsync(JS.d_all_jobs, js.data(), js.size() * sizeof(Shell4Job), cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaMemcpyAsync(JS.d_scatter_pre, pre.data(), pre.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -2346,6 +2230,8 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             fclose(f);
         }
     }
+    ctx->jobsets4.push_back(std::move(JS));
+    ctx->cur_jobset4 = (int)ctx->jobsets4.size() - 1;
     return TUNA_OK;
 }
 
@@ -2464,11 +2350,7 @@ static int jk_direct_accumulate(tuna_ctx* ctx, int nD, const double* dP, double 
     const bool fixed = shell;        // the shell engine accumulates order-independently in integers; the per-component kernel uses FP64 atomics
     const size_t nacc = (size_t)nD * ncc;
     if (fixed) {
-        if (ctx->cap_fix < 4 * nacc) {
-            ctx->cap_fix = 0;
-            if ((rc = dev_alloc(ctx, &ctx->d_fix, 4 * nacc))) return rc;
-            ctx->cap_fix = 4 * nacc;
-        }
+        GROW(ctx->d_fix, 4 * nacc);
         CK(cudaMemsetAsync(ctx->d_fix, 0, 4 * nacc * sizeof(long long), ctx->stream));
     } else {
         CK(cudaMemsetAsync(ctx->d_Jc, 0, nacc * sizeof(double), ctx->stream));
@@ -2478,7 +2360,7 @@ static int jk_direct_accumulate(tuna_ctx* ctx, int nD, const double* dP, double 
     if (shell) {
         k_add_transpose_signed<<<grid_for(ctx, (int64_t)nD * ncc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Pc, ctx->d_tmp, nD, nc, 0u);   // Psym = P + P^T
         ctx->launches++;
-        double* Jw = reinterpret_cast<double*>(ctx->d_fix);
+        double* Jw = reinterpret_cast<double*>(ctx->d_fix.get());
         double* Kw = reinterpret_cast<double*>(ctx->d_fix + 2 * nacc);
         if ((rc = launch_shell4_jobs(ctx, nD, ctx->d_Pc, ctx->d_tmp, Jw, Kw, tau, (long long)nacc))) return rc;
     } else {
@@ -2704,11 +2586,9 @@ static int jk_direct_group_core(tuna_ctx* const* ctxs, int nctx, int nD, const d
             }
         CK(cudaSetDevice(ctx->device));
         // 3. pull every peer's accumulators into the staging buffer once its accumulate is done (one auxiliary stream per peer)
-        if (ctx->cap_peer < npeer * words) {
+        if (ctx->d_peer.capacity() < npeer * words) {
             CK(cudaStreamSynchronize(ctx->stream));
-            ctx->cap_peer = 0;
-            if ((rc = dev_alloc(ctx, &ctx->d_peer, npeer * words))) return rc;
-            ctx->cap_peer = npeer * words;
+            GROW(ctx->d_peer, npeer * words);
         }
         for (int r = 1; r < nctx; ++r) CK(cudaStreamWaitEvent(ctx->stream, ctxs[r]->ev_group, 0));
         CK(cudaEventRecord(ctx->ev[6][0], ctx->stream));
@@ -2736,12 +2616,12 @@ static int jk_direct_group_core(tuna_ctx* const* ctxs, int nctx, int nD, const d
         CK(cudaSetDevice(ctx->device));
         // 4. sum into ctxs[0]'s accumulators, 5. finish there
         if (fixed) {
-            k_fix_reduce<<<grid_for(ctx, (int64_t)words, 256, 8), 256, 0, ctx->stream>>>(reinterpret_cast<unsigned long long*>(ctx->d_fix),
-                reinterpret_cast<const unsigned long long*>(ctx->d_peer), words, words, npeer);
+            k_fix_reduce<<<grid_for(ctx, (int64_t)words, 256, 8), 256, 0, ctx->stream>>>(reinterpret_cast<unsigned long long*>(ctx->d_fix.get()),
+                reinterpret_cast<const unsigned long long*>(ctx->d_peer.get()), words, words, npeer);
         } else {
-            const double* stage = reinterpret_cast<const double*>(ctx->d_peer);
-            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Jc, stage, nacc, words, npeer);
-            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Kc, stage + nacc, nacc, words, npeer);
+            const double* stage = reinterpret_cast<const double*>(ctx->d_peer.get());
+            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Jc.get(), stage, nacc, words, npeer);
+            k_fix_reduce<<<grid_for(ctx, (int64_t)nacc, 256, 8), 256, 0, ctx->stream>>>(ctx->d_Kc.get(), stage + nacc, nacc, words, npeer);
             ctx->launches++;
         }
         ctx->launches++;
@@ -2769,7 +2649,7 @@ int tuna_jk_direct(tuna_ctx* ctx, int nD, const double* P, double* J, double* K,
     unsigned anti_mask;
     if ((rc = stage_host_density(ctx, nD, P, &nDrun, &anti_mask))) return rc;
     CK(cudaMemcpyAsync(ctx->d_P, ctx->h_pin, (size_t)nDrun * ctx->nbf * ctx->nbf * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    if ((rc = jk_direct_core(ctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J : nullptr, K ? ctx->d_K : nullptr, tau))) return rc;
+    if ((rc = jk_direct_core(ctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J.get() : nullptr, K ? ctx->d_K.get() : nullptr, tau))) return rc;
     return unstage_host_results(ctx, nD, nDrun, J, K);
 } TUNA_CATCH
 
@@ -2794,7 +2674,7 @@ int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* 
         if ((rc = stage_host_density(ctx, nD, P, &nDrun, &anti_mask))) return rc;
         for (int r = 1; r < nctx; ++r) ctxs[r]->dens_bound = ctx->dens_bound;
         CK(cudaMemcpyAsync(ctx->d_P, ctx->h_pin, (size_t)nDrun * ctx->nbf * ctx->nbf * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        if ((rc = jk_direct_group_core(ctxs, nctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J : nullptr, K ? ctx->d_K : nullptr, tau))) return rc;
+        if ((rc = jk_direct_group_core(ctxs, nctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J.get() : nullptr, K ? ctx->d_K.get() : nullptr, tau))) return rc;
         return unstage_host_results(ctx, nD, nDrun, J, K);
     } TUNA_CATCH
 }
@@ -2837,9 +2717,8 @@ int tuna_algorithmic_flops(const tuna_ctx* c, double* eri_flops, double* digest)
 int tuna_fp64_peak_probe(tuna_ctx* ctx, double* tflops) {
     if (!ctx || !tflops) return TUNA_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
-    double* d = nullptr;
-    int rc;
-    if ((rc = dev_alloc(ctx, &d, (size_t)1))) return rc;
+    DevBuf<double> d;
+    GROW(d, (size_t)1);
     const int blocks = ctx->sm_count * 8, threads = 256, iters = 1 << 14;
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
@@ -2862,7 +2741,6 @@ int tuna_fp64_peak_probe(tuna_ctx* ctx, double* tflops) {
         nl = (int)std::min(4096.0, std::ceil(nl * 600.0 / std::max(ms, 1.0f)));
     }
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    dev_free(&d);
     *tflops = best;
     return TUNA_OK;
 }
