@@ -56,6 +56,12 @@ int tuna_eri_fill_cart(tuna_ctx* ctx);
 /* transform_to_spherical_harmonics, ERI part (tuna_kernel.py:504-523): (U (x) U) ERI (U (x) U)^T on the device.
  * keep_cart != 0 keeps the Cartesian tensor resident as well. */
 int tuna_eri_cart_to_sph(tuna_ctx* ctx, int keep_cart);
+/* The spherical tensor nbf^4 without the Cartesian one: the engine's fill mode, then a pass that rotates every shell quartet's
+ * Cartesian block with the per-shell blocks of U and writes one value to all eight images (bitwise reproducible, exact parity zeros).
+ * Needs tuna_set_basis and tuna_set_transform.  Leaves the spherical tensor resident as the stored tensor and no Cartesian tensor.
+ * Bases the engine does not fill, a U that is not block-diagonal over the basis's shells, and the identity U run
+ * tuna_eri_fill_cart + tuna_eri_cart_to_sph(ctx, 0) instead.  tuna_last_kernel_ms(0) times the fill. */
+int tuna_eri_fill_sph(tuna_ctx* ctx);
 /* Copy a resident tensor to the host: which = 0 Cartesian (ncart^4), 1 spherical (nbf^4). */
 int tuna_eri_download(tuna_ctx* ctx, int which, double* host_out);
 /* Adopt a dense n^4 tensor supplied by the caller as the stored tensor for tuna_jk_stored (a plain ndarray

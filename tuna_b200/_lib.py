@@ -15,7 +15,7 @@ OK, ERR_ARG, ERR_NOMEM, ERR_CUDA, ERR_STATE = 0, 1, 2, 3, 4
 
 EXPORTS = [
     "tuna_ctx_create", "tuna_ctx_destroy", "tuna_last_error", "tuna_set_stream", "tuna_set_basis", "tuna_set_transform",
-    "tuna_eri_fill_cart", "tuna_eri_cart_to_sph", "tuna_eri_download", "tuna_eri_upload", "tuna_eri_single", "tuna_schwarz",
+    "tuna_eri_fill_cart", "tuna_eri_cart_to_sph", "tuna_eri_fill_sph", "tuna_eri_download", "tuna_eri_upload", "tuna_eri_single", "tuna_schwarz",
     "tuna_jk_stored", "tuna_jk_stored_dev", "tuna_jk_direct", "tuna_jk_direct_dev", "tuna_set_shard", "tuna_get_counts",
     "tuna_last_kernel_ms", "tuna_algorithmic_flops", "tuna_fp64_peak_probe", "tuna_eri_transform", "tuna_eri_transform_dev",
     "tuna_eri_transform_spin_blocked", "tuna_one_electron", "tuna_cross_overlap", "tuna_jk_direct_group", "tuna_jk_direct_group_dev",
@@ -52,6 +52,7 @@ def load() -> ctypes.CDLL:
         "tuna_set_transform": (ci, [vp, ci, c_dp]),
         "tuna_eri_fill_cart": (ci, [vp]),
         "tuna_eri_cart_to_sph": (ci, [vp, ci]),
+        "tuna_eri_fill_sph": (ci, [vp]),
         "tuna_eri_download": (ci, [vp, ci, c_dp]),
         "tuna_eri_upload": (ci, [vp, ci, c_dp]),
         "tuna_eri_single": (ci, [vp, ci, ci, ci, ci, c_dp]),
@@ -174,6 +175,11 @@ class Context:
 
     def eri_cart_to_sph(self, keep_cart: bool = False):
         self._ck(self._lib.tuna_eri_cart_to_sph(self._h, int(keep_cart)))
+        self.n_stored = self.nbf
+
+    def eri_fill_sph(self):
+        """The spherical tensor as the stored tensor, without a Cartesian tensor on the engine path (tuna_eri_fill_sph)."""
+        self._ck(self._lib.tuna_eri_fill_sph(self._h))
         self.n_stored = self.nbf
 
     def eri_download(self, which: int, out=None):

@@ -743,4 +743,95 @@ TUNA_HD void shell4_fill_scatter(const Shell4Job& J, const ShellData& D, long lo
     }
 }
 
+// Per-shell Cartesian->spherical blocks (SphShells of shell_host.hpp, on the device)
+struct SphData {
+    const int* nsph; const int* sph; const int* uoff; const double* u; const int* par;
+};
+
+TUNA_HD int sph_ncart(int L) { return (L + 1) * (L + 2) / 2; }
+
+// Spherical fill, second pass: shell quartet `item` of a job straight into the spherical tensor (dimension n).  The CTA
+//   1. sums the primitive chunks of every fill entry in the order of shell4_fill_scatter, applies the component norms and stores the
+//      Cartesian block E[a][b][c][d] in `cart` (parity-forbidden entries zero);
+//   2. for every spherical function p of A: X[b][c][d] = sum_a U_A[p][a] E, then Y[q][c][d] = sum_b U_B[q][b] X, X[q][r][d] = sum_c U_C[r][c] Y,
+//      and each (q, r, s) sums over d and writes its value to the eight images.
+// Every sum runs in a fixed order (bitwise reproducible, no atomics).  Spherical quartets that another element of the same block represents
+// (A = B with q > p, C = D with s > r, bra pair = ket pair with (r, s) > (p, q)) are skipped, so every element has one value; a quartet whose
+// parities do not cancel is written as an exact zero.  cart holds nA nB nC nD doubles, X and Y nB nC nD each.
+template <class Pol>
+TUNA_HD void shell4_fill_sph(const Shell4Job& J, const ShellData& D, const SphData& Y, long long item, const double* __restrict__ fnorm,
+                             double* __restrict__ cart, double* __restrict__ X, double* __restrict__ Yb, double* __restrict__ out, long long n) {
+    const int tid = Pol::cta_thread(), nt = Pol::cta_threads();
+    const int nf = J.ct.nfill;
+    const int pab = J.fill_pairs[2 * item], pcd = J.fill_pairs[2 * item + 1];
+    const int shA = D.pairA[pab], shB = D.pairB[pab], shC = D.pairA[pcd], shD = D.pairB[pcd];
+    const int nA = sph_ncart(J.La), nB = sph_ncart(J.Lb), nC = sph_ncart(J.Lc), nD = sph_ncart(J.Ld);
+    const int mA = Y.nsph[shA], mB = Y.nsph[shB], mC = Y.nsph[shC], mD = Y.nsph[shD];
+    const double *uA = Y.u + Y.uoff[shA], *uB = Y.u + Y.uoff[shB], *uC = Y.u + Y.uoff[shC], *uD = Y.u + Y.uoff[shD];
+    const int ncd = nC * nD, nbcd = nB * ncd;
+    for (int x = tid; x < nA * nbcd; x += nt) cart[x] = 0.0;
+    Pol::sync_cta();
+    const double* s = J.fill_scratch + J.fill_base + item * J.psplit * nf;
+    for (int e = tid; e < nf; e += nt) {
+        const unsigned m = J.ct.fill[2 * e + 1];
+        const int a = m & 255, b = (m >> 8) & 255, c = (m >> 16) & 255, d = m >> 24;
+        double v = 0.0;
+        for (int pc = 0; pc < J.psplit; ++pc) v += s[(long long)pc * nf + e];
+        v *= fnorm[D.sh_ao[shA * SH_NCMAX + a]] * fnorm[D.sh_ao[shB * SH_NCMAX + b]] * fnorm[D.sh_ao[shC * SH_NCMAX + c]] * fnorm[D.sh_ao[shD * SH_NCMAX + d]];
+        cart[a * nbcd + b * ncd + c * nD + d] = v;
+    }
+    Pol::sync_cta();
+    const long long n2 = n * n, n3 = n2 * n;
+    for (int p = 0; p < mA; ++p) {
+        for (int x = tid; x < nbcd; x += nt) {
+            double v = 0.0;
+            for (int a = 0; a < nA; ++a) {
+                const double u = uA[p * nA + a];
+                if (u != 0.0) v = fma(u, cart[a * nbcd + x], v);
+            }
+            X[x] = v;
+        }
+        Pol::sync_cta();
+        for (int x = tid; x < mB * ncd; x += nt) {
+            const int q = x / ncd, cd = x - q * ncd;
+            double v = 0.0;
+            for (int b = 0; b < nB; ++b) {
+                const double u = uB[q * nB + b];
+                if (u != 0.0) v = fma(u, X[b * ncd + cd], v);
+            }
+            Yb[x] = v;
+        }
+        Pol::sync_cta();
+        for (int x = tid; x < mB * mC * nD; x += nt) {
+            const int qr = x / nD, d = x - qr * nD, q = qr / mC, r = qr - q * mC;
+            double v = 0.0;
+            for (int c = 0; c < nC; ++c) {
+                const double u = uC[r * nC + c];
+                if (u != 0.0) v = fma(u, Yb[(q * nC + c) * nD + d], v);
+            }
+            X[x] = v;
+        }
+        Pol::sync_cta();
+        const long long P = Y.sph[shA * SH_NCMAX + p];
+        for (int x = tid; x < mB * mC * mD; x += nt) {
+            const int qr = x / mD, sd = x - qr * mD, q = qr / mC, r = qr - q * mC;
+            if (shA == shB && q > p) continue;
+            if (shC == shD && sd > r) continue;
+            if (pab == pcd && (r > p || (r == p && sd > q))) continue;
+            const long long Q = Y.sph[shB * SH_NCMAX + q], R = Y.sph[shC * SH_NCMAX + r], S = Y.sph[shD * SH_NCMAX + sd];
+            double v = 0.0;
+            if ((Y.par[P] ^ Y.par[Q] ^ Y.par[R] ^ Y.par[S]) == 0)
+                for (int d = 0; d < nD; ++d) {
+                    const double u = uD[sd * nD + d];
+                    if (u != 0.0) v = fma(u, X[qr * nD + d], v);
+                }
+            out[P * n3 + Q * n2 + R * n + S] = v; out[Q * n3 + P * n2 + R * n + S] = v;
+            out[P * n3 + Q * n2 + S * n + R] = v; out[Q * n3 + P * n2 + S * n + R] = v;
+            out[R * n3 + S * n2 + P * n + Q] = v; out[S * n3 + R * n2 + P * n + Q] = v;
+            out[R * n3 + S * n2 + Q * n + P] = v; out[S * n3 + R * n2 + Q * n + P] = v;
+        }
+        Pol::sync_cta();
+    }
+}
+
 }  // namespace tuna

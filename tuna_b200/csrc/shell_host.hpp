@@ -181,6 +181,53 @@ inline long long build_item_prefix(const ShellSystem& S, int cb, int ck, double 
     return prefix.back();
 }
 
+// Cartesian->spherical rotation U (nbf x ncart, row-major) sliced by the engine's shells: block s holds the rows of the spherical
+// functions built from shell s (columns = the shell's components in ShellTab order).  The spherical fill (shell4_fill_sph) rotates
+// every shell quartet with these blocks, which is exact only when U is block-diagonal over the shells.
+struct SphShells {
+    std::vector<int> nsph;             // per shell: spherical functions (rows of its block)
+    std::vector<int> sph;              // [shell * SH_NCMAX + k] -> spherical function index
+    std::vector<int> uoff;             // per shell: first element of its block in u
+    std::vector<double> u;             // blocks, each nsph x nc[L] row-major
+    std::vector<int> par;              // per spherical function: x/y parity code (ShellTab::pg of every component in its row)
+};
+
+// True when every nonzero U[p][a] has p and a in the same shell, every row has a nonzero, all nonzeros of a row have one x/y parity
+// (so parity-forbidden spherical elements are exact zeros), and no shell has more rows than components.  Fills Y when true.
+inline bool build_sph_shells(const ShellSystem& S, const ShellTab& T, int nbf, int ncart, const double* U, SphShells& Y) {
+    Y = SphShells();
+    if (!S.ok) return false;
+    const int ns = (int)S.shells.size();
+    std::vector<int> shell_of(ncart, -1), comp_of(ncart, -1);
+    for (int s = 0; s < ns; ++s)
+        for (int c = 0; c < T.nc[S.shells[s].L]; ++c) { shell_of[S.shells[s].ao[c]] = s; comp_of[S.shells[s].ao[c]] = c; }
+    Y.nsph.assign(ns, 0);
+    Y.sph.assign((size_t)ns * SH_NCMAX, 0);
+    Y.par.assign(nbf, 0);
+    for (int p = 0; p < nbf; ++p) {
+        int sh = -1, pg = -1;
+        for (int a = 0; a < ncart; ++a) {
+            if (U[(size_t)p * ncart + a] == 0.0) continue;
+            const int g = T.pg[S.shells[shell_of[a]].L][comp_of[a]];
+            if (sh < 0) { sh = shell_of[a]; pg = g; }
+            if (shell_of[a] != sh || g != pg) return false;
+        }
+        if (sh < 0 || Y.nsph[sh] == T.nc[S.shells[sh].L]) return false;
+        Y.sph[(size_t)sh * SH_NCMAX + Y.nsph[sh]++] = p;
+        Y.par[p] = pg;
+    }
+    Y.uoff.assign(ns, 0);
+    size_t total = 0;
+    for (int s = 0; s < ns; ++s) { Y.uoff[s] = (int)total; total += (size_t)Y.nsph[s] * T.nc[S.shells[s].L]; }
+    Y.u.assign(total, 0.0);
+    for (int s = 0; s < ns; ++s) {
+        const int nc = T.nc[S.shells[s].L];
+        for (int k = 0; k < Y.nsph[s]; ++k)
+            for (int c = 0; c < nc; ++c) Y.u[Y.uoff[s] + (size_t)k * nc + c] = U[(size_t)Y.sph[(size_t)s * SH_NCMAX + k] * ncart + S.shells[s].ao[c]];
+    }
+    return true;
+}
+
 struct HostPtrOf {
     template <class V> const typename V::value_type* operator()(const V& v) const { return v.data(); }
 };

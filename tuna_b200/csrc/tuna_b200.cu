@@ -3,6 +3,8 @@
 // Kernels (DESIGN.md has the roofline of each):
 //   k_fill_scatter    dense tensor, second pass: the engine's fill mode (k_shell4_*) leaves the unique integrals of every work item in
 //                     scratch rows; this sums the primitive chunks in a fixed order and writes the eight images
+//   k_fill_scatter_sph  the same second pass straight into the spherical tensor: each shell quartet's Cartesian block is rotated with
+//                     the per-shell blocks of U and written to the eight images; no Cartesian tensor exists
 //   k_eri_fill        the dense tensor with one thread per AO quartet (uncontracted bases, bases that do not group into shells)
 //   k_schwarz         Q_ij = sqrt((ij|ij))
 //   k_rotate_axis     one index of the Cartesian->spherical rotation (sparse U), used 4x for the tensor, 2x for matrices
@@ -73,6 +75,11 @@ struct tuna_ctx {
     int nbf = 0;
     bool U_identity = false;
     CsrDev U, Ut;
+    // U is block-diagonal over the engine's shells with one x/y parity per row (build_sph_shells): tuna_eri_fill_sph rotates shell
+    // quartet by shell quartet with these per-shell blocks
+    bool U_shell_blocks = false;
+    DevBuf<int> d_sph_n, d_sph_idx, d_sph_uoff, d_sph_par;
+    DevBuf<double> d_sph_u;
 
     // dense tensors
     DevBuf<double> d_eri_cart;
@@ -963,6 +970,29 @@ __global__ void __launch_bounds__(256) k_fill_scatter(const Shell4Job* __restric
     }
 }
 
+// Spherical fill, second pass (shell4_fill_sph).  Same groups of whole shell quartets as k_fill_scatter; the CTA takes the quartets of a
+// group one after another.  Each CTA keeps the Cartesian block of its current quartet in its own slice of `ws` (ws_stride doubles, L2
+// resident) and the two contraction buffers (xsize doubles each) in dynamic shared memory.
+__global__ void __launch_bounds__(256) k_fill_scatter_sph(const Shell4Job* __restrict__ jobs, const long long* __restrict__ group_pre, int njobs, ShellData D,
+                                                          SphData Y, const double* __restrict__ fnorm, double* __restrict__ ws, long long ws_stride,
+                                                          int xsize, double* __restrict__ out, int n) {
+    extern __shared__ double smem_all[];
+    double* cart = ws + blockIdx.x * ws_stride;
+    const long long ngroups = group_pre[njobs];
+    for (long long t = blockIdx.x; t < ngroups; t += gridDim.x) {
+        int lo = 0, hi = njobs;
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (group_pre[mid] <= t) lo = mid; else hi = mid;
+        }
+        const Shell4Job& J = jobs[lo];
+        const int nf = J.ct.nfill, ipg = nf >= 256 ? 1 : 256 / nf;
+        const long long item0 = (t - group_pre[lo]) * ipg, cnt = min((long long)ipg, J.nitems - item0);
+#pragma unroll 1
+        for (long long k = 0; k < cnt; ++k) shell4_fill_sph<DevPolicy<256>>(J, D, Y, item0 + k, fnorm, cart, smem_all, smem_all + xsize, out, n);
+    }
+}
+
 // reproducible accumulation: (hi, lo) integer words -> FP64 (fixed_value), J and K in one launch
 __global__ void k_fixed_to_double(const long long* __restrict__ fix, double* __restrict__ J, double* __restrict__ K, size_t count) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x) {
@@ -1246,6 +1276,7 @@ int tuna_set_basis(tuna_ctx* ctx, int ncart, const double* origins_z, const int3
     ctx->d_eri_sph.reset();
     ctx->n_stored = 0;
     ctx->nbf = 0;
+    ctx->U_shell_blocks = false;
     build_shell_tab(ctx->stab);
     ctx->shell_ready = false;
     ctx->jobsets4.clear();
@@ -1284,8 +1315,33 @@ int tuna_set_transform(tuna_ctx* ctx, int nbf, const double* U) try {
     for (int p = 0; p < nbf && ctx->U_identity; ++p)
         for (int a = 0; a < nc; ++a)
             if (u[(size_t)p * nc + a] != (p == a ? 1.0 : 0.0)) { ctx->U_identity = false; break; }
+    ctx->U_shell_blocks = false;
+    SphShells Y;
+    if (build_sph_shells(ctx->ss, ctx->stab, nbf, nc, u.data(), Y)) {
+        GROW(ctx->d_sph_n, Y.nsph.size());
+        GROW(ctx->d_sph_idx, Y.sph.size());
+        GROW(ctx->d_sph_uoff, Y.uoff.size());
+        GROW(ctx->d_sph_par, Y.par.size());
+        GROW(ctx->d_sph_u, std::max<size_t>(Y.u.size(), 1));
+        CK(cudaMemcpyAsync(ctx->d_sph_n, Y.nsph.data(), Y.nsph.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->d_sph_idx, Y.sph.data(), Y.sph.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->d_sph_uoff, Y.uoff.data(), Y.uoff.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->d_sph_par, Y.par.data(), Y.par.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->d_sph_u, Y.u.data(), Y.u.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        ctx->U_shell_blocks = true;
+    }
     return TUNA_OK;
 } TUNA_CATCH
+
+// The dense tensor is filled by the shell-quartet engine (rather than k_eri_fill) for a basis that groups into shells and has contracted
+// shells, unless TUNA_B200_DIRECT_ENGINE=generic; TUNA_B200_FILL_ENGINE=1 / 0 forces the choice (reasons in tuna_eri_fill_cart).
+static bool fill_uses_engine(const tuna_ctx* ctx) {
+    bool contracted = false;
+    for (const auto& sh : ctx->ss.shells) contracted = contracted || sh.nprim > 1;
+    const char* ef = getenv("TUNA_B200_FILL_ENGINE");
+    return ctx->direct_engine == 1 && ctx->ss.ok && (ef ? atoi(ef) != 0 : contracted);
+}
 
 int tuna_eri_fill_cart(tuna_ctx* ctx) try {
     if (!ctx) return TUNA_ERR_ARG;
@@ -1299,10 +1355,7 @@ int tuna_eri_fill_cart(tuna_ctx* ctx) try {
     // followed by the scatter pass; an uncontracted basis keeps the per-AO-quartet kernel, which is as fast there (ET100: 1.40 vs 1.52 ms;
     // N2/cc-pVTZ: 3.7 vs 0.87 ms, Ne2/cc-pVQZ: 13.6 vs 5.4 ms).  TUNA_B200_FILL_ENGINE=1 / 0 forces one or the other.  Both leave the same
     // tensor: one value written to all eight images, exact zeros for the parity-forbidden elements.
-    bool contracted = false;
-    for (const auto& sh : ctx->ss.shells) contracted = contracted || sh.nprim > 1;
-    const char* ef = getenv("TUNA_B200_FILL_ENGINE");
-    bool engine = ctx->direct_engine == 1 && ctx->ss.ok && (ef ? atoi(ef) != 0 : contracted);
+    bool engine = fill_uses_engine(ctx);
     // the dense tensor is never sharded (every rank holds all of it): the fill runs as rank 0 of 1, whatever tuna_set_shard said
     struct ShardGuard { tuna_ctx* c; int r, n; ~ShardGuard() { c->shard_rank = r; c->shard_n = n; } } guard{ctx, ctx->shard_rank, ctx->shard_n};
     GROW(ctx->d_eri_cart, count);
@@ -1381,6 +1434,80 @@ int tuna_eri_cart_to_sph(tuna_ctx* ctx, int keep_cart) try {
     if (rc) { ctx->d_eri_sph.reset(); return rc; }
     ctx->n_stored = (int)nb;
     return check_pair_symmetry(ctx);
+} TUNA_CATCH
+
+int tuna_eri_fill_sph(tuna_ctx* ctx) try {
+    if (!ctx) return TUNA_ERR_ARG;
+    if (ctx->ncart == 0) FAIL(TUNA_ERR_STATE, "tuna_eri_fill_sph: call tuna_set_basis first");
+    if (ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_eri_fill_sph: call tuna_set_transform first");
+    CK(cudaSetDevice(ctx->device));
+    int rc;
+    if ((rc = ensure_pairs(ctx))) return rc;
+    // Bases the engine does not fill, a U that is not block-diagonal over the engine's shells, and CARTHARM (identity U, the Cartesian
+    // tensor is adopted) take the two-step path; so does a fill whose scratch rows do not fit (tuna_eri_fill_cart then uses k_eri_fill).
+    const auto two_step = [ctx]() { const int r = tuna_eri_fill_cart(ctx); return r ? r : tuna_eri_cart_to_sph(ctx, 0); };
+    if (!fill_uses_engine(ctx) || !ctx->U_shell_blocks || ctx->U_identity) return two_step();
+    ctx->d_eri_cart.reset();
+    ctx->d_eri_sph.reset();
+    ctx->n_stored = 0;
+    const size_t nb = ctx->nbf;
+    struct ShardGuard { tuna_ctx* c; int r, n; ~ShardGuard() { c->shard_rank = r; c->shard_n = n; } } guard{ctx, ctx->shard_rank, ctx->shard_n};
+    ctx->shard_rank = 0; ctx->shard_n = 1;
+    GROW(ctx->d_eri_sph, nb * nb * nb * nb);
+    rc = ensure_shell4(ctx, 0.0, 0);
+    if (rc) {
+        ctx->d_eri_sph.reset();
+        if (rc != TUNA_ERR_NOMEM) return rc;
+        return two_step();
+    }
+    const size_t js = (size_t)ctx->cur_jobset4;
+    // the fill job set holds the scratch rows: it is dropped after the pass, and on every error path with the half-built tensor
+    const auto fail = [ctx](int code) {
+        cudaStreamSynchronize(ctx->stream);
+        ctx->jobsets4.erase(ctx->jobsets4.begin() + ctx->cur_jobset4);
+        ctx->cur_jobset4 = -1;
+        ctx->d_eri_sph.reset();
+        return code;
+    };
+    // per-CTA Cartesian block (global, L2 resident) and contraction buffers (shared): sized by the largest class of the job set
+    long long blk = 1, xsz = 1;
+    for (const auto& jh : ctx->jobsets4[js].jobs) {
+        const long long nB = sph_ncart(jh.job.Lb), ncd = (long long)sph_ncart(jh.job.Lc) * sph_ncart(jh.job.Ld);
+        blk = std::max(blk, sph_ncart(jh.job.La) * nB * ncd);
+        xsz = std::max(xsz, nB * ncd);
+    }
+    xsz = (xsz + 1) & ~1LL;
+    const long long total = ctx->jobsets4[js].scatter_total;
+    const long long ws_cap = 64ll << 20;       // bytes of Cartesian blocks: at least one CTA per SM, at most four
+    const long long grid = std::max<long long>(1, std::min<long long>(total, std::max<long long>(ctx->sm_count, std::min<long long>(4ll * ctx->sm_count, ws_cap / (8 * blk)))));
+    DevBuf<double> ws;
+    if (const int g = ws.grow((size_t)(grid * blk), ctx->err)) return fail(g);
+    const size_t smem = (size_t)(2 * xsz) * sizeof(double);
+    if (smem > 48 * 1024) {
+        if (const cudaError_t e = opt_in_smem<k_fill_scatter_sph>(ctx)) { ctx->err = cudaGetErrorString(e); return fail(TUNA_ERR_CUDA); }
+    }
+    CK(cudaEventRecord(ctx->ev[0][0], ctx->stream));
+    if ((rc = launch_shell4_jobs(ctx, 0, nullptr, nullptr, nullptr, nullptr, 0.0, 0))) return fail(rc);
+    if (total > 0) {
+        const tuna_ctx::JobSet4& JS = ctx->jobsets4[js];
+        ShellData D;
+        D.pairA = ctx->d_pairA; D.pairB = ctx->d_pairB; D.pair_rec = ctx->d_pair_rec; D.rec = ctx->d_rec; D.pairQ = ctx->d_pairQ;
+        D.sh_ao = ctx->d_sh_ao; D.boys = ctx->d_boys; D.herm = ctx->d_herm; D.fix_lo = 0;
+        SphData Y;
+        Y.nsph = ctx->d_sph_n; Y.sph = ctx->d_sph_idx; Y.uoff = ctx->d_sph_uoff; Y.u = ctx->d_sph_u; Y.par = ctx->d_sph_par;
+        k_fill_scatter_sph<<<(unsigned)grid, 256, smem, ctx->stream>>>(JS.d_all_jobs, JS.d_scatter_pre, (int)JS.jobs.size(), D, Y, ctx->d_fnorm, ws, blk,
+                                                                       (int)xsz, ctx->d_eri_sph, (int)nb);
+        ctx->launches++;
+    }
+    cudaError_t le = cudaGetLastError();
+    if (le == cudaSuccess) le = cudaEventRecord(ctx->ev[0][1], ctx->stream);
+    if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
+    if (le != cudaSuccess) { ctx->err = cudaGetErrorString(le); return fail(TUNA_ERR_CUDA); }
+    ctx->jobsets4.erase(ctx->jobsets4.begin() + ctx->cur_jobset4);      // the scratch rows are only needed until the pass has run
+    ctx->cur_jobset4 = -1;
+    ctx->n_stored = (int)nb;
+    ctx->eri_pair_sym = true;          // one value is written to all eight images
+    return TUNA_OK;
 } TUNA_CATCH
 
 int tuna_eri_download(tuna_ctx* ctx, int which, double* host_out) try {

@@ -108,6 +108,7 @@ class ERIHandle:
     def __init__(self, ctx, n, basis_kind, mode):
         self.ctx, self.n, self.basis_kind, self.mode = ctx, int(n), basis_kind, mode
         self._host = None
+        self.pending_fill = False   # stored mode: the tensor is filled by transform_to_spherical_harmonics, or on first touch as an array
         self._jk_cache = []     # [(P, J, K)] most recent first
         self._group = None      # direct mode over several devices: DeviceGroup built on the first J/K call
 
@@ -121,19 +122,25 @@ class ERIHandle:
             if self.mode == "direct":
                 self._materialise_direct()
             else:
+                if self.pending_fill:
+                    self.ctx.eri_fill_cart()
+                    self.pending_fill = False
                 self._host = self.ctx.eri_download(0 if self.basis_kind == "cart" else 1)
         return self._host
 
     def _materialise_direct(self):
         ctx = self.ctx
-        need = 8 * ctx.ncart ** 4
+        if self.basis_kind == "cart" or not hasattr(ctx, "eri_fill_sph"):
+            need = 8 * ctx.ncart ** 4
+        else:   # the spherical fill: nbf^4 plus the engine's scratch rows, which are about as large as the unique Cartesian integrals
+            need = 8 * (ctx.nbf ** 4 + ctx.ncart ** 4 // 8)
         if need > 0.8 * _free_device_bytes():
             raise MemoryError(f"tuna_b200: a dense ERI tensor was requested in direct mode but {need / 1e9:.1f} GB do not fit on the device")
-        ctx.eri_fill_cart()
         if self.basis_kind == "cart":
+            ctx.eri_fill_cart()
             self._host = ctx.eri_download(0)
         else:
-            ctx.eri_cart_to_sph()
+            _fill_spherical(ctx)
             self._host = ctx.eri_download(1)
 
     def __array__(self, dtype=None, copy=None):
@@ -324,11 +331,29 @@ def calculate_two_electron_integrals(n_basis, basis_functions, calculation):
     timer("Two-electron integrals", 0)
     mode = _choose_mode(n_basis, calculation)
     ctx = _context_for(basis_functions)
-    if mode == "stored":
-        ctx.eri_fill_cart()
     handle = ERIHandle(ctx, n_basis, "cart", mode)
+    handle.pending_fill = mode == "stored"     # filled straight into the spherical basis once U is known (transform_to_spherical_harmonics)
     timer("Two-electron integrals", 1)
     return handle
+
+
+def _fill_spherical(ctx):
+    """The spherical tensor as the stored tensor: one pass without the Cartesian tensor where the library has it, else fill + rotation."""
+    if hasattr(ctx, "eri_fill_sph"):
+        ctx.eri_fill_sph()
+    else:
+        ctx.eri_fill_cart()
+        ctx.eri_cart_to_sph()
+
+
+def _stored_to_spherical(handle):
+    """Stored mode: the spherical tensor of a Cartesian handle, after ctx.set_transform.  A handle whose Cartesian tensor was already
+    filled (touched as an array) is rotated; otherwise the tensor is filled in the spherical basis directly."""
+    if handle.pending_fill:
+        handle.pending_fill = False
+        _fill_spherical(handle.ctx)
+    else:
+        handle.ctx.eri_cart_to_sph()
 
 
 def transform_to_spherical_harmonics(S_cart, T_cart, V_NE_cart, D_cart, Q_cart, ERI_AO_cart, molecule, calculation, silent):
@@ -341,7 +366,7 @@ def transform_to_spherical_harmonics(S_cart, T_cart, V_NE_cart, D_cart, Q_cart, 
     if cartharm:
         ctx.set_transform(np.eye(ctx.ncart))
         if ERI_AO_cart.mode == "stored":
-            ctx.eri_cart_to_sph()
+            _stored_to_spherical(ERI_AO_cart)
         return S_cart, T_cart, V_NE_cart, D_cart, Q_cart, ERIHandle(ctx, ctx.ncart, "sph", ERI_AO_cart.mode)
     timer = _ref_timer()
     timer("Spherical harmonic transformation", 0)
@@ -352,7 +377,7 @@ def transform_to_spherical_harmonics(S_cart, T_cart, V_NE_cart, D_cart, Q_cart, 
     Q = np.einsum("mw,awx,nx->amn", U, Q_cart, U, optimize=True)
     ctx.set_transform(U)
     if ERI_AO_cart.mode == "stored":
-        ctx.eri_cart_to_sph()
+        _stored_to_spherical(ERI_AO_cart)
     handle = ERIHandle(ctx, U.shape[0], "sph", ERI_AO_cart.mode)
     timer("Spherical harmonic transformation", 1)
     return S, T, V_NE, D, Q, handle
