@@ -104,6 +104,16 @@ int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks);
 int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* P, double* J, double* K, double tau);
 /* dP, dJ, dK on ctxs[0]'s device, enqueued on ctxs[0]'s stream; symmetric densities only, as tuna_jk_direct_dev. */
 int tuna_jk_direct_group_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau);
+/* Semi-direct J/K: keep the shell-quartet engine's contracted integrals of whole class jobs in device memory, up to budget_bytes
+ * (0, the default, = off), and replay them in later tuna_jk_direct* / tuna_jk_direct_group* builds instead of evaluating them again.
+ * The first build after the store is set (or dropped) plans it and fills it while it runs; jobs that do not fit run direct.  The budget
+ * is clamped to the device's free memory less headroom, and if the allocation fails the builds run direct without an error.  J and K
+ * are bitwise identical to the direct build.  tuna_set_basis, tuna_set_transform, tuna_set_shard and a new budget drop the store; a
+ * stored job whose kept quartet list changes (another tau or density bound) runs direct.  In a group every rank stores its own share.
+ * Bases that do not group into shells (per-component kernel) ignore the budget. */
+int tuna_set_integral_store(tuna_ctx* ctx, int64_t budget_bytes);
+/* info[0] bytes held, [1] work items held, [2] work items of the last build's job set (this rank), [3] builds served by replay. */
+int tuna_integral_store_info(const tuna_ctx* ctx, int64_t info[4]);
 
 /* AO -> MO / spin-orbital four-index transformation of a dense ERI tensor (SURVEY.md 8f-2):
  *   tuna_ci.transform_ERI_AO_to_MO(ERI_AO, C, ...)        tuna_ci.py:204-255   so_layout = 0, C1 = C2 = C

@@ -19,6 +19,7 @@ EXPORTS = [
     "tuna_jk_stored", "tuna_jk_stored_dev", "tuna_jk_direct", "tuna_jk_direct_dev", "tuna_set_shard", "tuna_get_counts",
     "tuna_last_kernel_ms", "tuna_algorithmic_flops", "tuna_fp64_peak_probe", "tuna_eri_transform", "tuna_eri_transform_dev",
     "tuna_eri_transform_spin_blocked", "tuna_one_electron", "tuna_cross_overlap", "tuna_jk_direct_group", "tuna_jk_direct_group_dev",
+    "tuna_set_integral_store", "tuna_integral_store_info",
 ]
 
 _lib = None
@@ -73,6 +74,8 @@ def load() -> ctypes.CDLL:
         "tuna_cross_overlap": (ci, [vp] + [ci, c_dp, c_ip, c_ip, c_lp, c_dp, c_dp] * 2 + [c_dp]),
         "tuna_jk_direct_group": (ci, [ctypes.POINTER(vp), ci, ci, c_dp, c_dp, c_dp, cd]),
         "tuna_jk_direct_group_dev": (ci, [ctypes.POINTER(vp), ci, ci, vp, vp, vp, cd]),
+        "tuna_set_integral_store": (ci, [vp, ctypes.c_int64]),
+        "tuna_integral_store_info": (ci, [vp, c_lp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -309,6 +312,16 @@ class Context:
     def set_shard(self, rank, nranks):
         self._ck(self._lib.tuna_set_shard(self._h, rank, nranks))
 
+    def set_integral_store(self, budget_bytes: int):
+        """Semi-direct J/K: keep up to budget_bytes of the engine's integrals on the device and replay them in later direct builds
+        (0 = off, the default).  J and K stay bitwise equal to the direct build (tuna_set_integral_store)."""
+        self._ck(self._lib.tuna_set_integral_store(self._h, int(budget_bytes)))
+
+    def integral_store_info(self) -> dict:
+        c = np.zeros(4, dtype=np.int64)
+        self._ck(self._lib.tuna_integral_store_info(self._h, c.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
+        return dict(zip(["bytes", "items", "items_last_build", "replayed_builds"], (int(x) for x in c)))
+
     def counts(self) -> dict:
         c = np.zeros(8, dtype=np.int64)
         self._ck(self._lib.tuna_get_counts(self._h, c.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
@@ -391,6 +404,18 @@ class DeviceGroup:
         """Device pointers on devices[0], enqueued on the stream of contexts[0]; symmetric densities only (tuna_jk_direct_dev)."""
         self._ck(self._lib.tuna_jk_direct_group_dev(self._ptrs, len(self.contexts), nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ), ctypes.c_void_p(dK),
                                                     ctypes.c_double(tau)))
+
+    def set_integral_store(self, budget_bytes: int):
+        """Semi-direct J/K on every rank: each stores its own share of the integrals on its own device, up to budget_bytes each."""
+        for c in self.contexts:
+            c.set_integral_store(budget_bytes)
+
+    def integral_store_info(self) -> dict:
+        """The ranks' store counters: bytes and items summed over the ranks, replayed builds of contexts[0]."""
+        per_rank = [c.integral_store_info() for c in self.contexts]
+        out = {k: sum(r[k] for r in per_rank) for k in ("bytes", "items", "items_last_build")}
+        out["replayed_builds"] = per_rank[0]["replayed_builds"]
+        return out
 
     def counts(self) -> dict:
         """Counters of contexts[0], with evaluated_last_direct summed over all ranks."""

@@ -78,6 +78,11 @@ struct Class4Dev {
     // scatter pass: fperm[(m - 1) * nfill + e'] = entry handled by position e' in mode m = 1, 2, 3 (entries ordered so that c, b or a is the
     // fastest index; mode 0 is the list order, d fastest): consecutive lanes then write neighbouring elements of the images of that mode
     const unsigned* fperm;
+    // integral store (semi-direct J/K): a stored work item keeps its contracted integral buffer as one row of nint doubles in the class's
+    // canonical order (bra pair functions in class order, each followed by the columns of its parity class), which does not depend on the
+    // chunk split.  canon[chunk_c0[ch] + slot] = canonical index of integral slot `slot` of chunk ch.
+    int nint;
+    const unsigned* canon; const int* chunk_c0;
 };
 
 // Phase 4 tile (two z combinations zc, zc+1 of one x/y combination):
@@ -111,7 +116,20 @@ struct Shell4Job {
     double* fill_scratch;
     long long fill_base;
     const int* fill_pairs;          // [2 * nitems] (bra pair, ket pair) of every shell quartet of the job: the scatter pass decodes an item with one load
+    // integral store: S4_DIRECT evaluates phases 0-4; S4_STORE evaluates them for EVERY work item of the rank (also those the density
+    // screens out of this build's digestion) and writes each item's contracted buffer to its row store[store_base + row * ct.nint];
+    // S4_REPLAY loads the rows instead of phases 0-4.  The rank's rows cover only the units it owns (shell4_store_row).
+    double* store = nullptr;
+    long long store_base = 0;
+    long long store_unit0 = 0;      // flat index of the job's first unit in the launch that shards it (k_shell4_multi: the job's unit prefix)
+    long long store_ubase = 0;      // (first flat unit this rank owns in the job) / store_nranks
+    int store_mode = 0, store_nranks = 1;
 };
+
+constexpr int S4_DIRECT = 0, S4_STORE = 1, S4_REPLAY = 2;
+// Quartet4::active: 0 = idle slot, 1 = evaluate and digest, S4_ONLY_STORE = evaluate and store, but the density test of this build screens
+// it out of the digestion (store pass only)
+constexpr int S4_ONLY_STORE = 2;
 
 // Work items of a shell quartet for a target number of primitive quartets per item (0 = never split).
 inline void shell4_split(Shell4Job& J, int target, bool split_ket) {
@@ -221,15 +239,26 @@ TUNA_HD void assemble4(const double* xyx, const double* xyy, const double* sp0, 
 
 // Header of one quartet of a batch, decoded once (by one lane) before the group starts on it.
 struct Quartet4 {
-    int active, shA, shB, shC, shD, ia0;      // the four shells (A, B of the bra pair, C, D of the ket pair); first bra primitive pair of this work item | first ket primitive pair << 16
+    int active, shA, shB, shC, shD, ia0;      // active: 0, 1 or S4_ONLY_STORE (above); the four shells (A, B of the bra pair, C, D of the ket pair); first bra primitive pair of this work item | first ket primitive pair << 16
     double w;                                 // degeneracy weight
     long long recA, recC;                     // offsets of the pairs' first primitive records in ShellData::rec
     double pA, zA, pC, zC;                    // exponent sum and centre of the FIRST primitive pair of bra and ket (Boys argument without a memory round trip)
 };
 
+// Integral store: row of the work item header hq points to.  A launch deals its FLAT units U (k_shell4_one: the job's own units,
+// k_shell4_multi: the units of all its jobs, job j starting at store_unit0) to ranks by U = r (mod n), so the units a rank owns in a job are
+// U = f, f + n, f + 2n, ... (f its first); unit U holds rows (U / n - f / n) * chunk + position in the unit.  (The NB quartets of a batch lie
+// in one unit, so their rows are consecutive.)  shell4_store_share gives f / n and the rows of a rank's share.
+template <class Pol>
+TUNA_HD long long shell4_store_row(const Shell4Job& J, const Quartet4* hq) {
+    const long long wi = Pol::work_item_of(J, hq);
+    return ((J.store_unit0 + wi / J.chunk) / J.store_nranks - J.store_ubase) * J.chunk + wi % J.chunk;
+}
+
 // NB shell quartets of one class processed together by one group of Pol::G lanes.  `tab` is the CTA's table area (shared memory on
-// the device), holding the tables of chunk `tab_chunk` on entry (updated when the class has several chunks).
-template <class Pol, int NB>
+// the device), holding the tables of chunk `tab_chunk` on entry (updated when the class has several chunks).  SEMI: the job may run as a
+// store pass or a replay (J.store_mode); the direct instantiation (SEMI = false) carries none of that code.
+template <class Pol, int NB, bool SEMI = false>
 TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quartet4* hq, double* __restrict__ sm, unsigned* tab, int& tab_chunk,
                              int nD, const double* __restrict__ Pf, const double* __restrict__ Psym, double* Jf, double* Kf, int ncart) {
     const Class4Dev& CT = J.ct;
@@ -249,12 +278,13 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
 #pragma unroll
     for (int q = 0; q < NB; ++q) if (qa < 0 && hq[q].active) qa = q;
     if (qa < 0) return;                                  // uniform over the group: nothing to do (no barrier inside was reached)
-    bool act[NB];
+    bool act[NB], dig[NB];                               // evaluated / digested (a store pass evaluates quartets its density screens out)
     const double* recA[NB]; const double* recC[NB];
     double w[NB];
 #pragma unroll
     for (int q = 0; q < NB; ++q) {
         act[q] = hq[q].active != 0;
+        dig[q] = SEMI ? hq[q].active == 1 : act[q];
         const Quartet4& h = act[q] ? hq[q] : hq[qa];      // an inactive slot runs on the data of an active one with weight zero
         w[q] = act[q] ? h.w : 0.0;
         recA[q] = D.rec + h.recA; recC[q] = D.rec + h.recC;
@@ -311,15 +341,29 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
     const bool single = J.nppAB * J.nppCD == 1;
     const unsigned slotb = NB * 8;                        // bytes of one NB-interleaved slot
 
+    const bool replay = SEMI && J.store_mode == S4_REPLAY;
+
     for (int ch = 0; ch < CT.nchunk; ++ch) {
         const int t0 = CT.chunk_t0[ch], nt = CT.chunk_t0[ch + 1] - t0;
-        if (!single) { for (int x = lane; x < CT.chunk_ni[ch] * NB; x += Pol::G) Itq[x] = 0.0; }
+        if (!single && !replay) { for (int x = lane; x < CT.chunk_ni[ch] * NB; x += Pol::G) Itq[x] = 0.0; }
         if (tab_chunk != ch) {                            // (only classes with several chunks ever get here)
             Pol::sync_cta();
             shell4_load_tables<NB>(CT, ch, tab, Pol::cta_thread(), Pol::cta_threads(), J.oIt, J.oP);
             tab_chunk = ch;
             Pol::sync_cta();
         }
+        if (replay) {
+            // ---- phases 0-4 replaced: the chunk's slots from the work items' stored rows (consecutive lanes read consecutive columns)
+            const unsigned* cn = CT.canon + CT.chunk_c0[ch];
+            const double* rows = J.store + J.store_base + shell4_store_row<Pol>(J, hq) * (long long)CT.nint;
+            for (int x = lane; x < CT.chunk_ni[ch]; x += Pol::G) {
+                const unsigned c = cn[x];
+                QVec<NB> v;
+#pragma unroll
+                for (int q = 0; q < NB; ++q) v.v[q] = act[q] ? rows[(long long)q * CT.nint + c] : 0.0;
+                qst<NB>(Itq + x * NB, v);
+            }
+        } else
         for (int it = 0; it < J.clen; ++it)
             for (int kk = 0; kk < J.klen; ++kk) {
                 // primitive pairs of every quartet of the batch (a work item past the last primitive pair runs on the last one with weight 0)
@@ -514,6 +558,17 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
                 }
             }
         Pol::sync();
+        if (SEMI && J.store_mode == S4_STORE) {
+            // the chunk's contracted integrals (the direct engine's own phase-4 results) to the work items' rows, canonical order
+            const unsigned* cn = CT.canon + CT.chunk_c0[ch];
+            double* rows = J.store + J.store_base + shell4_store_row<Pol>(J, hq) * (long long)CT.nint;
+            for (int x = lane; x < CT.chunk_ni[ch]; x += Pol::G) {
+                const unsigned c = cn[x];
+                const QVec<NB> v = qld<NB>(Itq + x * NB);
+#pragma unroll
+                for (int q = 0; q < NB; ++q) if (act[q]) rows[(long long)q * CT.nint + c] = v.v[q];
+            }
+        }
         // ---- phase 5: digestion of the chunk, one accumulator per lane; all addressing from the shared-memory tables
         if (J.fill_scratch) {
             // fill mode: the chunk's integrals go to the work items' scratch rows in list order (coalesced over the lanes)
@@ -571,7 +626,7 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
 #pragma unroll
                         for (int q = 0; q < NB; ++q) {
                             const double v = s0[q] + s1[q];
-                            if (!act[q] || v == 0.0) continue;
+                            if (!dig[q] || v == 0.0) continue;
                             const int* ao = aoq + q * 4 * aos;
                             Pol::accumulate(M, ao[ri] * ncart + ao[ci], v, D.fix_lo);
                         }
@@ -692,7 +747,7 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
             const QVec<NB> v = qld<NB>(Outq + (dn * nwork + x) * NB);
 #pragma unroll
             for (int q = 0; q < NB; ++q) {
-                if (!act[q] || v.v[q] == 0.0) continue;
+                if (!dig[q] || v.v[q] == 0.0) continue;
                 const int* ao = aoq + q * 4 * aos;
                 Pol::accumulate(Kd, ao[ri] * ncart + ao[ci], v.v[q], D.fix_lo);
             }
@@ -703,7 +758,7 @@ TUNA_HD void shell4_quartets(const Shell4Job& J, const ShellData& D, const Quart
             const QVec<NB> v = qld<NB>(Outq + (dn * nwork + (e >> 16)) * NB);
 #pragma unroll
             for (int q = 0; q < NB; ++q) {
-                if (!act[q] || v.v[q] == 0.0) continue;
+                if (!dig[q] || v.v[q] == 0.0) continue;
                 const int* ao = aoq + q * 4 * aos;
                 Pol::accumulate(Jd, ao[ri] * ncart + ao[ci], v.v[q], D.fix_lo);
             }

@@ -29,6 +29,8 @@ struct Class4Host {
     std::vector<unsigned> fill;            // fill mode: {slot, a | b << 8 | c << 16 | d << 24} per parity-allowed component quartet, chunk by chunk
     std::vector<int> chunk_f0;
     std::vector<unsigned> fperm;           // [3][nfill] entry orders of the scatter modes 1..3 (c, b, a fastest)
+    std::vector<unsigned> canon;           // integral store: canonical index of every integral slot, chunk by chunk (Class4Dev::canon)
+    std::vector<int> chunk_c0;             //                 first canon entry of a chunk
     long long allowed = 0;                 // parity-allowed component quartets = integrals per shell quartet
     long long nterms = 0;                  // digestion terms (table statistics)
     bool terms_possible(int term_max) const { return nterms + nwork <= term_max && itmax < 65535 && nstage < 65535; }
@@ -218,6 +220,8 @@ inline void build_class4_tables(const ShellTab& T, int La, int Lb, int Lc, int L
     // ---- per chunk: row order, slots, S layout, phase 3 / 4 lists, digestion tables ---------------------------------------------
     std::vector<int> beta_chunk(nbeta, -1), beta_pb(nbeta, -1);     // chunk of a beta, its position in the Pb staging order
     std::vector<int> Rb0;                                            // integral-buffer rows of chunk 0 (term mode needs a single chunk)
+    std::vector<int> canon_row(nbeta, 0);                            // canonical first index of a beta's row: betas in class order
+    for (int b = 1; b < nbeta; ++b) canon_row[b] = canon_row[b - 1] + C.ncols[betas[b - 1].pc];
     int pb_run = 0;
     C.chunk_s0.push_back(0); C.chunk_t0.push_back(0);
     for (int ch = 0; ch < nchunk; ++ch) {
@@ -243,6 +247,11 @@ inline void build_class4_tables(const ShellTab& T, int La, int Lb, int Lc, int L
             tab[C.jinfo_off + 4 * pc + 1] = (unsigned)n;
         }
         if (ch == 0) Rb0 = Rb;
+        C.chunk_c0.push_back((int)C.canon.size());
+        C.canon.resize(C.canon.size() + slots);
+        for (int b = 0; b < nbeta; ++b)
+            if (Rb[b] >= 0)
+                for (int k = 0; k < C.ncols[betas[b].pc]; ++k) C.canon[C.chunk_c0.back() + Rb[b] + k] = (unsigned)(canon_row[b] + k);
         C.chunk_ni.push_back(slots);
         C.itmax = std::max(C.itmax, slots);
         C.nint += slots;
@@ -338,6 +347,7 @@ inline void build_class4_tables(const ShellTab& T, int La, int Lb, int Lc, int L
             }
         }
     }
+    C.chunk_c0.push_back((int)C.canon.size());
     if (with_fill) {
         C.chunk_f0.push_back((int)C.fill.size() / 2);
         const int nf = (int)C.fill.size() / 2;
@@ -480,6 +490,23 @@ inline void build_class4_tables(const ShellTab& T, int La, int Lb, int Lc, int L
     C.uniq[5] = (La == Lb && Lb == Lc && Lc == Ld) ? count(true, true, true) : 0;
 }
 
+// Integral store: the share of one job that rank `rank` of `n` evaluates when the launch deals flat units by U = rank (mod n) and the job's
+// nwi work items form the units unit0 .. unit0 + ceil(nwi / chunk) - 1 (shell4_store_row): rows to allocate (owned units x chunk), work items
+// among them (the last unit may be partial) and ubase = (first owned unit) / n.
+struct StoreShare { long long rows = 0, items = 0, ubase = 0; };
+inline StoreShare shell4_store_share(long long nwi, int chunk, long long unit0, int rank, int n) {
+    StoreShare S;
+    const long long nunits = (nwi + chunk - 1) / chunk, end = unit0 + nunits;
+    const long long first = unit0 + ((rank - unit0 % n) % n + n) % n;
+    S.ubase = first / n;
+    if (first >= end) return S;
+    const long long owned = (end - 1 - first) / n + 1;
+    S.rows = owned * chunk;
+    S.items = S.rows;
+    if ((end - 1 - first) % n == 0) S.items -= nunits * chunk - nwi;      // the job's last unit is this rank's and is partial
+    return S;
+}
+
 // View of the tables with the given base pointers (host vectors for the CPU test build, device copies for the GPU).
 template <class PtrOf>
 inline Class4Dev class4_view(const Class4Host& C, PtrOf ptr) {
@@ -501,6 +528,7 @@ inline Class4Dev class4_view(const Class4Host& C, PtrOf ptr) {
     V.acc = ptr(C.acc); V.pmap = ptr(C.pmap); V.omap = ptr(C.omap);
     V.jst_ptr = ptr(C.jst_ptr); V.jst_list = ptr(C.jst_list); V.jflush = ptr(C.jflush); V.njfl = (int)C.jflush.size();
     V.nfill = (int)C.fill.size() / 2; V.fill = ptr(C.fill); V.chunk_f0 = ptr(C.chunk_f0); V.fperm = ptr(C.fperm);
+    V.nint = C.nint; V.canon = ptr(C.canon); V.chunk_c0 = ptr(C.chunk_c0);
     return V;
 }
 

@@ -116,12 +116,17 @@ struct tuna_ctx {
     cudaEvent_t ev_fork = nullptr, ev_join[NAUX] = {};
     // generation-4 shell engine (shell4.cuh): per-class tables and the job list; the pair data above is shared
     struct ClassTab4Dev { Class4Host host; Class4Dev view; DevBuf<unsigned char> blob; };
-    struct Job4Host { Shell4Job job; int G = 1, threads = 128, gpc = 1, nb = 1; size_t smem = 0; double allowed = 0; bool own_launch = true; };
+    struct Job4Host { Shell4Job job; int G = 1, threads = 128, gpc = 1, nb = 1; size_t smem = 0; double allowed = 0; bool own_launch = true;
+                      int cb = 0, ck = 0;            // bra / ket pair class
+                      uint64_t list_sum = 0;         // checksum of the kept quartet list (item prefix): the integral store's validity key
+                      double cost_per_byte = 0;      // estimated phase 0-4 work of a work item over the bytes of its stored row
+                      long long unit0 = 0; };        // flat index of the job's first unit in its launch (grouped jobs: the unit prefix)
     std::map<int, ClassTab4Dev> class_tabs4;     // key La | Lb<<4 | Lc<<8 | Ld<<12 | nD<<16
     // job lists are cached per (threshold, densities per pass, rank count): a build with nD = 5 runs passes of 2, 2 and 1 densities, and
     // direct SCF alternates between thresholds rarely - none of that may rebuild lists or reallocate inside a Fock build
     struct Group4 { int G = 1, threads = 128, njobs = 0, job_off = 0, ctas_per_sm = 1; long long nunits = 0; size_t smem = 0;
-                    DevBuf<Shell4Job> d_jobs; DevBuf<long long> d_unit_prefix; };      // light jobs of one group size in one persistent launch
+                    DevBuf<Shell4Job> d_jobs; DevBuf<long long> d_unit_prefix;         // light jobs of one group size in one persistent launch
+                    std::vector<int> members; std::vector<Shell4Job> host_jobs; };     // indices into JobSet4::jobs, the descriptors as in d_jobs
     struct JobSet4 { double tau = -1.0, dens_bound = 0.0; int nD = 0, shard_n = 0; std::vector<Job4Host> jobs; std::vector<Group4> groups; DevBuf<long long> d_prefix;
                      // fill job set (nD == 0): scratch rows of all work items, every job's descriptor and the prefix of (shell quartet, fill entry) counts for the scatter pass
                      DevBuf<double> d_scratch; DevBuf<Shell4Job> d_all_jobs; DevBuf<long long> d_scatter_pre; long long scatter_total = 0;
@@ -140,6 +145,15 @@ struct tuna_ctx {
     CsrDev Uf, Uft;                 // U * diag(f) and its transpose: per-component norms folded into the rotation
     int direct_engine = 1;          // 1 = shell engine when the basis groups into shells, 0 = per-component kernel
 
+    // integral store (semi-direct J/K, tuna_set_integral_store): the contracted integral buffers of whole class jobs, one row per work
+    // item of this rank, planned at the first direct build after the store was set or dropped and filled by that build
+    struct StoreEntry { int cb, ck, psplit, chunk, nint; uint64_t list_sum; long long unit0, base, items; bool filled; };
+    int64_t store_budget = 0;        // bytes asked for; 0 = off
+    bool store_planned = false;
+    std::vector<StoreEntry> store;
+    DevBuf<double> d_store;
+    int64_t store_replays = 0, store_items_last = 0;
+    bool store_served = false;       // a job of the current build ran from the store
 };
 
 #define CK(call)                                                                                   \
@@ -172,6 +186,7 @@ static uint64_t checksum(const void* p, size_t bytes, uint64_t h = 1469598103934
 static int check_pair_symmetry(tuna_ctx* ctx);
 static int ensure_shell4(tuna_ctx* ctx, double tau, int nD);
 static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const double* Psym, double* Jc, double* Kc, double tau, long long fix_lo);
+static void drop_store(tuna_ctx* ctx);
 
 
 // Opt-in to more than 48 KB of dynamic shared memory.  The attribute is PER DEVICE (a process may hold contexts on several GPUs), so the
@@ -815,7 +830,8 @@ struct DevPolicy {
     __device__ __forceinline__ static void sync_cta() { __syncthreads(); }
     __device__ __forceinline__ static int cta_thread() { return threadIdx.x; }
     __device__ __forceinline__ static int cta_threads() { return blockDim.x; }
-    // fill mode: index of the work item header hq points to (the unit's first work item is kept behind the headers, see shell4_unit)
+    // fill mode and integral store: index of the work item header hq points to (the unit's first work item is kept behind the headers,
+    // see shell4_unit)
     __device__ __forceinline__ static long long work_item_of(const Shell4Job& J, const Quartet4* hq) {
         extern __shared__ double smem_all[];
         const Quartet4* hdr0 = reinterpret_cast<const Quartet4*>(smem_all + J.hdr_off);
@@ -841,8 +857,8 @@ struct DevPolicy {
 #define TUNA_SHELL4_REGS 80
 #endif
 // One CTA work unit: decode the unit's work items ONCE (item -> bra / ket pair, Schwarz test, degeneracy weight, record offsets) into the
-// shared-memory headers, then let the CTA's groups take them NB at a time.
-template <int GG, int NB>
+// shared-memory headers, then let the CTA's groups take them NB at a time.  SEMI: see shell4_quartets.
+template <int GG, int NB, bool SEMI>
 __device__ __forceinline__ void shell4_unit(const Shell4Job& J, const ShellData& D, long long unit, int nD, const double* __restrict__ Pf,
                                             const double* __restrict__ Psym, double* Jf, double* Kf, int ncart, double tau, double dmax,
                                             double* smem_all, int& tab_chunk, double& done) {
@@ -863,7 +879,7 @@ __device__ __forceinline__ void shell4_unit(const Shell4Job& J, const ShellData&
             if (J.item_prefix[mid] <= first_item) lo = mid; else hi = mid;
         }
         s_ib0 = lo;
-        *reinterpret_cast<long long*>(reinterpret_cast<char*>(hdr + CH) + 8) = first;      // read by DevPolicy::work_item_of (fill mode)
+        *reinterpret_cast<long long*>(reinterpret_cast<char*>(hdr + CH) + 8) = first;      // read by DevPolicy::work_item_of (fill mode, integral store)
     }
     __syncthreads();
     for (int k = threadIdx.x; k < CH; k += blockDim.x) {
@@ -877,25 +893,26 @@ __device__ __forceinline__ void shell4_unit(const Shell4Job& J, const ShellData&
             while (J.item_prefix[ib + 1] <= item) ++ib;
             const int pab = J.bra_list[ib], pcd = J.ket_list[(int)(item - J.item_prefix[ib])];
             h.active = !(tau > 0.0 && D.pairQ[pab] * D.pairQ[pcd] * dmax < tau);
+            if (SEMI && !h.active && J.store_mode == S4_STORE) h.active = S4_ONLY_STORE;      // stored for later builds, not digested in this one
             h.shA = D.pairA[pab]; h.shB = D.pairB[pab]; h.shC = D.pairA[pcd]; h.shD = D.pairB[pcd];
             const bool ab = h.shA == h.shB, cd = h.shC == h.shD, dg = pab == pcd;
             h.w = J.fill_scratch ? 1.0 : (ab ? 0.5 : 1.0) * (cd ? 0.5 : 1.0) * (dg ? 0.5 : 1.0);      // fill mode stores plain integrals
             h.recA = D.pair_rec[pab]; h.recC = D.pair_rec[pcd];
             if (h.active) {
                 h.pA = D.rec[h.recA]; h.zA = D.rec[h.recA + 1]; h.pC = D.rec[h.recC]; h.zC = D.rec[h.recC + 1];
-                if (pchunk == 0) done += J.uniq[dg ? (ab ? 5 : 4) : (ab ? (cd ? 3 : 1) : (cd ? 2 : 0))];
+                if (pchunk == 0 && (!SEMI || h.active == 1)) done += J.uniq[dg ? (ab ? 5 : 4) : (ab ? (cd ? 3 : 1) : (cd ? 2 : 0))];
             }
         }
         hdr[k] = h;
     }
     __syncthreads();
     for (int k0 = 0; k0 < CH; k0 += gpc * NB)
-        shell4_quartets<DevPolicy<GG>, NB>(J, D, hdr + k0 + gid * NB, sm, tab, tab_chunk, nD, Pf, Psym, Jf, Kf, ncart);
+        shell4_quartets<DevPolicy<GG>, NB, SEMI>(J, D, hdr + k0 + gid * NB, sm, tab, tab_chunk, nD, Pf, Psym, Jf, Kf, ncart);
 }
 
 // Heavy class jobs: one job per launch, the descriptor travels as a kernel parameter (constant bank / uniform registers).  A CTA work
 // unit (= multi-GPU sharding unit) is J.chunk consecutive work items.
-template <int GG, int NB, int REGS = TUNA_SHELL4_REGS>
+template <int GG, int NB, int REGS = TUNA_SHELL4_REGS, bool SEMI = false>
 __global__ void __launch_bounds__((GG > 128) ? GG : 128, 65536 / (((GG > 128) ? GG : 128) * REGS))
 k_shell4_one(Shell4Job J, ShellData D, int nD, const double* __restrict__ Pf, const double* __restrict__ Psym, double* Jf, double* Kf, int ncart,
              double tau, const unsigned long long* scalars, double* evaluated, int rank, int nranks) {
@@ -906,7 +923,7 @@ k_shell4_one(Shell4Job J, ShellData D, int nD, const double* __restrict__ Pf, co
     int tab_chunk = 0;
     double done = 0.0;
     for (long long gc = (long long)blockIdx.x * nranks + rank; gc < nunit; gc += (long long)gridDim.x * nranks)
-        shell4_unit<GG, NB>(J, D, gc, nD, Pf, Psym, Jf, Kf, ncart, tau, dmax, smem_all, tab_chunk, done);
+        shell4_unit<GG, NB, SEMI>(J, D, gc, nD, Pf, Psym, Jf, Kf, ncart, tau, dmax, smem_all, tab_chunk, done);
     if (done != 0.0) atomicAdd(reinterpret_cast<unsigned long long*>(evaluated), (unsigned long long)(done + 0.5));      // integer counter: no FP64 atomics in the engine
 }
 
@@ -914,7 +931,7 @@ k_shell4_one(Shell4Job J, ShellData D, int nD, const double* __restrict__ Pf, co
 // the launch count (N2/cc-pVTZ: 231 class jobs of ~10 us each).  The work units of the jobs form one flat list (unit_prefix); a CTA walks
 // it with a grid stride (dealt round-robin to ranks like the single-job kernel) and keeps the descriptor of its current job in shared
 // memory, reloading descriptor and digestion tables when it crosses into the next job.
-template <int GG, int NB>
+template <int GG, int NB, bool SEMI = false>
 __global__ void __launch_bounds__((GG > 128) ? GG : 128, 65536 / (((GG > 128) ? GG : 128) * TUNA_SHELL4_REGS))
 k_shell4_multi(const Shell4Job* __restrict__ jobs, const long long* __restrict__ unit_prefix, int njobs, int job_off, ShellData D, int nD,
                const double* __restrict__ Pf, const double* __restrict__ Psym, double* Jf, double* Kf, int ncart, double tau,
@@ -940,7 +957,7 @@ k_shell4_multi(const Shell4Job* __restrict__ jobs, const long long* __restrict__
             shell4_load_tables<NB>(J.ct, 0, reinterpret_cast<unsigned*>(smem_all + J.tab_off), threadIdx.x, blockDim.x, J.oIt, J.oP);
             cur = lo; tab_chunk = 0;
         }
-        shell4_unit<GG, NB>(J, D, u - unit_prefix[lo], nD, Pf, Psym, Jf, Kf, ncart, tau, dmax, smem_all, tab_chunk, done);
+        shell4_unit<GG, NB, SEMI>(J, D, u - unit_prefix[lo], nD, Pf, Psym, Jf, Kf, ncart, tau, dmax, smem_all, tab_chunk, done);
     }
     if (done != 0.0) atomicAdd(reinterpret_cast<unsigned long long*>(evaluated), (unsigned long long)(done + 0.5));      // integer counter: no FP64 atomics in the engine
 }
@@ -1279,6 +1296,7 @@ int tuna_set_basis(tuna_ctx* ctx, int ncart, const double* origins_z, const int3
     ctx->U_shell_blocks = false;
     build_shell_tab(ctx->stab);
     ctx->shell_ready = false;
+    drop_store(ctx);
     ctx->jobsets4.clear();
     ctx->cur_jobset4 = -1;
     detect_shells(ctx->hb, ctx->stab, ctx->ss);     // ss.ok == false -> direct mode uses the per-component kernel
@@ -1292,6 +1310,7 @@ int tuna_set_transform(tuna_ctx* ctx, int nbf, const double* U) try {
     if (ctx->ncart == 0) FAIL(TUNA_ERR_STATE, "tuna_set_transform: call tuna_set_basis first");
     if (nbf <= 0 || !U) FAIL(TUNA_ERR_ARG, "tuna_set_transform: bad arguments");
     CK(cudaSetDevice(ctx->device));
+    drop_store(ctx);
     const int nc = ctx->ncart;
     std::vector<double> u(U, U + (size_t)nbf * nc), ut((size_t)nc * nbf);
     for (int p = 0; p < nbf; ++p)
@@ -1804,10 +1823,32 @@ int tuna_jk_stored(tuna_ctx* ctx, int nD, const double* P, double* J, double* K)
     return TUNA_OK;
 } TUNA_CATCH
 
-int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks) {
+int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks) try {
     if (!ctx) return TUNA_ERR_ARG;
     if (nranks < 1 || rank < 0 || rank >= nranks) FAIL(TUNA_ERR_ARG, "tuna_set_shard: bad rank / nranks");
+    CK(cudaSetDevice(ctx->device));
+    drop_store(ctx);            // the store holds the rows of this rank's units only
     ctx->shard_rank = rank; ctx->shard_n = nranks;
+    return TUNA_OK;
+} TUNA_CATCH
+
+int tuna_set_integral_store(tuna_ctx* ctx, int64_t budget_bytes) try {
+    if (!ctx) return TUNA_ERR_ARG;
+    if (budget_bytes < 0) FAIL(TUNA_ERR_ARG, "tuna_set_integral_store: negative budget");
+    CK(cudaSetDevice(ctx->device));
+    if (budget_bytes != ctx->store_budget) drop_store(ctx);
+    ctx->store_budget = budget_bytes;
+    return TUNA_OK;
+} TUNA_CATCH
+
+int tuna_integral_store_info(const tuna_ctx* ctx, int64_t info[4]) {
+    if (!ctx || !info) return TUNA_ERR_ARG;
+    int64_t items = 0;
+    for (const auto& e : ctx->store) if (e.filled) items += e.items;
+    info[0] = items > 0 ? (int64_t)(ctx->d_store.capacity() * sizeof(double)) : 0;
+    info[1] = items;
+    info[2] = ctx->store_items_last;
+    info[3] = ctx->store_replays;
     return TUNA_OK;
 }
 
@@ -2152,6 +2193,7 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     const size_t o_tm = add(C.terms.data(), C.terms.size() * 4), o_tp = add(C.tptr.data(), C.tptr.size() * 4);
     const size_t o_wf = add(C.wfl.data(), C.wfl.size() * 4), o_wl = add(C.wlist.data(), C.wlist.size() * 2);
     const size_t o_fl = add(C.fill.data(), C.fill.size() * 4), o_f0 = add(C.chunk_f0.data(), C.chunk_f0.size() * 4), o_fp = add(C.fperm.data(), C.fperm.size() * 4);
+    const size_t o_cn = add(C.canon.data(), C.canon.size() * 4), o_c0 = add(C.chunk_c0.data(), C.chunk_c0.size() * 4);
     std::vector<unsigned char> host(total, 0);
     for (const Piece& p : pieces) if (p.bytes) std::memcpy(host.data() + p.off, p.src, p.bytes);
     GROW(E.blob, total);
@@ -2167,6 +2209,7 @@ static int get_class4_tables(tuna_ctx* ctx, int La, int Lb, int Lc, int Ld, int 
     V.terms = (const unsigned*)(E.blob + o_tm); V.tptr = (const unsigned*)(E.blob + o_tp);
     V.wfl = (const unsigned*)(E.blob + o_wf); V.wlist = (const unsigned short*)(E.blob + o_wl);
     V.fill = (const unsigned*)(E.blob + o_fl); V.chunk_f0 = (const int*)(E.blob + o_f0); V.fperm = (const unsigned*)(E.blob + o_fp);
+    V.canon = (const unsigned*)(E.blob + o_cn); V.chunk_c0 = (const int*)(E.blob + o_c0);
     *out = &ctx->class_tabs4.emplace(key, std::move(E)).first->second;
     return TUNA_OK;
 }
@@ -2178,6 +2221,74 @@ static int shell4_one_regs(const tuna_ctx::Job4Host& jh) {
     static const bool tiers = !(getenv("TUNA_B200_REG_TIER") && atoi(getenv("TUNA_B200_REG_TIER")) == 0);
     const size_t by_smem = std::max<size_t>(1, (size_t)(228 * 1024) / (jh.smem + 1024));
     return tiers && jh.G == 256 && jh.nb <= 2 && by_smem * jh.threads * 128 <= 65536 ? 128 : TUNA_SHELL4_REGS;
+}
+
+// ---- integral store (semi-direct J/K) --------------------------------------------------------------------------------------------
+// Estimated phase 0-4 work of one work item (arbitrary units, one per FMA-sized step): the Boys values of phase 0, the entries of phases
+// 1-3 and the assembly FMAs of the phase-4 tiles, per primitive quartet, times the primitive quartets of the item.
+static double store_cost_per_item(const Class4Host& C, const Shell4Job& J) {
+    const int Ltot = C.La + C.Lb + C.Lc + C.Ld;
+    double w = 40.0 * (Ltot + 1) + 4.0 * (C.t_rt.size() + C.t_xy.size() + C.t_u.size() / 2 + C.t_s.size() / 2);
+    for (size_t t = 0; t < C.p4.size(); t += 4) {
+        const unsigned w2 = C.p4[t + 2];
+        const int nx = (int)((w2 >> 4) & 15) - (int)(w2 & 15) + 1, ny = (w2 >> 12) & 15;
+        w += nx * (2.0 * ny + 2.0);
+    }
+    return w * (double)J.clen * (double)J.klen;
+}
+
+// This rank's share of job jh: the units its launch deals to it (shell4_store_share, shell4_store_row).
+static StoreShare store_share(const tuna_ctx* ctx, const tuna_ctx::Job4Host& jh) {
+    return shell4_store_share(jh.job.nitems * jh.job.psplit, jh.job.chunk, jh.unit0, ctx->shard_rank, ctx->shard_n);
+}
+
+static void drop_store(tuna_ctx* ctx) {
+    if (ctx->d_store) cudaStreamSynchronize(ctx->stream);      // no build in flight reads the rows any more
+    ctx->store.clear();
+    ctx->d_store.reset();
+    ctx->store_planned = false;
+}
+
+// Plans the store from the current job set: whole jobs by decreasing cost per byte while they fit the budget, the budget clamped to the
+// device's free memory less headroom for the build's own buffers.  One allocation; if it fails the store stays empty (the builds run
+// direct) until the budget is set again.
+static void plan_store(tuna_ctx* ctx) {
+    ctx->store_planned = true;
+    ctx->store.clear();
+    const auto& jobs = ctx->jobsets4[ctx->cur_jobset4].jobs;
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); return; }
+    const size_t headroom = std::max<size_t>((size_t)2 << 30, total_b / 16);
+    const long long budget = std::min<long long>(ctx->store_budget, free_b > headroom ? (long long)(free_b - headroom) : 0);
+    std::vector<int> order(jobs.size());
+    for (size_t j = 0; j < jobs.size(); ++j) order[j] = (int)j;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return jobs[x].cost_per_byte > jobs[y].cost_per_byte; });
+    long long used = 0;      // doubles
+    for (int j : order) {
+        const tuna_ctx::Job4Host& jh = jobs[j];
+        const StoreShare sh = store_share(ctx, jh);
+        const long long need = sh.rows * jh.job.ct.nint;
+        if (need == 0 || (used + need) * 8 > budget) continue;
+        ctx->store.push_back({jh.cb, jh.ck, jh.job.psplit, jh.job.chunk, jh.job.ct.nint, jh.list_sum, jh.unit0, used, sh.items, false});
+        used += need;
+    }
+    if (used == 0) return;
+    std::string err;
+    if (ctx->d_store.grow((size_t)used, err) != TUNA_OK) ctx->store.clear();      // optional memory: run direct, report nothing
+}
+
+// Mode of job jh in this build, and its first row.  A stored job whose kept quartet list or split differs from the stored one runs
+// direct, and so does one whose unit size or flat unit offset (own launch or grouped, the group's other jobs) differs on a sharded
+// context, where they decide which units, hence rows, the rank owns.  Such a job is not stored again.
+static int store_mode_of(const tuna_ctx* ctx, const tuna_ctx::Job4Host& jh, long long* base) {
+    for (const auto& e : ctx->store) {
+        if (e.cb != jh.cb || e.ck != jh.ck) continue;
+        if (e.list_sum != jh.list_sum || e.psplit != jh.job.psplit || e.nint != jh.job.ct.nint || (ctx->shard_n > 1 && (e.chunk != jh.job.chunk || e.unit0 != jh.unit0)))
+            return S4_DIRECT;
+        *base = e.base;
+        return e.filled ? S4_REPLAY : S4_STORE;
+    }
+    return S4_DIRECT;
 }
 
 // Job list of the shell-quartet engine for threshold tau and nD densities.
@@ -2240,6 +2351,9 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             if (fill) { J.fill_base = fill_run; fill_run += J.nitems * J.psplit * J.ct.nfill; }
             jh.allowed = (double)ctd->host.allowed;
             for (int u = 0; u < 6; ++u) J.uniq[u] = ctd->host.uniq[u];
+            jh.cb = cb; jh.ck = ck;
+            jh.list_sum = checksum(prefix.data(), prefix.size() * sizeof(long long), (uint64_t)J.nitems);
+            jh.cost_per_byte = store_cost_per_item(ctd->host, J) / (8.0 * ctd->host.nint);
             int nb = env_nb ? atoi(env_nb) : 2;
             if (nb != 1 && nb != 2 && nb != 4) nb = 2;
             while (nb > 1 && (size_t)nb * J.total * 8 > nb_bytes) nb >>= 1;
@@ -2305,17 +2419,21 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
         }
         for (int G = 256; G >= 1; G >>= 1) {
             std::vector<Shell4Job> js;
+            std::vector<int> members;
             std::vector<long long> up(1, 0);
             size_t max_smem = 0;
             int threads = 128;
-            for (const auto& jh : jobs4) {
+            for (size_t j = 0; j < jobs4.size(); ++j) {
+                const auto& jh = jobs4[j];
                 if (jh.own_launch || jh.G != G) continue;
                 js.push_back(jh.job);
+                members.push_back((int)j);
                 up.push_back(up.back() + (jh.job.nitems * jh.job.psplit + jh.job.chunk - 1) / jh.job.chunk);
                 max_smem = std::max(max_smem, jh.smem);
                 threads = jh.threads;
             }
             if (js.size() < 2) { for (auto& jh : jobs4) if (!jh.own_launch && jh.G == G) jh.own_launch = true; continue; }
+            for (size_t i = 0; i < members.size(); ++i) jobs4[members[i]].unit0 = up[i];      // ranks own the group's FLAT units
             tuna_ctx::Group4 g;
             g.G = G; g.threads = threads; g.njobs = (int)js.size(); g.nunits = up.back();
             g.job_off = (int)(((max_smem + 7) / 8 + 1) & ~(size_t)1);
@@ -2326,6 +2444,8 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
             CK(cudaMemcpyAsync(g.d_jobs, js.data(), js.size() * sizeof(Shell4Job), cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaMemcpyAsync(g.d_unit_prefix, up.data(), up.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaStreamSynchronize(ctx->stream));
+            g.members = std::move(members);
+            g.host_jobs = std::move(js);
             JS.groups.push_back(std::move(g));
         }
     }
@@ -2362,11 +2482,11 @@ static int ensure_shell4(tuna_ctx* ctx, double tau, int nD) {
     return TUNA_OK;
 }
 
-template <int GG, int NB, int REGS>
+template <int GG, int NB, int REGS, bool SEMI>
 static cudaError_t launch_shell4_one_r(tuna_ctx* ctx, const tuna_ctx::Job4Host& jh, const ShellData& D, int nD, const double* Pf, const double* Psym,
                                        double* Jf, double* Kf, double tau, cudaStream_t stream, long long blocks) {
-    if (cudaError_t e = opt_in_smem<k_shell4_one<GG, NB, REGS>>(ctx); e != cudaSuccess) return e;
-    k_shell4_one<GG, NB, REGS><<<(int)blocks, jh.threads, jh.smem, stream>>>(jh.job, D, nD, Pf, Psym, Jf, Kf, ctx->ncart, tau, ctx->d_scalars, ctx->d_eval,
+    if (cudaError_t e = opt_in_smem<k_shell4_one<GG, NB, REGS, SEMI>>(ctx); e != cudaSuccess) return e;
+    k_shell4_one<GG, NB, REGS, SEMI><<<(int)blocks, jh.threads, jh.smem, stream>>>(jh.job, D, nD, Pf, Psym, Jf, Kf, ctx->ncart, tau, ctx->d_scalars, ctx->d_eval,
                                                                             ctx->shard_rank, ctx->shard_n);
     ctx->launches++;
     return cudaGetLastError();
@@ -2381,10 +2501,23 @@ static cudaError_t launch_shell4_one(tuna_ctx* ctx, const tuna_ctx::Job4Host& jh
     const size_t by_smem = std::max<size_t>(1, (size_t)(228 * 1024) / (jh.smem + 1024));
     const size_t by_thr = std::max<size_t>(1, 2048 / jh.threads);
     blocks = std::min<long long>(blocks, (long long)ctx->sm_count * (long long)std::min(by_smem, by_thr) * 2);
+    const bool semi = jh.job.store_mode != S4_DIRECT;      // store pass or replay: the kernel variant with the integral-store paths
     if constexpr (GG == 256 && NB <= 2) {
-        if (shell4_one_regs(jh) == 128) return launch_shell4_one_r<GG, NB, 128>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
+        if (shell4_one_regs(jh) == 128)
+            return semi ? launch_shell4_one_r<GG, NB, 128, true>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks)
+                        : launch_shell4_one_r<GG, NB, 128, false>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
     }
-    return launch_shell4_one_r<GG, NB, TUNA_SHELL4_REGS>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
+    return semi ? launch_shell4_one_r<GG, NB, TUNA_SHELL4_REGS, true>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks)
+                : launch_shell4_one_r<GG, NB, TUNA_SHELL4_REGS, false>(ctx, jh, D, nD, Pf, Psym, Jf, Kf, tau, stream, blocks);
+}
+
+template <int GG, bool SEMI>
+static cudaError_t launch_shell4_multi(tuna_ctx* ctx, const tuna_ctx::Group4& g, const ShellData& D, int nD, const double* Pc, const double* Psym,
+                                       double* Jc, double* Kc, double tau, cudaStream_t st, long long blocks) {
+    if (cudaError_t e = opt_in_smem<k_shell4_multi<GG, 2, SEMI>>(ctx); e != cudaSuccess) return e;
+    k_shell4_multi<GG, 2, SEMI><<<(int)blocks, g.threads, g.smem, st>>>(g.d_jobs, g.d_unit_prefix, g.njobs, g.job_off, D, nD, Pc, Psym, Jc, Kc, ctx->ncart,
+                                                                     tau, ctx->d_scalars, ctx->d_eval, ctx->shard_rank, ctx->shard_n);
+    return cudaGetLastError();
 }
 
 static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const double* Psym, double* Jc, double* Kc, double tau, long long fix_lo) {
@@ -2392,11 +2525,46 @@ static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const dou
     D.pairA = ctx->d_pairA; D.pairB = ctx->d_pairB; D.pair_rec = ctx->d_pair_rec; D.rec = ctx->d_rec; D.pairQ = ctx->d_pairQ;
     D.sh_ao = ctx->d_sh_ao; D.boys = ctx->d_boys; D.herm = ctx->d_herm;
     D.fix_lo = fix_lo;
+    tuna_ctx::JobSet4& JS = ctx->jobsets4[ctx->cur_jobset4];
+    // integral store: every job's mode in this build (direct / store pass / replay); the fill job set (nD = 0) never uses it
+    const bool use_store = nD > 0 && ctx->store_budget > 0;
+    if (use_store && !ctx->store_planned) plan_store(ctx);
+    std::vector<int> modes(JS.jobs.size(), S4_DIRECT);
+    std::vector<long long> bases(JS.jobs.size(), 0);
+    if (use_store) {
+        long long items_all = 0;
+        for (size_t j = 0; j < JS.jobs.size(); ++j) {
+            modes[j] = store_mode_of(ctx, JS.jobs[j], &bases[j]);
+            items_all += store_share(ctx, JS.jobs[j]).items;
+        }
+        ctx->store_items_last = items_all;
+    }
+    auto with_store = [&](Shell4Job& J, size_t j) {
+        J.store = modes[j] == S4_DIRECT ? nullptr : ctx->d_store.get();
+        J.store_base = bases[j]; J.store_mode = modes[j]; J.store_nranks = ctx->shard_n;
+        J.store_unit0 = JS.jobs[j].unit0; J.store_ubase = store_share(ctx, JS.jobs[j]).ubase;
+    };
+    for (auto& g : JS.groups) {          // grouped descriptors live on the device: re-upload when a job's store fields change
+        bool changed = false;
+        for (size_t i = 0; i < g.members.size(); ++i) {
+            Shell4Job want = g.host_jobs[i];
+            with_store(want, (size_t)g.members[i]);
+            Shell4Job& have = g.host_jobs[i];
+            if (want.store != have.store || want.store_base != have.store_base || want.store_mode != have.store_mode || want.store_nranks != have.store_nranks ||
+                want.store_unit0 != have.store_unit0 || want.store_ubase != have.store_ubase) {
+                have = want;
+                changed = true;
+            }
+        }
+        if (changed) CK(cudaMemcpyAsync(g.d_jobs, g.host_jobs.data(), g.host_jobs.size() * sizeof(Shell4Job), cudaMemcpyHostToDevice, ctx->stream));
+    }
     CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
     for (int a = 0; a < ctx->naux; ++a) CK(cudaStreamWaitEvent(ctx->aux[a], ctx->ev_fork, 0));
     int jn = 0;
-    for (const auto& jh : ctx->jobsets4[ctx->cur_jobset4].jobs) {
-        if (!jh.own_launch) continue;
+    for (size_t j = 0; j < JS.jobs.size(); ++j) {
+        if (!JS.jobs[j].own_launch) continue;
+        tuna_ctx::Job4Host jh = JS.jobs[j];
+        with_store(jh.job, j);
         cudaStream_t st = ctx->aux[jn++ % ctx->naux];
         cudaError_t e;
 #define TUNA_ONE4(GV) (jh.nb == 4 ? launch_shell4_one<GV, 4>(ctx, jh, D, nD, Pc, Psym, Jc, Kc, tau, st) \
@@ -2416,18 +2584,16 @@ static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const dou
 #undef TUNA_ONE4
         if (e != cudaSuccess) FAIL(TUNA_ERR_CUDA, std::string("k_shell4_one launch: ") + cudaGetErrorString(e));
     }
-    for (const auto& g : ctx->jobsets4[ctx->cur_jobset4].groups) {
+    for (const auto& g : JS.groups) {
         cudaStream_t st = ctx->aux[jn++ % ctx->naux];
         long long blocks = (g.nunits - ctx->shard_rank + ctx->shard_n - 1) / ctx->shard_n;       // units owned by this rank
         if (blocks <= 0) continue;
         blocks = std::min<long long>(blocks, (long long)ctx->sm_count * g.ctas_per_sm);
         cudaError_t e = cudaSuccess;
-#define TUNA_MULTI4(GV) \
-        if ((e = opt_in_smem<k_shell4_multi<GV, 2>>(ctx)) == cudaSuccess) { \
-            k_shell4_multi<GV, 2><<<(int)blocks, g.threads, g.smem, st>>>(g.d_jobs, g.d_unit_prefix, g.njobs, g.job_off, D, nD, Pc, Psym, Jc, Kc, ctx->ncart, tau, \
-                                                                       ctx->d_scalars, ctx->d_eval, ctx->shard_rank, ctx->shard_n); \
-            e = cudaGetLastError(); \
-        }
+        bool semi = false;                              // a job of the group stores or replays: the kernel variant with those paths
+        for (const Shell4Job& hj : g.host_jobs) semi |= hj.store_mode != S4_DIRECT;
+#define TUNA_MULTI4(GV) e = semi ? launch_shell4_multi<GV, true>(ctx, g, D, nD, Pc, Psym, Jc, Kc, tau, st, blocks) \
+                                 : launch_shell4_multi<GV, false>(ctx, g, D, nD, Pc, Psym, Jc, Kc, tau, st, blocks);
         switch (g.G) {
             case 1: TUNA_MULTI4(1) break;
             case 2: TUNA_MULTI4(2) break;
@@ -2446,6 +2612,13 @@ static int launch_shell4_jobs(tuna_ctx* ctx, int nD, const double* Pc, const dou
     for (int a = 0; a < ctx->naux; ++a) {
         CK(cudaEventRecord(ctx->ev_join[a], ctx->aux[a]));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[a], 0));
+    }
+    // the store pass is enqueued: later builds (stream-ordered behind it) replay those jobs
+    for (size_t j = 0; j < JS.jobs.size(); ++j) {
+        if (modes[j] == S4_REPLAY) ctx->store_served = true;
+        if (modes[j] != S4_STORE) continue;
+        for (auto& e : ctx->store)
+            if (e.cb == JS.jobs[j].cb && e.ck == JS.jobs[j].ck) e.filled = true;
     }
     return TUNA_OK;
 }
@@ -2544,12 +2717,14 @@ static int jk_direct_core(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
     if (nD <= 0 || nD > 16 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct: bad arguments (1 <= nD <= 16)");
     const int per = direct_pass_densities(ctx, nD);
     const size_t nn = (size_t)ctx->nbf * ctx->nbf;
+    ctx->store_served = false;
     for (int d0 = 0; d0 < nD; d0 += per) {
         const int nd = std::min(per, nD - d0);
         int rc = jk_direct_accumulate(ctx, nd, dP + d0 * nn, tau);
         if (!rc) rc = jk_direct_finish(ctx, nd, (anti_mask >> d0) & ((1u << nd) - 1u), dJ ? dJ + d0 * nn : nullptr, dK ? dK + d0 * nn : nullptr);
         if (rc) return rc;
     }
+    if (ctx->store_served) ++ctx->store_replays;
     return TUNA_OK;
 }
 
@@ -2664,6 +2839,7 @@ static int jk_direct_group_core(tuna_ctx* const* ctxs, int nctx, int nD, const d
     const int per = direct_pass_densities(ctx, nD);
     const size_t nn = (size_t)nb * nb;
     int rc;
+    for (int r = 0; r < nctx; ++r) ctxs[r]->store_served = false;
     for (int d0 = 0; d0 < nD; d0 += per) {
         const int nd = std::min(per, nD - d0);
         const size_t nacc = (size_t)nd * nc * nc, words = fixed ? 4 * nacc : 2 * nacc;     // one rank's accumulators
@@ -2756,6 +2932,8 @@ static int jk_direct_group_core(tuna_ctx* const* ctxs, int nctx, int nD, const d
         if ((rc = jk_direct_finish(ctx, nd, (anti_mask >> d0) & ((1u << nd) - 1u), dJ ? dJ + d0 * nn : nullptr, dK ? dK + d0 * nn : nullptr))) return rc;
         CK(cudaEventRecord(ctx->ev[6][1], ctx->stream));
     }
+    for (int r = 0; r < nctx; ++r)
+        if (ctxs[r]->store_served) ++ctxs[r]->store_replays;
     return TUNA_OK;
 }
 

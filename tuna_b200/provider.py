@@ -28,6 +28,8 @@ from .basis import flatten
 DEFAULT_TAU = float(os.environ.get("TUNA_B200_TAU", "1e-16"))      # Schwarz threshold of direct mode (SURVEY.md 8d)
 _settings = {"mode": os.environ.get("TUNA_B200_MODE", "auto"), "device": int(os.environ.get("TUNA_B200_DEVICE", "0")),
              "stored_fraction": 0.40, "tau": DEFAULT_TAU}
+# semi-direct J/K: direct mode keeps the engine's integrals in up to this fraction of each device's free memory (0 = off)
+_store_fraction = float(os.environ.get("TUNA_B200_STORE_FRACTION", "0.5"))
 _devices = None      # devices of direct J/K (None: _settings["device"] alone); "all" = every visible device, resolved on first use
 
 
@@ -68,11 +70,15 @@ if os.environ.get("TUNA_B200_DEVICES", "").strip():
     _set_devices(os.environ["TUNA_B200_DEVICES"])
 
 
-def configure(mode=None, device=None, tau=None, stored_fraction=None, devices=None):
+def configure(mode=None, device=None, tau=None, stored_fraction=None, devices=None, store_fraction=None):
     """mode: 'stored' (dense tensor on the device), 'direct' (integral-driven J/K) or 'auto' (stored when
     8*ncart^4 bytes fit in `stored_fraction` of free device memory or a post-HF consumer needs the tensor).
     devices: 'all' or a list of ordinals (or a comma list); direct-mode J/K of one Fock build is spread over all of them
-    (DeviceGroup), everything else runs on devices[0].  device=d is devices=[d]."""
+    (DeviceGroup), everything else runs on devices[0].  device=d is devices=[d].
+    store_fraction: direct mode keeps the integrals it evaluates in up to this fraction of each device's free memory and replays
+    them in later Fock builds (semi-direct J/K, bitwise equal to the direct build); 0 = off.  Applies to handles whose first J/K call
+    comes after it."""
+    global _store_fraction
     if mode is not None:
         if mode not in ("stored", "direct", "auto"):
             raise _lib.error_class(f"tuna_b200: unknown mode {mode!r}")
@@ -87,6 +93,10 @@ def configure(mode=None, device=None, tau=None, stored_fraction=None, devices=No
         _settings["tau"] = float(tau)
     if stored_fraction is not None:
         _settings["stored_fraction"] = float(stored_fraction)
+    if store_fraction is not None:
+        if not 0.0 <= float(store_fraction) <= 1.0:
+            raise _lib.error_class(f"tuna_b200: store_fraction must lie in [0, 1], got {store_fraction!r}")
+        _store_fraction = float(store_fraction)
 
 
 def _free_device_bytes():
@@ -111,6 +121,8 @@ class ERIHandle:
         self.pending_fill = False   # stored mode: the tensor is filled by transform_to_spherical_harmonics, or on first touch as an array
         self._jk_cache = []     # [(P, J, K)] most recent first
         self._group = None      # direct mode over several devices: DeviceGroup built on the first J/K call
+        self._store_for = None  # direct mode: the Context / DeviceGroup whose integral store this handle has enabled
+        self._store_dropped = False     # a dense tensor was materialised: the store stays off so the tensor keeps today's memory
 
     shape = property(lambda self: (self.n,) * 4)
     ndim = 4
@@ -130,6 +142,9 @@ class ERIHandle:
 
     def _materialise_direct(self):
         ctx = self.ctx
+        # the integral store gives its memory back before the dense tensor's size is checked
+        _release_integral_stores([t for t in (ctx, self._group) if t is not None])
+        self._store_for, self._store_dropped = None, True
         if self.basis_kind == "cart" or not hasattr(ctx, "eri_fill_sph"):
             need = 8 * ctx.ncart ** 4
         else:   # the spherical fill: nbf^4 plus the engine's scratch rows, which are about as large as the unique Cartesian integrals
@@ -270,6 +285,7 @@ def _context_for(bfs, cached=True):
     ctx.set_basis(*flat)
     if cached:
         _ctx_cache.insert(0, (dev, key, ctx))
+        _release_integral_stores([c for _, _, c in _ctx_cache[2:]])      # a context leaving the cache keeps no store
         del _ctx_cache[2:]
     return ctx
 
@@ -315,6 +331,7 @@ def _dense_needed(calculation) -> bool:
 
 
 def _choose_mode(n_cart, calculation):
+    _release_integral_stores()                 # a new geometry: earlier handles' stores give their memory back before it is measured
     mode = _settings["mode"]
     if mode != "auto":
         return mode
@@ -426,8 +443,37 @@ def coulomb_and_exchange(P, ERI_AO, want_j=True, want_k=True):
             group.set_basis(*h.ctx.basis_flat)
             group.set_transform(h.ctx.U)
             h._group = group
+        _enable_store(h, h._group, h._group.contexts)
         return h._group.jk_direct(P, _settings["tau"], want_j, want_k)
+    _enable_store(h, h.ctx, [h.ctx])
     return h.ctx.jk_direct(P, _settings["tau"], want_j, want_k)
+
+
+_store_holders = weakref.WeakSet()      # Contexts / DeviceGroups whose integral store a direct-mode handle turned on
+
+
+def _release_integral_stores(targets=None):
+    """Give back the memory of the integral stores the provider turned on (all of them, or those of `targets`).  A new geometry's mode is
+    decided against the free device memory, which a finished handle's store must not hold; a handle whose store was released runs its
+    later builds direct."""
+    for t in list(_store_holders if targets is None else [t for t in targets if t in _store_holders]):
+        if getattr(t, "_h", True):             # a closed Context has nothing left to release
+            t.set_integral_store(0)
+        _store_holders.discard(t)
+
+
+def _enable_store(h, target, contexts):
+    """Semi-direct J/K on the first direct J/K call of a handle: every context of `target` may keep up to store_fraction of its device's
+    free memory (the library clamps it further and allocates only what the stored class jobs need)."""
+    if h._store_for is target or h._store_dropped:
+        return
+    frac = _store_fraction
+    if frac > 0.0:
+        import torch  # plumbing only: device memory query
+        for c in contexts:
+            c.set_integral_store(int(frac * torch.cuda.mem_get_info(c.device)[0]))
+        _store_holders.add(target)
+    h._store_for = target
 
 
 def _cached_jk(P, ERI_AO, which):
