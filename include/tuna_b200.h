@@ -84,12 +84,19 @@ int tuna_jk_stored_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, doub
  * tau <= 0 disables screening.  tuna_jk_direct accepts any real P (a non-symmetric density is split into its symmetric and
  * antisymmetric parts: J[P] = J[S], K[P] = K[S] + K[A]).  tuna_jk_direct_dev REQUIRES symmetric densities and does not check:
  * it builds K = U (Kacc + Kacc^T) U^T, symmetric by construction, so for a non-symmetric P it silently drops K[A].  Callers with
- * possibly asymmetric densities (e.g. guess densities, asymmetric at ~1e-8) use tuna_jk_direct.
+ * possibly asymmetric densities (e.g. guess densities, asymmetric at ~1e-8) use tuna_jk_direct, or tuna_jk_direct_general_dev with
+ * device buffers.
  * The cached quartet lists are pre-screened with tau / (1e3 max(1, max|P|)) for host densities; tuna_jk_direct_dev assumes max|P| <= ~10
- * (scale larger device densities down - J and K are linear in P).  J and K are accumulated as 64-bit integers (order independent):
+ * (scale larger device densities down - J and K are linear in P; tuna_jk_direct_general_dev measures max|P| itself).  J and K are accumulated as 64-bit integers (order independent):
  * repeated builds are bitwise identical; |J|, |K| < 2^42 in the unnormalised Cartesian working basis is required. */
 int tuna_jk_direct(tuna_ctx* ctx, int nD, const double* P, double* J, double* K, double tau);
 int tuna_jk_direct_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, double* dK, double tau);
+/* tuna_jk_direct with DEVICE pointers (dP, dJ, dK on the context's device, enqueued on its stream): any real P, 1 <= nD <= 8, J or K may
+ * be NULL.  max|P| and max|P - P^T| are taken on the device and read back (16 bytes, ONE stream synchronise, the only one of the call);
+ * they set the pre-screening bound and decide the symmetric / antisymmetric split exactly as tuna_jk_direct does on the host, and the split
+ * and the sum K[S] + K[A] run on the device with the host's arithmetic.  J and K are bitwise identical to tuna_jk_direct for the same P,
+ * tau, shard and integral store state.  Everything after the read-back is enqueued without a further synchronise. */
+int tuna_jk_direct_general_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, double* dK, double tau);
 /* Multi-GPU sharding of the quartet list for tuna_jk_direct*: this context evaluates only its share and
  * returns PARTIAL J/K, to be summed over ranks by the caller (one all-reduce per build, SURVEY.md 8e). */
 int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks);
@@ -102,8 +109,13 @@ int tuna_set_shard(tuna_ctx* ctx, int rank, int nranks);
  * transform (ncart, nbf, checksums of the arrays given to tuna_set_basis / tuna_set_transform) or a shard other than (r, nctx).
  * Errors are reported through tuna_last_error(ctxs[0]), the failing rank named. */
 int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* P, double* J, double* K, double tau);
-/* dP, dJ, dK on ctxs[0]'s device, enqueued on ctxs[0]'s stream; symmetric densities only, as tuna_jk_direct_dev. */
+/* dP, dJ, dK on ctxs[0]'s device, enqueued on ctxs[0]'s stream; symmetric densities only, as tuna_jk_direct_dev (any real P:
+ * tuna_jk_direct_group_general_dev). */
 int tuna_jk_direct_group_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau);
+/* tuna_jk_direct_group with DEVICE pointers on ctxs[0]'s device, as tuna_jk_direct_general_dev: the scan, its read-back (one synchronise of
+ * ctxs[0]'s stream), the split and K[S] + K[A] run on ctxs[0].  Bitwise identical to tuna_jk_direct_group and to tuna_jk_direct on one
+ * context; the group's errors are those of tuna_jk_direct_group. */
+int tuna_jk_direct_group_general_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau);
 /* Semi-direct J/K: keep the shell-quartet engine's contracted integrals of whole class jobs in device memory, up to budget_bytes
  * (0, the default, = off), and replay them in later tuna_jk_direct* / tuna_jk_direct_group* builds instead of evaluating them again.
  * The first build after the store is set (or dropped) plans it and fills it while it runs; jobs that do not fit run direct.  The budget

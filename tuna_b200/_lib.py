@@ -19,7 +19,7 @@ EXPORTS = [
     "tuna_jk_stored", "tuna_jk_stored_dev", "tuna_jk_direct", "tuna_jk_direct_dev", "tuna_set_shard", "tuna_get_counts",
     "tuna_last_kernel_ms", "tuna_algorithmic_flops", "tuna_fp64_peak_probe", "tuna_eri_transform", "tuna_eri_transform_dev",
     "tuna_eri_transform_spin_blocked", "tuna_one_electron", "tuna_cross_overlap", "tuna_jk_direct_group", "tuna_jk_direct_group_dev",
-    "tuna_set_integral_store", "tuna_integral_store_info",
+    "tuna_set_integral_store", "tuna_integral_store_info", "tuna_jk_direct_general_dev", "tuna_jk_direct_group_general_dev",
 ]
 
 _lib = None
@@ -76,6 +76,8 @@ def load() -> ctypes.CDLL:
         "tuna_jk_direct_group_dev": (ci, [ctypes.POINTER(vp), ci, ci, vp, vp, vp, cd]),
         "tuna_set_integral_store": (ci, [vp, ctypes.c_int64]),
         "tuna_integral_store_info": (ci, [vp, c_lp]),
+        "tuna_jk_direct_general_dev": (ci, [vp, ci, vp, vp, vp, cd]),
+        "tuna_jk_direct_group_general_dev": (ci, [ctypes.POINTER(vp), ci, ci, vp, vp, vp, cd]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -309,6 +311,14 @@ class Context:
     def jk_direct_dev(self, nD, dP, dJ, dK, tau=1e-16):
         self._ck(self._lib.tuna_jk_direct_dev(self._h, nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ), ctypes.c_void_p(dK), tau))
 
+    def jk_direct_general_dev(self, nD, dP, dJ, dK, tau=1e-16):
+        """jk_direct on device buffers: nD (1-8) densities of any real P at dP, J and K (either may be 0) written to dJ and dK, all
+        on this context's device, enqueued on its stream.  Bitwise equal to jk_direct for the same P.  Synchronises the stream once,
+        to read back max|P| and max|P - P^T|, which decide the screening bound and the symmetric / antisymmetric split
+        (tuna_jk_direct_general_dev)."""
+        self._ck(self._lib.tuna_jk_direct_general_dev(self._h, nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ), ctypes.c_void_p(dK),
+                                                      ctypes.c_double(tau)))
+
     def set_shard(self, rank, nranks):
         self._ck(self._lib.tuna_set_shard(self._h, rank, nranks))
 
@@ -401,9 +411,17 @@ class DeviceGroup:
         return J, K
 
     def jk_direct_dev(self, nD, dP, dJ, dK, tau=1e-16):
-        """Device pointers on devices[0], enqueued on the stream of contexts[0]; symmetric densities only (tuna_jk_direct_dev)."""
+        """Device pointers on devices[0], enqueued on the stream of contexts[0]; symmetric densities only (tuna_jk_direct_dev).
+        Any real P: jk_direct_general_dev."""
         self._ck(self._lib.tuna_jk_direct_group_dev(self._ptrs, len(self.contexts), nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ), ctypes.c_void_p(dK),
                                                     ctypes.c_double(tau)))
+
+    def jk_direct_general_dev(self, nD, dP, dJ, dK, tau=1e-16):
+        """jk_direct on device buffers on devices[0], enqueued on the stream of contexts[0]: any real P, 1 <= nD <= 8, bitwise equal to
+        jk_direct and to one Context's jk_direct_general_dev.  Synchronises that stream once, after the density scan on devices[0]
+        (tuna_jk_direct_group_general_dev)."""
+        self._ck(self._lib.tuna_jk_direct_group_general_dev(self._ptrs, len(self.contexts), nD, ctypes.c_void_p(dP), ctypes.c_void_p(dJ),
+                                                            ctypes.c_void_p(dK), ctypes.c_double(tau)))
 
     def set_integral_store(self, budget_bytes: int):
         """Semi-direct J/K on every rank: each stores its own share of the integrals on its own device, up to budget_bytes each."""

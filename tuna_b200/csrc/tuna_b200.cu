@@ -12,6 +12,8 @@
 //   k_shell4_one / k_shell4_multi          direct J/K: the shell-quartet engine of shell4.cuh (one class job per launch / all light
 //                                          class jobs of one group size in one persistent launch), reproducible integer accumulation
 //   k_jk_direct       per-component direct J/K for bases that do not group into full shells (FP64 atomics)
+//   k_density_scan / k_density_split / k_add_into   device densities of any real P: max|P| and max|P - P^T|, the split into symmetric
+//                     and antisymmetric parts, K[S] + K[A]
 //   k_axis_gemm, k_spin_block              AO->MO / spin-orbital transformation on the FP64 tensor cores (mo_transform.cuh)
 //   k_one_electron, k_cross_overlap        one-electron integrals (oneel_core.cuh)
 // Reference being replaced: TUNA/tuna_integrals/tuna_integral.pyx:1267-1355 (ERI driver), TUNA/tuna_kernel.py:504-523
@@ -29,6 +31,7 @@
 #include <vector>
 
 #include "../../include/tuna_b200.h"
+#include "density_split.hpp"
 #include "devbuf.hpp"
 #include "eri_core.cuh"
 #include "pairtable.hpp"
@@ -93,7 +96,8 @@ struct tuna_ctx {
     DevBuf<double> d_Kpart;
     DevBuf<double> d_fnorm;           // per-component norms (shell engine fill mode)
     PinnedBuf<double> h_pin;
-    DevBuf<unsigned long long> d_scalars;      // [0] max|P| bits, [1] evaluated-quartet counter
+    DevBuf<unsigned long long> d_scalars;      // [0] max|P| bits, [1] evaluated-quartet counter, [2..3] read back by the caller (k_pair_sym_check, k_density_scan)
+    PinnedBuf<unsigned long long> h_scan;      // tuna_jk_direct_general_dev: the two maxima of k_density_scan, read back
 
     int shard_rank = 0, shard_n = 1;
     cudaEvent_t ev[7][2] = {};
@@ -135,8 +139,8 @@ struct tuna_ctx {
     int cur_jobset4 = -1;
     // The job lists are pre-screened on the host with tau / dens_bound, dens_bound = an upper bound of max |P| in the engine's working
     // basis; the device applies the exact test Q_ab Q_cd max|P| < tau.  1e3 covers |P| <= ~10 in the spherical basis (the Cartesian
-    // back-rotation of an h shell can amplify by ~1e2).  tuna_jk_direct raises it for larger host densities; callers of the _dev entry
-    // point with larger densities scale them down (J and K are linear in P).
+    // back-rotation of an h shell can amplify by ~1e2).  tuna_jk_direct and tuna_jk_direct_general_dev set it from max|P| (plan_density);
+    // callers of tuna_jk_direct_dev with larger densities scale them down (J and K are linear in P).
     double dens_bound = 1e3;
     DevBuf<long long> d_fix;          // reproducible accumulation: [J hi | J lo | K hi | K lo], nD * ncart^2 words each
     DevBuf<long long> d_peer;         // tuna_jk_direct_group on ctxs[0]: the other ranks' accumulators, pulled for k_fix_reduce
@@ -1038,6 +1042,42 @@ __global__ void k_add_transpose_signed(const double* __restrict__ acc, double* _
         const double t = acc[d * nn + (int64_t)j * n + i];
         out[x] = ((anti_mask >> d) & 1u) ? acc[x] - t : acc[x] + t;
     }
+}
+
+// max|P| into out[0] and max|P - P^T| into out[1] over a stack of nD n x n densities (bit patterns of non-negative doubles order like
+// integers).  density_extrema takes the same two maxima on the host.
+__global__ void k_density_scan(const double* __restrict__ P, int nD, int n, unsigned long long* out) {
+    const int64_t nn = (int64_t)n * n, total = nD * nn;
+    double pm = 0.0, am = 0.0;
+    for (int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; x < total; x += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t d = x / nn, ij = x % nn;
+        const int i = (int)(ij / n), j = (int)(ij % n);
+        const double v = P[x], t = P[d * nn + (int64_t)j * n + i];
+        pm = fmax(pm, fabs(v));
+        am = fmax(am, fabs(v - t));
+    }
+    for (int o = 16; o > 0; o >>= 1) { pm = fmax(pm, __shfl_down_sync(0xffffffffu, pm, o)); am = fmax(am, __shfl_down_sync(0xffffffffu, am, o)); }
+    if ((threadIdx.x & 31) == 0) {
+        atomicMax(out, (unsigned long long)__double_as_longlong(pm));
+        atomicMax(out + 1, (unsigned long long)__double_as_longlong(am));
+    }
+}
+
+// S = (P + P^T) / 2 into densities 0 .. nD-1 of out, A = (P - P^T) / 2 into nD .. 2 nD-1: the arithmetic of stage_host_density
+__global__ void k_density_split(const double* __restrict__ P, double* __restrict__ out, int nD, int n) {
+    const int64_t nn = (int64_t)n * n, total = nD * nn;
+    for (int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; x < total; x += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t d = x / nn, ij = x % nn;
+        const int i = (int)(ij / n), j = (int)(ij % n);
+        const double v = P[x], t = P[d * nn + (int64_t)j * n + i];
+        out[x] = 0.5 * (v + t);
+        out[total + x] = 0.5 * (v - t);
+    }
+}
+
+// K[P] = K[S] + K[A] of a split stack: out = a + b, one FP64 add per element as in unstage_host_results
+__global__ void k_add_into(double* __restrict__ out, const double* __restrict__ a, const double* __restrict__ b, size_t count) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x) out[i] = a[i] + b[i];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2728,40 +2768,72 @@ static int jk_direct_core(tuna_ctx* ctx, int nD, const double* dP, unsigned anti
     return TUNA_OK;
 }
 
-// Host densities -> ctx's pinned staging buffer h_pin.  A general P splits into symmetric S and antisymmetric A parts: J[P] = J[S],
-// K[P] = K[S] + K[A] with K[A] antisymmetric.  SCF densities are symmetric to round-off (reference guess densities are not always:
-// asymmetry ~1e-8 was observed); a density stack with max|P - P^T| > 1e-15 max|P| runs as 2 nD densities, S first, the A parts marked in
-// anti_mask.  Sets ctx->dens_bound from max|P|.
+// Host densities -> ctx's pinned staging buffer h_pin, split as plan_density (density_split.hpp) decides.  Sets ctx->dens_bound.
 static int stage_host_density(tuna_ctx* ctx, int nD, const double* P, int* nDrun, unsigned* anti_mask) {
     const int nb = ctx->nbf;
     const size_t nn = (size_t)nb * nb;
-    double pmax = 0.0, amax = 0.0;
-    for (int d = 0; d < nD; ++d)
-        for (int i = 0; i < nb; ++i)
-            for (int j = 0; j <= i; ++j) {
-                const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
-                pmax = std::max(pmax, std::max(std::fabs(x), std::fabs(y)));
-                amax = std::max(amax, std::fabs(x - y));
-            }
-    const bool general = amax > 1e-15 * pmax;
-    ctx->dens_bound = std::max(1e3, 1e3 * pmax);          // static pre-screening stays below the device's exact density-weighted test
-    *nDrun = general ? 2 * nD : nD;
-    *anti_mask = 0;
+    double pmax, amax;
+    density_extrema(P, nD, nb, &pmax, &amax);
+    const DensityPlan plan = plan_density(nD, pmax, amax);
+    ctx->dens_bound = plan.dens_bound;
+    *nDrun = plan.nDrun;
+    *anti_mask = plan.anti_mask;
     int rc;
     if ((rc = ensure_mats(ctx, *nDrun, nb, ctx->ncart))) return rc;
     double* hP = ctx->h_pin;
-    if (!general) {
+    if (*nDrun == nD) {
         std::memcpy(hP, P, (size_t)nD * nn * sizeof(double));
     } else {
-        for (int d = 0; d < nD; ++d) {
-            *anti_mask |= 1u << (nD + d);
+        for (int d = 0; d < nD; ++d)
             for (int i = 0; i < nb; ++i)
                 for (int j = 0; j < nb; ++j) {
                     const double x = P[d * nn + (size_t)i * nb + j], y = P[d * nn + (size_t)j * nb + i];
                     hP[d * nn + (size_t)i * nb + j] = 0.5 * (x + y);
                     hP[(nD + d) * nn + (size_t)i * nb + j] = 0.5 * (x - y);
                 }
-        }
+    }
+    return TUNA_OK;
+}
+
+// Device densities (caller's dP, ctx's device and stream) -> ctx->d_P, planned exactly as stage_host_density: k_density_scan, one 16-byte
+// read-back and stream synchronise for plan_density, then the split (k_density_split) or a copy.  Sets ctx->dens_bound.
+static int stage_device_density(tuna_ctx* ctx, int nD, const double* dP, int* nDrun, unsigned* anti_mask) {
+    const int nb = ctx->nbf;
+    const size_t nn = (size_t)nb * nb;
+    GROW(ctx->h_scan, (size_t)2);
+    CK(cudaMemsetAsync(ctx->d_scalars + 2, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    k_density_scan<<<grid_for(ctx, (int64_t)nD * nn, 256, 4), 256, 0, ctx->stream>>>(dP, nD, nb, ctx->d_scalars + 2);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(ctx->h_scan, ctx->d_scalars + 2, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    double pmax, amax;
+    std::memcpy(&pmax, ctx->h_scan.get(), sizeof(double));
+    std::memcpy(&amax, ctx->h_scan.get() + 1, sizeof(double));
+    const DensityPlan plan = plan_density(nD, pmax, amax);
+    ctx->dens_bound = plan.dens_bound;
+    *nDrun = plan.nDrun;
+    *anti_mask = plan.anti_mask;
+    int rc;
+    if ((rc = ensure_mats(ctx, *nDrun, nb, ctx->ncart))) return rc;
+    if (*nDrun == nD) {
+        CK(cudaMemcpyAsync(ctx->d_P, dP, (size_t)nD * nn * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    } else {
+        k_density_split<<<grid_for(ctx, (int64_t)nD * nn, 256, 8), 256, 0, ctx->stream>>>(dP, ctx->d_P, nD, nb);
+        ctx->launches++;
+        CK(cudaGetLastError());
+    }
+    return TUNA_OK;
+}
+
+// ctx->d_J / d_K of a split stack (2 nD densities, as staged by stage_device_density) -> the caller's device J = J[S] and K = K[S] + K[A].
+static int unstage_device_results(tuna_ctx* ctx, int nD, double* dJ, double* dK) {
+    const size_t count = (size_t)nD * ctx->nbf * ctx->nbf;
+    if (dJ) CK(cudaMemcpyAsync(dJ, ctx->d_J, count * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    if (dK) {
+        k_add_into<<<grid_for(ctx, (int64_t)count, 256, 8), 256, 0, ctx->stream>>>(dK, ctx->d_K, ctx->d_K + count, count);
+        ctx->launches++;
+        CK(cudaGetLastError());
     }
     return TUNA_OK;
 }
@@ -2981,6 +3053,35 @@ int tuna_jk_direct_group(tuna_ctx* const* ctxs, int nctx, int nD, const double* 
         CK(cudaMemcpyAsync(ctx->d_P, ctx->h_pin, (size_t)nDrun * ctx->nbf * ctx->nbf * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
         if ((rc = jk_direct_group_core(ctxs, nctx, nDrun, ctx->d_P, anti_mask, J ? ctx->d_J.get() : nullptr, K ? ctx->d_K.get() : nullptr, tau))) return rc;
         return unstage_host_results(ctx, nD, nDrun, J, K);
+    } TUNA_CATCH
+}
+
+int tuna_jk_direct_general_dev(tuna_ctx* ctx, int nD, const double* dP, double* dJ, double* dK, double tau) try {
+    if (!ctx) return TUNA_ERR_ARG;
+    if (ctx->ncart == 0 || ctx->nbf == 0) FAIL(TUNA_ERR_STATE, "tuna_jk_direct_general_dev: basis and transform must be set first");
+    if (nD <= 0 || nD > 8 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_general_dev: bad arguments (1 <= nD <= 8)");
+    CK(cudaSetDevice(ctx->device));
+    int rc, nDrun;
+    unsigned anti_mask;
+    if ((rc = stage_device_density(ctx, nD, dP, &nDrun, &anti_mask))) return rc;
+    if (nDrun == nD) return jk_direct_core(ctx, nD, ctx->d_P, anti_mask, dJ, dK, tau);
+    if ((rc = jk_direct_core(ctx, nDrun, ctx->d_P, anti_mask, dJ ? ctx->d_J.get() : nullptr, dK ? ctx->d_K.get() : nullptr, tau))) return rc;
+    return unstage_device_results(ctx, nD, dJ, dK);
+} TUNA_CATCH
+
+int tuna_jk_direct_group_general_dev(tuna_ctx* const* ctxs, int nctx, int nD, const double* dP, double* dJ, double* dK, double tau) {
+    tuna_ctx* ctx = (ctxs && nctx >= 1) ? ctxs[0] : nullptr;
+    try {
+        int rc, nDrun;
+        if ((rc = group_check(ctxs, nctx))) return rc;
+        if (nD <= 0 || nD > 8 || !dP) FAIL(TUNA_ERR_ARG, "tuna_jk_direct_group_general_dev: bad arguments (1 <= nD <= 8)");
+        CK(cudaSetDevice(ctx->device));
+        unsigned anti_mask;
+        if ((rc = stage_device_density(ctx, nD, dP, &nDrun, &anti_mask))) return rc;
+        for (int r = 1; r < nctx; ++r) ctxs[r]->dens_bound = ctx->dens_bound;
+        if (nDrun == nD) return jk_direct_group_core(ctxs, nctx, nD, ctx->d_P, anti_mask, dJ, dK, tau);
+        if ((rc = jk_direct_group_core(ctxs, nctx, nDrun, ctx->d_P, anti_mask, dJ ? ctx->d_J.get() : nullptr, dK ? ctx->d_K.get() : nullptr, tau))) return rc;
+        return unstage_device_results(ctx, nD, dJ, dK);
     } TUNA_CATCH
 }
 

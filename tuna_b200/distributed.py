@@ -59,23 +59,20 @@ class FockBuilder:
         single = P.ndim == 2
         Ps = P.reshape(self.nD, self.n, self.n)
         # build_device (tuna_jk_direct_dev) takes every density as symmetric.  A guess density can be asymmetric at the 1e-8 level;
-        # such a P goes through tuna_jk_direct, which splits it into symmetric and antisymmetric parts (same 1e-15 relative test) and
-        # honours the shard, so its partial J/K are all-reduced like those of build_device.
-        if np.abs(Ps - Ps.transpose(0, 2, 1)).max() > 1e-15 * np.abs(Ps).max():
-            self.ctx.set_stream(self.stream.cuda_stream)
-            J, K = self.ctx.jk_direct(Ps, self.tau)
-            self.hJK.numpy()[0], self.hJK.numpy()[1] = J, K
-            with self.torch.cuda.stream(self.stream):
+        # such a P goes through tuna_jk_direct_general_dev, which splits it into symmetric and antisymmetric parts on the device (same
+        # 1e-15 relative test, bitwise the J and K of tuna_jk_direct) and honours the shard, so its partial J/K are all-reduced alike.
+        general = np.abs(Ps - Ps.transpose(0, 2, 1)).max() > 1e-15 * np.abs(Ps).max()
+        self.hP.numpy()[...] = Ps
+        with self.torch.cuda.stream(self.stream):
+            self.dP.copy_(self.hP, non_blocking=True)
+            if general:
+                self.ctx.set_stream(self.stream.cuda_stream)
+                self.ctx.jk_direct_general_dev(self.nD, self.dP.data_ptr(), self.dJK[0].data_ptr(), self.dJK[1].data_ptr(), self.tau)
                 if self.world > 1:
-                    self.dJK.copy_(self.hJK, non_blocking=True)
                     self.dist.all_reduce(self.dJK, group=self.group)
-                    self.hJK.copy_(self.dJK, non_blocking=True)
-        else:
-            self.hP.numpy()[...] = Ps
-            with self.torch.cuda.stream(self.stream):
-                self.dP.copy_(self.hP, non_blocking=True)
+            else:
                 self.build_device()
-                self.hJK.copy_(self.dJK, non_blocking=True)
+            self.hJK.copy_(self.dJK, non_blocking=True)
         self.stream.synchronize()
         J, K = self.hJK.numpy()[0].copy(), self.hJK.numpy()[1].copy()
         return (J[0], K[0]) if single else (J, K)
