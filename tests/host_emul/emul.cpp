@@ -67,6 +67,7 @@ int emul_eri_fill(int ncart, const double* oz, const int* lmn, const int* nprim,
 }
 
 // ---- shell-quartet engine (shell_jk.cuh) with the serial HostPolicy ------------------------------------------------
+#include "../../tuna_b200/csrc/density_split.hpp"
 #include "../../tuna_b200/csrc/shell_host.hpp"
 #include "../../tuna_b200/csrc/shell4_host.hpp"
 
@@ -116,6 +117,9 @@ extern "C" int emul_jk_shell4(int ncart, const double* oz, const int* lmn, const
                 Pf[d * nn + (size_t)i * ncart + j] = S.fnorm[i] * S.fnorm[j] * P[d * nn + (size_t)i * ncart + j];
                 dmax = std::max(dmax, std::fabs(P[d * nn + (size_t)i * ncart + j]));
             }
+    double pmax, amax;      // the job lists are pre-screened with the bound the device build sets for this stack (plan_density)
+    density_extrema(P, nD, ncart, &pmax, &amax);
+    const double dens_bound = plan_density(nD, pmax, amax).dens_bound;
     std::vector<double> Psym(nD * nn);
     for (int d = 0; d < nD; ++d)
         for (int i = 0; i < ncart; ++i)
@@ -141,7 +145,7 @@ extern "C" int emul_jk_shell4(int ncart, const double* oz, const int* lmn, const
             }
             J.bra_list = S.classes[cb].pairs.data(); J.ket_list = S.classes[ck].pairs.data();
             std::vector<long long> prefix;
-            J.nitems = build_item_prefix(S, cb, ck, tau * 1e-3, prefix);
+            J.nitems = build_item_prefix(S, cb, ck, tau / dens_bound, prefix);
             J.item_prefix = prefix.data(); J.nbra = (int)S.classes[cb].pairs.size(); J.same_class = (cb == ck);
             Class4Host CH;
             const char* eb = getenv("TUNA_EMUL_IT_BUDGET");      // small budgets force the multi-chunk path in tests

@@ -163,6 +163,9 @@ def test_group_bitwise_equals_one_device(name, n):
     _assert_bitwise(group.jk_direct(P, 1e-16), ref)
     _assert_bitwise(group.jk_direct(P, 1e-16), ref)                 # a second build on the same group
     assert group.counts()["evaluated_last_direct"] == solo.counts()["evaluated_last_direct"]
+    ref = solo.jk_direct(P, 1e-10)                                  # a direct SCF's threshold: the ranks drop what one device drops
+    _assert_bitwise(group.jk_direct(P, 1e-10), ref)
+    assert group.counts()["evaluated_last_direct"] == solo.counts()["evaluated_last_direct"]
     if name == "ne2_uhf_ccpvqz":
         from tuna_b200 import workloads as w
         g = load_golden(name)

@@ -230,6 +230,21 @@ def test_asymmetric_density_and_screening_changes():
 
 
 @pytest.mark.gpu
+def test_threshold_ladder_bitwise():
+    """The Schwarz threshold up from 1e-14 to 1e-6 and back down, with a small, a x 1e3 and a small density in turn: a stored job whose
+    kept quartet list changes with tau runs direct, and the result is bitwise that of a context without the store at every step."""
+    flat, U, g = _case("et100")
+    P = _sequence(g)[-1]
+    taus = (1e-14, 1e-12, 1e-10, 1e-8, 1e-6)
+    direct, semi = _ctx(flat, U), _ctx(flat, U, budget=BIG)
+    for i, t in enumerate(taus + taus[::-1]):
+        Q = (P, 1e3 * P, P)[i % 3]
+        _bitwise(semi.jk_direct(Q, t), direct.jk_direct(Q, t), f"build {i} tau {t:g}")
+        assert semi.counts()["evaluated_last_direct"] == direct.counts()["evaluated_last_direct"]
+    assert semi.integral_store_info()["replayed_builds"] >= 1
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("name", ["n2_ccpvtz", "et100"])
 def test_budgets(name):
     """Budgets of nothing, a small part, half and everything: the same J and K, never more bytes than the budget."""

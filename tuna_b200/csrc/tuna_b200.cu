@@ -138,8 +138,9 @@ struct tuna_ctx {
     std::vector<JobSet4> jobsets4;
     int cur_jobset4 = -1;
     // The job lists are pre-screened on the host with tau / dens_bound, dens_bound = an upper bound of max |P| in the engine's working
-    // basis; the device applies the exact test Q_ab Q_cd max|P| < tau.  1e3 covers |P| <= ~10 in the spherical basis (the Cartesian
-    // back-rotation of an h shell can amplify by ~1e2).  tuna_jk_direct and tuna_jk_direct_general_dev set it from max|P| (plan_density);
+    // basis; the device applies the exact test Q_ab Q_cd max|P| < tau.  The margin of 1e3 over the caller's max|P| covers the Cartesian
+    // amplification max|U^T P U| / max|P| <= (max_a sum_p |U_pa|)^2: 2.4 to 3.5 for the cc-pVTZ / cc-pVQZ transforms, 9 for an h-shell
+    // one (tests/test_screening.py).  tuna_jk_direct and tuna_jk_direct_general_dev set it from max|P| (plan_density);
     // callers of tuna_jk_direct_dev with larger densities scale them down (J and K are linear in P).
     double dens_bound = 1e3;
     DevBuf<long long> d_fix;          // reproducible accumulation: [J hi | J lo | K hi | K lo], nD * ncart^2 words each
